@@ -170,17 +170,6 @@ int kw_gmm_mstep_finalize(int n_components, int dim, double reg_covar, int weigh
                           double* prec_chol_dev, double* aux_dev, int32_t* info_dev,
                           void* stream);
 
-/* Exchange form of the statistics for the all-reduce between ranks: the second-moment blocks are
- * symmetric, so [n_k, first moments, upper triangle] per component plus the two tail scalars carry
- * everything -- K (1 + D + D (D + 1) / 2) + 2 doubles, about half of kw_gmm_stats_len.  Pack, sum
- * the packed vectors over the ranks, unpack (the lower triangle is mirrored).  Optional: worth it
- * where the link bandwidth bounds the all-reduce; over NVLink the full vector is as fast. */
-size_t kw_gmm_stats_packed_len(int n_components, int dim);
-int kw_gmm_stats_pack(int n_components, int dim, const double* stats_dev, double* packed_dev,
-                      void* stream);
-int kw_gmm_stats_unpack(int n_components, int dim, const double* packed_dev, double* stats_dev,
-                        void* stream);
-
 /* prec_chol / aux from given covariances (precisions_cholesky_ of an existing model). */
 int kw_gmm_precision_cholesky(int n_components, int dim, const double* weights_dev,
                               const double* means_dev, const double* covariances_dev,

@@ -34,9 +34,6 @@ SIGNATURES = {
     'kw_gmm_normalize_resp': (_i, [_i64, _i, _i, _vp, _vp, _sz, _vp]),
     'kw_gmm_hard_labels': (_i, [_i64, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
     'kw_gmm_mstep_accumulate': (_i, [_i64, _vp, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _sz, _vp]),
-    'kw_gmm_stats_packed_len': (_sz, [_i, _i]),
-    'kw_gmm_stats_pack': (_i, [_i, _i, _vp, _vp, _vp]),
-    'kw_gmm_stats_unpack': (_i, [_i, _i, _vp, _vp, _vp]),
     'kw_gmm_mstep_finalize': (_i, [_i, _i, _dbl, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                    _vp]),
     'kw_gmm_precision_cholesky': (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -58,51 +58,11 @@ __global__ void mc2b_kernel(long long total, int width, double alpha, int zero_p
     }
 }
 
-// The second-moment block of the statistics is symmetric: what travels between ranks is
-// [n_k, first moments, upper triangle] per component plus the two tail scalars -- half the bytes.
-// packed layout per component: 1 + D + D (D + 1) / 2 doubles, triangle row by row (i <= j).
-// grid (K, slices): about four elements per thread, so the copies run at bandwidth instead of
-// one component's memory latency per CTA
-static int stats_slices(int K, int D) {
-    const long long per = ((long long)D * D + 1023) / 1024;
-    return (int)std::max<long long>(1, std::min<long long>(per, 64));
-}
-
-__global__ void stats_pack_kernel(int K, int D, const double* __restrict__ stats,
-                                  double* __restrict__ packed) {
-    const size_t sb = 1 + (size_t)D + (size_t)D * D, pb = 1 + (size_t)D + (size_t)D * (D + 1) / 2;
-    const int k = blockIdx.x;
-    const double* s = stats + (size_t)k * sb;
-    double* p = packed + (size_t)k * pb;
-    const int tid = blockIdx.y * blockDim.x + threadIdx.x, nthr = gridDim.y * blockDim.x;
-    for (int e = tid; e < 1 + D; e += nthr) p[e] = s[e];
-    for (int e = tid; e < D * D; e += nthr) {
-        const int i = e / D, j = e - i * D;
-        if (j >= i) p[1 + D + (size_t)i * D - (size_t)i * (i - 1) / 2 + (j - i)] = s[1 + D + e];
-    }
-    if (k == 0 && tid < 2) packed[(size_t)K * pb + tid] = stats[(size_t)K * sb + tid];
-}
-__global__ void stats_unpack_kernel(int K, int D, const double* __restrict__ packed,
-                                    double* __restrict__ stats) {
-    const size_t sb = 1 + (size_t)D + (size_t)D * D, pb = 1 + (size_t)D + (size_t)D * (D + 1) / 2;
-    const int k = blockIdx.x;
-    double* s = stats + (size_t)k * sb;
-    const double* p = packed + (size_t)k * pb;
-    const int tid = blockIdx.y * blockDim.x + threadIdx.x, nthr = gridDim.y * blockDim.x;
-    for (int e = tid; e < 1 + D; e += nthr) s[e] = p[e];
-    for (int e = tid; e < D * D; e += nthr) {
-        const int i = e / D, j = e - i * D;
-        const int a = min(i, j), b = max(i, j);
-        s[1 + D + e] = p[1 + D + (size_t)a * D - (size_t)a * (a - 1) / 2 + (b - a)];
-    }
-    if (k == 0 && tid < 2) stats[(size_t)K * sb + tid] = packed[(size_t)K * pb + tid];
-}
-
 }  // namespace kw
 
 using namespace kw;
 
-extern "C" int kw_abi_version(void) { return 2; }
+extern "C" int kw_abi_version(void) { return 3; }
 
 extern "C" const char* kw_last_error(void) { return g_error; }
 
@@ -140,28 +100,6 @@ extern "C" int kw_mc2b(int64_t total_frames, int width, double alpha, int zero_p
     KW_REQUIRE(total_frames > 0 && width > 0, "kw_mc2b: bad sizes");
     mc2b_kernel<<<(unsigned)((total_frames + 127) / 128), 128, 0, st>>>(
         total_frames, width, alpha, zero_power, mc_dev, b_dev);
-    KW_CUDA_CHECK(cudaGetLastError());
-    return KW_OK;
-}
-
-extern "C" size_t kw_gmm_stats_packed_len(int K, int D) {
-    return (size_t)K * (1 + (size_t)D + (size_t)D * (D + 1) / 2) + 2;
-}
-
-extern "C" int kw_gmm_stats_pack(int K, int D, const double* stats_dev, double* packed_dev,
-                                 void* stream) {
-    KW_REQUIRE(K > 0 && D > 0, "kw_gmm_stats_pack: K, D must be positive");
-    stats_pack_kernel<<<dim3(K, stats_slices(K, D)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        K, D, stats_dev, packed_dev);
-    KW_CUDA_CHECK(cudaGetLastError());
-    return KW_OK;
-}
-
-extern "C" int kw_gmm_stats_unpack(int K, int D, const double* packed_dev, double* stats_dev,
-                                   void* stream) {
-    KW_REQUIRE(K > 0 && D > 0, "kw_gmm_stats_unpack: K, D must be positive");
-    stats_unpack_kernel<<<dim3(K, stats_slices(K, D)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        K, D, packed_dev, stats_dev);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }

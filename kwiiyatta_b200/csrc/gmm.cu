@@ -410,17 +410,13 @@ static size_t finalize_smem_bytes(int D) {
     return sizeof(double) * ((size_t)D * S + (size_t)D * (FIN_NB + 1) + 3 * (size_t)D);
 }
 
-__device__ long long fin_prof[8];     // KW_FIN_PROF: phase clocks of block 0 (diagnostics)
-
 __global__ void __launch_bounds__(FIN_THREADS)
 gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_stats,
                     const double* __restrict__ stats, const double* __restrict__ centres,
                     double* __restrict__ weights, double* __restrict__ means,
                     double* __restrict__ covariances, double* __restrict__ prec_chol,
-                    double* __restrict__ aux, int32_t* __restrict__ info, int prof) {
+                    double* __restrict__ aux, int32_t* __restrict__ info) {
     extern __shared__ double A[];
-    const bool prof_on = prof != 0 && blockIdx.x == 0 && threadIdx.x == 0;
-    if (prof_on) fin_prof[0] = clock64();
     const int S = D | 1;
     double* T = A + (size_t)D * S;            // [column][FIN_NB + 1] scratch of the inverse
     double* dg = T + (size_t)D * (FIN_NB + 1);   // L[j][j]
@@ -470,7 +466,6 @@ gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_st
     if (tid == 0) sh_fail = 0;
     __syncthreads();
 
-    if (prof_on) fin_prof[1] = clock64();
     // ---- Cholesky, left-looking by panels of FIN_NB columns --------------------------------
     // Per element the products are subtracted in ascending column order (the arithmetic of an
     // unblocked left-looking sweep).
@@ -520,9 +515,9 @@ gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_st
             __syncthreads();
         }
         // Inside the panel, two barriers instead of one per column.  Per element the products are
-        // still subtracted in ascending column order.  (Measured with finer clocks than KW_FIN_PROF
-        // keeps: of the Cholesky's 136k clk the left-looking panel updates take 69k -- few warps
-        // are active in the late panels and the dot products wait for shared memory -- the
+        // still subtracted in ascending column order.  (Measured with clocks in block 0 before
+        // commit 3a91ef5: of the Cholesky's 136k clk the left-looking panel updates take 69k -- few
+        // warps are active in the late panels and the dot products wait for shared memory -- the
         // diagonal blocks 80k, 550 clk per pivot in one warp, the rows below 22k.)
         // (a) the nb x nb diagonal block in ONE warp: lane r keeps row r in registers, the pivot
         //     column travels through a small shared-memory line.
@@ -632,7 +627,6 @@ gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_st
         }
         __syncthreads();
     }
-    if (prof_on) fin_prof[2] = clock64();
     // (A[j][j] still holds the pre-pivot value; the diagonal of L lives in dg)
     for (int j = tid; j < D; j += FIN_THREADS) zd[j] = 1.0 / dg[j];
     __syncthreads();
@@ -704,7 +698,6 @@ gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_st
         }
         __syncthreads();
     }
-    if (prof_on) fin_prof[3] = clock64();
     // prec_chol (upper) = Z^T; diagonal 1 / L[j][j]
     double* pc = prec_chol + (size_t)k * D * D;
     for (int r = tid >> 5; r < D; r += FIN_THREADS / 32)
@@ -735,7 +728,6 @@ gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_st
         ak[D + 1] = log(wk);
         info[k] = sh_fail;
     }
-    if (prof_on) fin_prof[4] = clock64();
 }
 
 static int m_chunks(int K) {
@@ -830,17 +822,9 @@ int finalize_launch(int K, int D, double reg_covar, int weight_norm, int from_st
     const size_t smem = finalize_smem_bytes(D);
     KW_CUDA_CHECK(cudaFuncSetAttribute(gmm_finalize_kernel,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const bool prof = getenv("KW_FIN_PROF") != nullptr;      // diagnostics only
     gmm_finalize_kernel<<<K, FIN_THREADS, smem, st>>>(K, D, reg_covar, weight_norm, from_stats, stats,
-                                              centres, weights, means, cov, pc, aux, info, prof);
+                                              centres, weights, means, cov, pc, aux, info);
     KW_CUDA_CHECK(cudaGetLastError());
-    if (prof) {
-        long long h[8];
-        KW_CUDA_CHECK(cudaStreamSynchronize(st));
-        KW_CUDA_CHECK(cudaMemcpyFromSymbol(h, fin_prof, sizeof(h)));
-        fprintf(stderr, "[finalize block 0] statistics -> covariance %lld clk, Cholesky %lld, inverse %lld, "
-                        "write-out %lld\n", h[1] - h[0], h[2] - h[1], h[3] - h[2], h[4] - h[3]);
-    }
     return KW_OK;
 }
 

@@ -24,7 +24,6 @@
 #include <cuda_fp16.h>
 
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -61,12 +60,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
         : "r"(smem_u32(bar)), "r"(parity)
         : "memory");
     return ok != 0;
-}
-// Cycle counter for the optional role profiles; compiled out of the production kernels (reading
-// the clock serialises the issuing warp).
-template <bool PROF> __device__ __forceinline__ long long tick() {
-    if constexpr (PROF) return clock64();
-    return 0;
 }
 // Bounded wait: a protocol bug must trap, not hang the GPU.
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
@@ -546,14 +539,13 @@ enum { BAR_A_FULL = 0, BAR_A_EMPTY, BAR_BLO_FULL0, BAR_BLO_FULL1, BAR_BLO_EMPTY0
        BAR_BHI_FULL0, BAR_BHI_FULL1,
        BAR_BHI_EMPTY0, BAR_BHI_EMPTY1, BAR_TM_FULL0, BAR_TM_FULL1, BAR_TM_EMPTY0, BAR_TM_EMPTY1 };
 
-template <bool PROF, int G>
+template <int G>
 __global__ void __launch_bounds__(576, 1)
 estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                 uint32_t tmem_cols, const __half* __restrict__ xt, const __half* __restrict__ bt,
                 const double* __restrict__ cst,
                 double* __restrict__ wlpT, int mode, int32_t* __restrict__ mix,
-                int32_t* __restrict__ cand, double near_tie, int late_release,
-                unsigned long long* __restrict__ prof) {
+                int32_t* __restrict__ cand, double near_tie, int late_release) {
     extern __shared__ __align__(128) unsigned char smem[];
     const EstepSmem L = estep_smem(DP, G);
     __half* a_hi = reinterpret_cast<__half*>(smem + L.a);
@@ -626,8 +618,6 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
             const uint64_t d_b_hi0 = make_desc(smem_u32(b_hi0), 128, 256);
             const uint64_t d_b_hi1 = make_desc(smem_u32(b_hi0 + item_elems), 128, 256);
             constexpr uint64_t KSTEP = 256 >> 4;      // A: 16 fp16 along K = two core matrices
-            long long p_tm = 0, p_blo = 0, p_bhi = 0, p_issue = 0;
-            const long long p_start = tick<PROF>();
             const uint32_t ta_hi = tmem_base + 2u * acc_w;              // A (hi) after the accumulators
             const uint32_t ta_lo = ta_hi + (uint32_t)DP / 2 + 8;        // hi has the ones k-step too
             const uint64_t bias_off = (uint64_t)(G * bbias_off(DP) * 2) >> 4;   // descriptor address units
@@ -655,12 +645,8 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                         tmem_cp_128x256b(ta_hi + 8 * (uint32_t)ksteps, d_a_hi + (uint64_t)ksteps * KSTEP);
                         umma_commit(bars + BAR_A_EMPTY);
                     }
-                    const long long c0 = tick<PROF>();
                     mbar_wait(bars + BAR_TM_EMPTY0 + s, (u & 1u) ^ 1u);
-                    const long long c1 = tick<PROF>();
                     mbar_wait(bars + BAR_BLO_FULL0 + s, u & 1u);
-                    const long long c2 = tick<PROF>();
-                    p_tm += c1 - c0; p_blo += c2 - c1;
                     tc_fence_after();
                     {
                         uint64_t db = s ? d_b_lo1 : d_b_lo0;          // x_hi . l_lo
@@ -673,10 +659,7 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                         }
                     }
                     umma_commit(bars + BAR_BLO_EMPTY0 + s);
-                    const long long c3 = tick<PROF>();
                     mbar_wait(bars + BAR_BHI_FULL0 + s, u & 1u);
-                    const long long c4 = tick<PROF>();
-                    p_bhi += c4 - c3; p_issue += c3 - c2;
                     tc_fence_after();
                     {
                         uint64_t db = d_b_hi;          // x_lo . l_hi
@@ -703,15 +686,7 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                     }
                     umma_commit(bars + BAR_BHI_EMPTY0 + s);
                     umma_commit(bars + BAR_TM_FULL0 + s);
-                    p_issue += tick<PROF>() - c4;
                 }
-            }
-            if (prof != nullptr && blockIdx.x == 0 && lane == 0) {
-                prof[0] = (unsigned long long)(tick<PROF>() - p_start);
-                prof[1] = (unsigned long long)p_tm;
-                prof[2] = (unsigned long long)p_blo;
-                prof[3] = (unsigned long long)p_bhi;
-                prof[4] = (unsigned long long)p_issue;
             }
         }
     } else {
@@ -719,15 +694,12 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
         // Four warps per TMEM lane quarter, each takes a quarter of the accumulator columns; the
         // partial q of parts 1..3 goes through shared memory to part 0, which finishes.  (The
         // epilogue, not the MMA, bounds this kernel: more warps = more latency hiding.)
-        const int et = threadIdx.x - 64;            // 0..511
         const uint32_t quarter = (uint32_t)(warp & 3);
         const int part = (warp - 2) >> 2;           // 0..3
         const int row = (int)quarter * 32 + lane;   // TMEM lane = row of the tile
         const int n_chunks = G * ksteps;            // 16-column chunks of an accumulator stage
         const int c_begin = (n_chunks * part) / 4, c_end = (n_chunks * (part + 1)) / 4;
         const double LOG2PI = 1.8378770664093453;
-        long long q_bar = 0, q_wait = 0, q_work = 0;
-        const long long q_start = tick<PROF>();
         int it = 0;
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
             const long long n = (long long)tile * TILE_M + row;
@@ -754,11 +726,7 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
 #pragma unroll
                     for (int e = 0; e < 3; ++e) cc[c][e] = nc[c][e];
                 if (item + 1 < KI) fetch(item + 1);
-                const long long e0 = tick<PROF>();
-                const long long e1 = tick<PROF>();
                 mbar_wait(bars + BAR_TM_FULL0 + s, u & 1u);
-                const long long e2 = tick<PROF>();
-                q_bar += e1 - e0; q_wait += e2 - e1;
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((quarter * 32u) << 16) + s * acc_w;
                 // with G = 2 a chunk holds 8 columns of the item's first component, then 8 of
@@ -809,13 +777,11 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                     qp[0] = qa;
                     qp[1] = qb;
                 }
-                const long long e3 = tick<PROF>();
                 // The only CTA-level synchronisation of an item: parts 1..3 signal that their
                 // partial sums are in shared memory (named barrier 3 + slot, they do not wait),
                 // part 0 waits for them.
                 if (part == 0) asm volatile("bar.sync %0, 512;" ::"r"(3u + q4) : "memory");
                 else asm volatile("bar.arrive %0, 512;" ::"r"(3u + q4) : "memory");
-                q_work += e3 - e2; q_bar += tick<PROF>() - e3;
                 if (part == 0) {
 #pragma unroll
                     for (int pp = 0; pp < 3; ++pp) {
@@ -823,7 +789,7 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                         qa += qp[0];
                         qb += qp[1];
                     }
-                    if (late_release) {      // experiment: the stage freed after the partial sums
+                    if (late_release) {      // the stage freed after the partial sums
                         __syncwarp();
                         if (lane == 0) mbar_arrive(bars + BAR_TM_EMPTY0 + s);
                     }
@@ -849,13 +815,6 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                 mix[n] = k1;
                 cand[n] = (K > 1 && v1 - v2 < near_tie) ? k2 : -1;   // runner-up to re-check in fp64
             }
-        }
-        if (prof != nullptr && blockIdx.x == 0 && (et == 0 || et == 511)) {
-            unsigned long long* pp = prof + (et == 0 ? 8 : 12);
-            pp[0] = (unsigned long long)(tick<PROF>() - q_start);
-            pp[1] = (unsigned long long)q_bar;
-            pp[2] = (unsigned long long)q_wait;
-            pp[3] = (unsigned long long)q_work;
         }
     }
     tc_fence_before();
@@ -1272,9 +1231,10 @@ lse_prep_kernel(long long N, long long Npad, int K, const double* __restrict__ w
 // flags of mstats_tc_prep_kernel / lse_prep_kernel + the producer's ballot over 32 tiles); work
 // items are drawn from a global counter, longest first (mstats_tc_order_kernel), and handed to the
 // other roles through a 4-slot ring, because frames sorted by dominant component make them very
-// uneven.  With dense data the kernel runs into the board's power cap (tools/time_mstep.py); on
-// real posteriors the per-tile hand-offs bound it (tools/time_mstep_real.py): the dbg bits exist
-// to take such measurements.
+// uneven.  With dense data the kernel runs into the board's power cap (tools/time_mstep.py; 984 W
+// of 1 kW on a B200, commit 1c8d74c); on real posteriors the per-tile hand-offs bound it, as
+// measured with per-role wait clocks and switches that turned roles off (commits 1c8d74c to
+// 5493bff; the instrumentation is in git history up to a73b842).
 // ------------------------------------------------------------------------------------------
 constexpr int M2_NB = 3;           // B stages
 struct Mstep2Smem {
@@ -1299,17 +1259,12 @@ __host__ __device__ inline Mstep2Smem mstep2_smem(int DP) {
 enum { M2_B_FULL = 0, M2_B_EMPTY = 3, M2_A_FULL = 6, M2_A_EMPTY = 8, M2_TM_FULL = 10,
        M2_TM_EMPTY = 12, M2_IT_FULL = 14, M2_IT_EMPTY = 18 };
 
-__device__ unsigned long long m2_prof[40];    // KW_TC_MSWAP & 16384: per-role wait clocks of CTA 0
-
 __global__ void __launch_bounds__(640, 1)
 mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk, int n_chunks,
                   int K, int DP, const __half* __restrict__ xt, const float* __restrict__ wts,
                   const float* __restrict__ mu32, float* __restrict__ partial,
                   int* __restrict__ item_counter, const int* __restrict__ item_order,
-                  const unsigned char* __restrict__ tflags, int n_mt_pad, int dbg) {
-    // dbg (timing experiments only, 0 in production): 1 = no MMAs, 2 = no operand generation,
-    // 4 = no epilogue loads, 1024 = no bulk copies, 2048 = no corner MMAs, 16384 = CTA 0 reports
-    // the clocks each role spends in its barrier waits
+                  const unsigned char* __restrict__ tflags, int n_mt_pad) {
     extern __shared__ __align__(128) unsigned char smem[];
     const MstepGeom G = mstep_geom(DP);
     const Mstep2Smem L = mstep2_smem(DP);
@@ -1380,29 +1335,6 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
         t1 = min(n_mtiles, t0 + tiles_per_chunk);
     };
 
-    // dbg & 16384: CTA 0 adds up the clocks each role spends in its barrier waits (m2_prof)
-    const bool prof_on = (dbg & 16384) != 0 && blockIdx.x == 0;
-    long long pw[4] = {0, 0, 0, 0};
-    const long long p_begin = prof_on ? clock64() : 0;
-    long long p_tiles = 0;
-    auto twait = [&](uint64_t* bar, uint32_t parity, long long& acc) {
-        if (!prof_on) {
-            mbar_wait(bar, parity);
-            return;
-        }
-        const long long t0 = clock64();
-        mbar_wait(bar, parity);
-        acc += clock64() - t0;
-    };
-    auto report = [&](int role) {
-        if (prof_on && lane == 0) {
-            unsigned long long* o = m2_prof + role * 8;
-            o[0] = (unsigned long long)(clock64() - p_begin);
-            o[1] = (unsigned long long)p_tiles;
-            for (int i = 0; i < 4; ++i) o[2 + i] = (unsigned long long)pw[i];
-        }
-    };
-
     if (warp < 4) {
       reg_dec<48>();
       if (warp == 0) {
@@ -1418,7 +1350,7 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
             // The item's tiles that carry weight, in order.  This warp is one serial instruction
             // stream per tile, and at ~200 instructions per tile (weights through registers, tile
             // maximum, scale) it was the slowest role of the kernel on real posteriors
-            // (tools/time_mstep_real.py, KW_TC_MSWAP=16384: busy 83 % of the time, the MMA warp
+            // (per-role wait clocks, commit 5493bff: busy 83 % of the time, the MMA warp
             // waiting).  All of that now happens beforehand in mstats_tc_prep_kernel; here a tile
             // is three bulk copies: packed frames hi, lo and the prepared weights.
             for (int tb = t0; tb < t1; tb += 32) {
@@ -1428,23 +1360,17 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                     const int t = tb + __ffs(mask) - 1;
                     mask &= mask - 1;
                     const uint32_t s = g % M2_NB, u = g / M2_NB;
-                    twait(bars + M2_B_EMPTY + s, (u & 1u) ^ 1u, pw[0]);
-                    ++p_tiles;
+                    mbar_wait(bars + M2_B_EMPTY + s, (u & 1u) ^ 1u);
                     if (lane == 0) {
                         pent[s] = t;
-                        if (dbg & 1024) {                 // no bulk copies
-                            mbar_arrive(bars + M2_B_FULL + s);
-                        } else {
-                            mbar_expect_tx(bars + M2_B_FULL + s, 2 * part_b + WSTRIDE * 4);
-                            const __half* tile = xt + (size_t)(t >> 1) * X_PARTS * tile_elems(DP) +
-                                                 3 * tile_elems(DP) + (size_t)(t & 1) * MT * DPB;
-                            unsigned char* dst = b_base + s * L.b_stage;
-                            bulk_g2s(dst, tile, part_b, bars + M2_B_FULL + s);
-                            bulk_g2s(dst + part_b, tile + tile_elems(DP), part_b,
-                                     bars + M2_B_FULL + s);
-                            bulk_g2s(r_s + s * WSTRIDE, wk + (size_t)t * WSTRIDE, WSTRIDE * 4,
-                                     bars + M2_B_FULL + s);
-                        }
+                        mbar_expect_tx(bars + M2_B_FULL + s, 2 * part_b + WSTRIDE * 4);
+                        const __half* tile = xt + (size_t)(t >> 1) * X_PARTS * tile_elems(DP) +
+                                             3 * tile_elems(DP) + (size_t)(t & 1) * MT * DPB;
+                        unsigned char* dst = b_base + s * L.b_stage;
+                        bulk_g2s(dst, tile, part_b, bars + M2_B_FULL + s);
+                        bulk_g2s(dst + part_b, tile + tile_elems(DP), part_b, bars + M2_B_FULL + s);
+                        bulk_g2s(r_s + s * WSTRIDE, wk + (size_t)t * WSTRIDE, WSTRIDE * 4,
+                                 bars + M2_B_FULL + s);
                     }
                     __syncwarp();
                     ++g;
@@ -1461,7 +1387,6 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 ++g;
             }
         }
-        report(0);
       } else if (warp == 1) {
         // ---------------- MMA issuer: A from TMEM, B K-major from shared memory -----------------
         const uint32_t idesc = make_idesc(128, G.N1);
@@ -1481,12 +1406,11 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 const uint32_t sb = g % M2_NB, ub = g / M2_NB;
                 const uint32_t sa = g & 1u, ua = g >> 1;
                 const uint32_t ts = f & 1u, tu = f >> 1;
-                twait(bars + M2_B_FULL + sb, ub & 1u, pw[0]);
+                mbar_wait(bars + M2_B_FULL + sb, ub & 1u);
                 const int tt = pent[sb];
                 const float tile_inv = r_s[sb * WSTRIDE + MT];
-                twait(bars + M2_TM_EMPTY + ts, (tu & 1u) ^ 1u, pw[1]);
-                twait(bars + M2_A_FULL + sa, ua & 1u, pw[2]);
-                ++p_tiles;
+                mbar_wait(bars + M2_TM_EMPTY + ts, (tu & 1u) ^ 1u);
+                mbar_wait(bars + M2_A_FULL + sa, ua & 1u);
                 tc_fence_after();
                 ++g;
                 if (tt < 0) {
@@ -1507,14 +1431,10 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 const uint64_t b_hi = d_b[sb][0], b_lo = d_b[sb][1];
                 // cross passes first (2^-11 of the main term), so only the four A_hi B_hi MMAs
                 // truncate the accumulator at full magnitude
-                if (!(dbg & 1))
 #pragma unroll
                 for (int pass = 0; pass < 3; ++pass) {
                     const uint32_t ta = (pass == 1) ? a_lo : a_hi;
                     uint64_t db = (pass == 0) ? b_lo : b_hi;
-                    if ((pass == 0 && (dbg & 32)) || (pass == 1 && (dbg & 64)) ||
-                        (pass == 2 && (dbg & 128)))
-                        continue;
 #pragma unroll
                     for (int ks = 0; ks < MT / 16; ++ks) {
                         umma_f16_ts(acc, ta + 8u * ks, db, idesc, (pass > 0 || ks > 0) ? 1u : 0u);
@@ -1533,7 +1453,6 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 ++f;
             }
         }
-        report(1);
       } else if (corner) {
         // ---------------- corner warps 2, 3: features 128..143 x columns 128..151 -----------
         // mma.sync m16n8k16 from the K-major tiles: A rows = the 16 corner features (their own
@@ -1563,13 +1482,12 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
             for (;;) {
                 const uint32_t sb = g % M2_NB, ub = g / M2_NB;
                 const uint32_t sa = g & 1u, ua = g >> 1;
-                twait(bars + M2_B_FULL + sb, ub & 1u, pw[0]);
+                mbar_wait(bars + M2_B_FULL + sb, ub & 1u);
                 const int tt = pent[sb];
                 const float tile_inv = r_s[sb * WSTRIDE + MT];
-                twait(bars + M2_A_FULL + sa, ua & 1u, pw[1]);
-                ++p_tiles;
+                mbar_wait(bars + M2_A_FULL + sa, ua & 1u);
                 ++g;
-                if (tt >= 0 && !(dbg & 2048)) {
+                if (tt >= 0) {
                     const uint32_t ab = a_s0 + sa * 4096u + la, bb = b_s0 + sb * L.b_stage;
 #pragma unroll
                     for (int kq = 0; kq < MT / 32; ++kq) {
@@ -1631,7 +1549,6 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 }
             asm volatile("bar.sync 3, 64;" ::: "memory");
         }
-        if (warp == 2) report(2);
       }
     } else if (warp < 12) {
         reg_dec<88>();
@@ -1664,10 +1581,9 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
             for (;;) {
                 const uint32_t sb = g % M2_NB, ub = g / M2_NB;
                 const uint32_t sa = g & 1u, ua = g >> 1;
-                twait(bars + M2_B_FULL + sb, ub & 1u, pw[0]);
+                mbar_wait(bars + M2_B_FULL + sb, ub & 1u);
                 const int tt = pent[sb];
-                twait(bars + M2_A_EMPTY + sa, (ua & 1u) ^ 1u, pw[1]);
-                ++p_tiles;
+                mbar_wait(bars + M2_A_EMPTY + sa, (ua & 1u) ^ 1u);
                 tc_fence_after();
                 const unsigned char* bh = b_base + sb * L.b_stage;
                 const float* rt = r_s + sb * WSTRIDE;
@@ -1698,7 +1614,7 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                         zl[e] = *reinterpret_cast<const uint32_t*>(&zl2);
                     }
                 };
-                if (tt >= 0 && !(dbg & 2)) {
+                if (tt >= 0) {
 #pragma unroll
                     for (int kk = 0; kk < 2; ++kk) {
                         const int ks = 2 * h + kk;
@@ -1707,12 +1623,8 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                                  zh, zl);
                         convert8(row_off + ((((uint32_t)(2 * ks + 1)) ^ row_x) << 4), 2 * ks + 1, mu_i,
                                  valid, zh + 4, zl + 4);
-                        if (!(dbg & 16)) {
-                            tmem_st8(t_lane + sa * 64u + 8u * ks, zh);
-                            tmem_st8(t_lane + sa * 64u + 32u + 8u * ks, zl);
-                        } else if (zh[0] == 0x12345678u && zl[3] == 0x9abcdef0u) {
-                            pent[0] = 0;      // (keeps the conversion alive)
-                        }
+                        tmem_st8(t_lane + sa * 64u + 8u * ks, zh);
+                        tmem_st8(t_lane + sa * 64u + 32u + 8u * ks, zl);
                     }
                     if (on_c) {
                         // 4 frames of a corner feature
@@ -1738,7 +1650,7 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                         *reinterpret_cast<uint2*>(dst) = make_uint2(zh[0], zh[1]);
                         *reinterpret_cast<uint2*>(dst + 2048u) = make_uint2(zl[0], zl[1]);
                     }
-                    if (!(dbg & 8)) tmem_st_wait();
+                    tmem_st_wait();
                 }
                 tc_fence_before();
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -1751,7 +1663,6 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 if (tt < 0) break;
             }
         }
-        if (warp == 4) report(3);
     } else {
         reg_inc<128>();
         // ---------------- epilogue (warps 12..19): TMEM -> fp32 registers -> partials -----------
@@ -1772,8 +1683,7 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 for (int j = 0; j < 16; ++j) acc[c][j] = 0.f;
             for (;;) {
                 const uint32_t ts = f & 1u, tu = f >> 1;
-                twait(bars + M2_TM_FULL + ts, tu & 1u, pw[0]);
-                ++p_tiles;
+                mbar_wait(bars + M2_TM_FULL + ts, tu & 1u);
                 tc_fence_after();
                 const int fl = gflag[ts];         // bit 0: the group holds data, bit 1: last group
                 const bool empty = (fl & 1) == 0;
@@ -1782,7 +1692,7 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                 const uint32_t tbase = tmem_base + ((quarter * 32u) << 16) + ts * acc_cols;
 #pragma unroll
                 for (int c = 0; c < 5; ++c) {
-                    if (!empty && c1_begin + c < c1_end && !(dbg & 4)) {
+                    if (!empty && c1_begin + c < c1_end) {
                         uint32_t v[16];
                         tmem_ld16(tbase + (uint32_t)(c1_begin + c) * 16, v);
                         tmem_ld_wait();
@@ -1819,7 +1729,6 @@ mstats_tc2_kernel(long long N, long long Npad, int n_mtiles, int tiles_per_chunk
                     out[(size_t)128 * G.N1 + (size_t)row * G.N2 + half * 16 + j] = 0.f;
             }
         }
-        if (warp == 12) report(4);
     }
     tc_fence_before();
     __syncthreads();
@@ -1922,10 +1831,6 @@ constexpr int TC_STAT_CHUNKS = 1184;
 // split-fp16 contraction itself (tools/time_mstep_real.py).  The FP64 path keeps 1e-16 per frame.
 constexpr float TC_TILE_FLOOR = 1e-8f;
 constexpr int TC_RESP_FORM1_MAX_K = 384;     // K x 64 frames of doubles in shared memory
-static float tile_floor_tc() {
-    const char* floor_env = getenv("KW_TC_TILE_FLOOR");      // experiments only
-    return floor_env != nullptr ? (float)atof(floor_env) : TC_TILE_FLOOR;
-}
 
 struct TcWorkspace {
     double* colpartial;
@@ -2056,8 +1961,7 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
     const long long n_tiles = (N + tc::TILE_M - 1) / tc::TILE_M;
     const long long Npad = resp_pad(N);
     // two components per MMA when both accumulators fit N <= 256 and TMEM (DP <= 96)
-    const char* g_env = getenv("KW_TC_G");                 // experiments only
-    const int G = (g_env != nullptr && atoi(g_env) == 1) ? 1 : ((DP <= 96 && K >= 2) ? 2 : 1);
+    const int G = (DP <= 96 && K >= 2) ? 2 : 1;
     const int KI = (K + G - 1) / G;
     tc::pack_l_kernel<<<dim3(KI * G, tc::PACK_L_SLICES), 256, 3 * sizeof(double) * DP, st>>>(K, D, DP, G, means, pc, aux,
                                                                 w.xinfo, w.bt, w.cst);
@@ -2067,41 +1971,23 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
     uint32_t cols = 32;
     while (cols < 2u * G * DP + DP + 16) cols <<= 1;  // two accumulator stages + the frame tile (hi+ones, lo)
     const int grid = (int)std::min<long long>(n_tiles, sms);
-    // when the epilogue frees an accumulator stage: measured on one box (tools/ab_release.py),
-    // early release takes 4 % off the EM E-step (one component per item, 27 MMAs: the MMA warp was
+    // When the epilogue frees an accumulator stage, measured on one B200 (commit 5844b33): early
+    // release takes 4 % off the EM E-step (one component per item, 27 MMAs: the MMA warp was
     // waiting for the stage) and adds 10 % to the conversion posterior (two components per item,
-    // a third of the MMA work: the MMAs running further ahead slow the epilogue's TMEM loads)
-    const char* lr_env = getenv("KW_TC_LATE_RELEASE");      // experiments only
-    const int late_release = lr_env != nullptr ? atoi(lr_env) : (G == 2 ? 1 : 0);
-    auto launch = [&](auto kern, unsigned long long* pd) -> int {
+    // a third of the MMA work: the MMAs running further ahead slow the epilogue's TMEM loads).
+    // The policy is a kernel argument rather than a constant of the instantiation: folded in at
+    // compile time, the late release is hoisted above the partial-sum additions, which frees the
+    // stage earlier and made the conversion posterior 9 % slower (B200, 1000 W).
+    const int late_release = G == 2 ? 1 : 0;
+    auto launch = [&](auto kern) -> int {
         KW_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)L.total));
         kern<<<grid, 576, L.total, st>>>(N, Npad, (int)n_tiles, K, D, DP, cols, w.xt, w.bt, w.cst,
-                                         resp, mode, mix, w.cand, 0.05, late_release, pd);
+                                         resp, mode, mix, w.cand, 0.05, late_release);
         return KW_OK;
     };
-#ifdef KW_TC_PROFILE_BUILD
-    // role profile (cycle counters of CTA 0): a separate instantiation, reading the clock
-    // serialises the issuing warp.  Build with -DKW_TC_PROFILE_BUILD to get it.
-    unsigned long long* prof_dev = nullptr;
-    cudaMalloc(&prof_dev, 16 * sizeof(unsigned long long));
-    rc = (G == 2) ? launch(tc::estep_tc_kernel<true, 2>, prof_dev)
-                  : launch(tc::estep_tc_kernel<true, 1>, prof_dev);
+    rc = (G == 2) ? launch(tc::estep_tc_kernel<2>) : launch(tc::estep_tc_kernel<1>);
     if (rc != KW_OK) return rc;
-    {
-        unsigned long long h[16];
-        cudaMemcpy(h, prof_dev, sizeof(h), cudaMemcpyDeviceToHost);
-        cudaFree(prof_dev);
-        fprintf(stderr, "[estep_tc cta0] mma: total %llu wait_tmem %llu wait_blo(+a) %llu wait_bhi %llu "
-                        "issue %llu | epi(part0): total %llu barriers %llu wait_tmfull %llu work %llu | "
-                        "epi(part3): barriers %llu wait %llu work %llu\n",
-                h[0], h[1], h[2], h[3], h[4], h[8], h[9], h[10], h[11], h[13], h[14], h[15]);
-    }
-#else
-    rc = (G == 2) ? launch(tc::estep_tc_kernel<false, 2>, nullptr)
-                  : launch(tc::estep_tc_kernel<false, 1>, nullptr);
-    if (rc != KW_OK) return rc;
-#endif
     KW_CUDA_CHECK(cudaGetLastError());
     if (mode == 1) {
         tc::refine_argmax_kernel<<<sms * 4, 256, 0, st>>>(N, D, X, pc, aux, mix, w.cand);
@@ -2124,7 +2010,7 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
         tc::lse_prep_kernel<64><<<lgrid, 128, sm, st>>>(
             N, Npad, K, resp, w.lse_partial, n_mt_pad, w.tflags, w.wts, w.tsum,
-            tile_floor_tc(), w.tiles_per_chunk, w.item_count);
+            TC_TILE_FLOOR, w.tiles_per_chunk, w.item_count);
     } else {
         tc::lse_kernel<<<lgrid, 128, 0, st>>>(N, Npad, K, resp, w.lse_partial);
     }
@@ -2167,33 +2053,19 @@ int mstats_tc(long long N, const double* X, int K, int D, const double* resp, co
         const long long warps = (long long)K * (n_mt_pad / 4);
         tc::mstats_tc_prep_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(
             N, resp_pad(N), w.n_mtiles, n_mt_pad, K, resp, w.tflags, w.wts, w.tsum,
-            tile_floor_tc(), w.tiles_per_chunk, w.item_count);
+            TC_TILE_FLOOR, w.tiles_per_chunk, w.item_count);
         KW_CUDA_CHECK(cudaGetLastError());
     }
     tc::mstats_tc_order_kernel<<<1, 1024, 0, st>>>(items, w.item_count, w.item_order);
     KW_CUDA_CHECK(cudaGetLastError());
-    // timing experiments only (tools/time_mstep.py): bits that switch parts of the kernel off
-    const char* dbg_env = getenv("KW_TC_MSWAP");
-    const int dbg = dbg_env != nullptr ? atoi(dbg_env) : 0;
     const tc::Mstep2Smem L2 = tc::mstep2_smem(DP);
     KW_CUDA_CHECK(cudaFuncSetAttribute(tc::mstats_tc2_kernel,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)L2.total));
     tc::mstats_tc2_kernel<<<grid, 640, L2.total, st>>>(
         N, resp_pad(N), w.n_mtiles, w.tiles_per_chunk, w.m_chunks, K, DP, w.xt, w.wts, w.mu32,
-        w.mpartial, w.item_counter, w.item_order, w.tflags, n_mt_pad, dbg);
+        w.mpartial, w.item_counter, w.item_order, w.tflags, n_mt_pad);
     KW_CUDA_CHECK(cudaGetLastError());
-    if (dbg & 16384) {
-        unsigned long long h[40];
-        KW_CUDA_CHECK(cudaStreamSynchronize(st));
-        KW_CUDA_CHECK(cudaMemcpyFromSymbol(h, tc::m2_prof, sizeof(h)));
-        const char* role[5] = {"producer  [B_EMPTY]", "mma       [B_FULL, TM_EMPTY, A_FULL]",
-                               "corner    [B_FULL, A_FULL]", "generator [B_FULL, A_EMPTY]",
-                               "epilogue  [TM_FULL]"};
-        for (int r = 0; r < 5; ++r)
-            fprintf(stderr, "[mstats_tc2 cta0] %-38s total %9llu clk, %5llu tiles, waits %9llu %9llu %9llu\n",
-                    role[r], h[r * 8], h[r * 8 + 1], h[r * 8 + 2], h[r * 8 + 3], h[r * 8 + 4]);
-    }
     tc::mstats_tc_reduce_kernel<<<dim3((G.partial_len + 256) / 256, K), 256, 0, st>>>(
         K, G.partial_len, w.m_chunks, w.mpartial, w.mraw);
     KW_CUDA_CHECK(cudaGetLastError());

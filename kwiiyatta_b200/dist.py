@@ -20,33 +20,12 @@ def shard_indices(sizes, world_size):
     return [np.array(sorted(s), dtype=np.int64) for s in shards]
 
 
-def allreduce_stats(stats, group=None, n_components=None, dim=None, exchange_form=False):
+def allreduce_stats(stats, group=None):
     """In-place sum of a statistics vector over the ranks of ``group`` (no-op when
-    torch.distributed is not initialised or the world has one rank).
-
-    ``exchange_form`` (CUDA vector with its layout given by ``n_components``, ``dim``): only
-    n_k, the first moments and the upper triangle of the symmetric second moments travel -- half
-    the bytes (kw_gmm_stats_pack / kw_gmm_stats_unpack).  Off by default: over NVLink the full
-    10.7 MB vector (K = 64, D = 144) is reduced in 48 us, the packed one in 56 us including the
-    two copy kernels (tools/time_allreduce.py, 2 x B200) -- the exchange is latency bound there,
-    so halving the bytes buys nothing; it is for links where bandwidth is the limit."""
+    torch.distributed is not initialised or the world has one rank)."""
     import torch.distributed as dist
-    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
-        return stats
-    if not exchange_form or n_components is None or dim is None or not stats.is_cuda:
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
         dist.all_reduce(stats, group=group)
-        return stats
-    import torch
-    from . import _lib
-    lib = _lib.lib()
-    packed = torch.empty(lib.kw_gmm_stats_packed_len(n_components, dim), dtype=torch.float64,
-                         device=stats.device)
-    stream = torch.cuda.current_stream(stats.device).cuda_stream
-    _lib.check(lib.kw_gmm_stats_pack(n_components, dim, stats.data_ptr(), packed.data_ptr(),
-                                     stream), 'kw_gmm_stats_pack')
-    dist.all_reduce(packed, group=group)
-    _lib.check(lib.kw_gmm_stats_unpack(n_components, dim, packed.data_ptr(), stats.data_ptr(),
-                                       stream), 'kw_gmm_stats_unpack')
     return stats
 
 

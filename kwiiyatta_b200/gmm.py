@@ -104,9 +104,6 @@ class GaussianMixture:
         self._x_used = None
         self._iters_done = 0
         self._resp_log = False      # `_resp` holds log-probabilities (see _estep)
-        # per-stage precision (diagnostics: tools/tc_error_split.py); a precision-1 workspace
-        # also holds what the FP64 kernels need
-        self._precision_e = self._precision_m = self.precision
 
     # ------------------------------------------------------------------ device plumbing
     def _alloc(self, torch, n, d, dev):
@@ -168,12 +165,12 @@ class GaussianMixture:
         responsibilities themselves are never written (kw_gmm_estep resp_form 1)."""
         x = self._frames(x)
         n, d = x.shape
-        self._resp_log = (bool(for_mstep) and self._precision_e == 1 and self._precision_m == 1
+        self._resp_log = (bool(for_mstep) and self.precision == 1
                           and self.n_components <= RESP_FORM1_MAX_COMPONENTS)
         rc = _lib.lib().kw_gmm_estep(
             n, x.data_ptr(), self.n_components, d, self._means[self._cur].data_ptr(),
             self._pc.data_ptr(), self._aux.data_ptr(), self._resp.data_ptr(),
-            self._stats.data_ptr(), self._precision_e, int(self._resp_log),
+            self._stats.data_ptr(), self.precision, int(self._resp_log),
             self._ws.data_ptr(), self._ws_bytes, _lib.stream_ptr(torch))
         _lib.check(rc, 'kw_gmm_estep')
 
@@ -193,20 +190,14 @@ class GaussianMixture:
         n, d = x.shape
         rc = _lib.lib().kw_gmm_mstep_accumulate(
             n, x.data_ptr(), self.n_components, d, self._resp.data_ptr(), centres.data_ptr(),
-            self._stats.data_ptr(), self._precision_m, int(self._resp_log),
+            self._stats.data_ptr(), self.precision, int(self._resp_log),
             self._ws.data_ptr(), self._ws_bytes, _lib.stream_ptr(torch))
         _lib.check(rc, 'kw_gmm_mstep_accumulate')
-
-    # all-reduce the triangle-packed statistics instead of the full vector (see
-    # dist.allreduce_stats: slower over NVLink, for bandwidth-limited links)
-    exchange_form = False
 
     def _allreduce(self, torch):
         """The path's one exchange: sum of the statistics vector over the ranks."""
         from . import dist as kdist
-        k, d = self._means[self._cur].shape
-        kdist.allreduce_stats(self._stats, self.process_group, n_components=k, dim=d,
-                              exchange_form=self.exchange_form)
+        kdist.allreduce_stats(self._stats, self.process_group)
 
     def _finalize(self, torch, centres, weight_norm):
         k, d = centres.shape
@@ -276,7 +267,6 @@ class GaussianMixture:
             dist.all_reduce(count, group=self.process_group)
         if self.precision_request == 'auto':
             self.precision = resolve_precision('auto', int(count.item()), k, d)
-            self._precision_e = self._precision_m = self.precision
         self._alloc(torch, n, d, dev)
         self._x_src, self._x_used, self._iters_done = x, None, 0
         if self.verbose:
@@ -467,7 +457,7 @@ class GaussianMixture:
         self._stats = torch.zeros(lib.kw_gmm_stats_len(k, d), dtype=torch.float64,
                                   device=x.device)
         if self.precision < 0:      # 'auto' on a model that was loaded, not fitted: FP64 posteriors
-            self.precision = self._precision_e = self._precision_m = 0
+            self.precision = 0
         self._ws_bytes = lib.kw_gmm_workspace_bytes(n, k, d, self.precision)
         self._ws = torch.empty(max(self._ws_bytes, 1), dtype=torch.uint8, device=x.device)
         self._pack(torch, x)

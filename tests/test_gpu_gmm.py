@@ -147,34 +147,6 @@ def test_kmeans_initialised_fit_is_as_good_as_sklearns(cuda):
     assert inertia <= 1.02 * sk_inertia
 
 
-def test_statistics_exchange_form_round_trip(cuda):
-    """kw_gmm_stats_pack / kw_gmm_stats_unpack: what the ranks all-reduce (n_k, first moments,
-    upper triangle, tail) reproduces the symmetric statistics vector exactly."""
-    import torch
-    from kwiiyatta_b200 import _lib
-    lib = _lib.lib()
-    rng = np.random.default_rng(2)
-    for k, d in ((1, 1), (3, 5), (64, 144)):
-        sb = 1 + d + d * d
-        stats = np.empty(k * sb + 2)
-        for c in range(k):
-            a = rng.standard_normal((d, d))
-            stats[c * sb] = rng.uniform(1, 9)
-            stats[c * sb + 1:c * sb + 1 + d] = rng.standard_normal(d)
-            stats[c * sb + 1 + d:(c + 1) * sb] = (a + a.T).ravel()
-        stats[-2:] = [-123.5, 4567.0]
-        n_packed = lib.kw_gmm_stats_packed_len(k, d)
-        assert n_packed == k * (1 + d + d * (d + 1) // 2) + 2
-        dev = torch.from_numpy(stats).cuda()
-        packed = torch.empty(n_packed, dtype=torch.float64, device='cuda')
-        back = torch.zeros_like(dev)
-        stream = torch.cuda.current_stream().cuda_stream
-        _lib.check(lib.kw_gmm_stats_pack(k, d, dev.data_ptr(), packed.data_ptr(), stream), 'pack')
-        _lib.check(lib.kw_gmm_stats_unpack(k, d, packed.data_ptr(), back.data_ptr(), stream),
-                   'unpack')
-        assert np.array_equal(back.cpu().numpy(), stats)
-
-
 def test_tensor_core_mstep_tile_floor(cuda):
     """The tensor-core M-step leaves out, per component, the 64-frame tiles in which every
     responsibility is <= 1e-8 (include/kwiiyatta_b200.h, kw_gmm_mstep_accumulate).  What that

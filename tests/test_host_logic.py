@@ -23,7 +23,7 @@ def test_library_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(lib, name), f'{name} declared in the header but not exported'
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
-    assert lib.kw_abi_version() == 2
+    assert lib.kw_abi_version() == 3
     assert lib.kw_gmm_stats_len(64, 144) == 64 * (1 + 144 + 144 * 144) + 2
 
 

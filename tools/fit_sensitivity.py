@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """The bench's user-level fit (KMeans initialisation on the device, tol = 1e-3, max_iter = 100):
-final lower bound per precision / tile floor -- how far 100 iterations carry rounding-level
-differences of the M-step."""
+final lower bound per precision -- how far 100 iterations carry rounding-level differences of
+the M-step."""
 import os, sys, warnings
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -11,11 +11,7 @@ kw.hooks.bind(pad_silence=lambda f, n: f, feature=synth.feature, resample=synth.
 padded = [synth.make_padded_pair(i) for i in range(503)]
 x = kw.joint_array_from_pairs(padded, pad_silence=True, pad_len=synth.PAD_LEN)
 dev = torch.device('cuda', 0)
-for prec, floor in (('tc', None), ('tc', '1e-16'), ('tc', '1e-10'), ('fp64', None)):
-    if floor is None:
-        os.environ.pop('KW_TC_TILE_FLOOR', None)
-    else:
-        os.environ['KW_TC_TILE_FLOOR'] = floor
+for prec in ('tc', 'fp64'):
     conv = kw.B200GMMFeatureConverter(components=64, random_state=0, verbose=0, device=dev,
                                       precision=prec)
     with warnings.catch_warnings():
@@ -23,6 +19,6 @@ for prec, floor in (('tc', None), ('tc', '1e-16'), ('tc', '1e-10'), ('fp64', Non
         conv._train(x)
     g = conv.gmm
     lbs = np.asarray(g.lower_bounds_)
-    print(f'{prec} floor {floor}: n_iter {g.n_iter_} lower bound {g.lower_bound_:.6f}; after 1/10/50 '
+    print(f'{prec}: n_iter {g.n_iter_} lower bound {g.lower_bound_:.6f}; after 1/10/50 '
           f'iterations {lbs[0]:.6f} {lbs[9]:.6f} {lbs[49]:.6f}; smallest n_k '
           f'{g.weights_.min() * len(x):.1f}')

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """CUDA-event time of kw_gmm_mstep_accumulate on the dense synthetic workload of prof_stage.py
-(every tile carries weight for every component) -- for kernel experiments via KW_TC_MSWAP."""
+(every tile carries weight for every component).  KW_CLOCKS=1 also samples the SM clock, the
+power draw and the clock-event reasons with nvidia-smi over 1500 calls."""
 import os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -28,7 +29,7 @@ e0.record()
 for _ in range(5):
     gm._accumulate(torch, xd, cen)
 e1.record(); e1.synchronize()
-print(f'KW_TC_MSWAP={os.environ.get("KW_TC_MSWAP")}: mstep_accumulate {e0.elapsed_time(e1) / 5:.3f} ms (dense)')
+print(f'mstep_accumulate {e0.elapsed_time(e1) / 5:.3f} ms (dense)')
 if os.environ.get('KW_CLOCKS'):
     import subprocess, threading, time
     samples = []
