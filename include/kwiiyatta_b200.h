@@ -200,6 +200,46 @@ int kw_convert_batch(int n_utts, const int64_t* off_dev, int64_t total_frames, i
                      const double* prepared_dev, double* out_dev, int32_t* mix_dev,
                      int precision, void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* Global variance (GV; Toda, Black & Tokuda, IEEE TASLP 15(8), 2007; oracle/gv_ref.py).
+ *
+ * kw_gv_estimate: for the columns [col0, col0 + ncols) of the row-major (total_rows, ld) device
+ * matrix x_dev, cut into n_utts utterances by int64 row offsets off_dev[n_utts + 1]:
+ *   utt_var_dev (n_utts, ncols)  v = (1/T) sum_t (x_t - mean)^2 per utterance (0 where T = 0);
+ *   mean_dev, var_dev (ncols)    mu_v and sigma^2_v = population variance of v, over the
+ *                                utterances with T >= 1, sigma^2_v floored at 1e-12;
+ *   sums_dev (2 ncols + 1)       [ sum v | sum v^2 | number of utterances ] (may be NULL), to be
+ *                                summed over ranks and turned into mu_v, sigma^2_v by
+ *                                kw_gv_from_sums (sigma^2_v = sum v^2 / n - mu_v^2, floored).
+ * Every sum has a fixed order: the results are bitwise reproducible.
+ *
+ * kw_convert_gv_batch: kw_convert_batch followed by GV-considered generation per (utterance,
+ * static dim): variance scaling of the ML trajectory to mu_v (gv_iter = 0 stops there: the GV
+ * postfilter), then gv_iter steps of step-controlled diagonal-Newton ascent on
+ *   F(y) = w_traj (-1/2 y^T R y + y^T r) - w_gv 1/2 (v(y) - mu_v)^2 / sigma^2_v
+ * (R y = r the MLPG normal equations; w_traj > 0, w_gv >= 0).  gv_mean_dev / gv_var_dev
+ * (static_dim) are mu_v and sigma^2_v.  Diff mode (a `prepared` block made with diff = 1):
+ * static_src_dev points at the source static features, row stride static_ld (usually src_dev
+ * itself, static_ld = dim_half); GV then applies to source + output.  NULL = plain conversion.
+ * f_dev (n_utts, static_dim) receives the final F (of source + output in diff mode),
+ * accepted_dev (n_utts, static_dim) the number of accepted steps; either may be NULL.
+ * max_frames sizes the shared-memory staging (utterances above min(max_frames, 1024) frames are
+ * iterated in global memory).  Workspace: kw_convert_gv_workspace_bytes.
+ * ------------------------------------------------------------------------------------------ */
+int kw_gv_estimate(int n_utts, const int64_t* off_dev, int64_t total_rows, int ld, int col0,
+                   int ncols, const double* x_dev, double* utt_var_dev, double* sums_dev,
+                   double* mean_dev, double* var_dev, void* stream);
+int kw_gv_from_sums(int ncols, const double* sums_dev, double* mean_dev, double* var_dev,
+                    void* stream);
+size_t kw_convert_gv_workspace_bytes(int64_t total_frames, int n_components, int dim_half,
+                                     int precision);
+int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t total_frames, int max_frames,
+                        const double* src_dev, int n_components, int dim_half,
+                        const double* prepared_dev, const double* gv_mean_dev,
+                        const double* gv_var_dev, int gv_iter, double w_traj, double w_gv,
+                        const double* static_src_dev, int static_ld, double* out_dev,
+                        int32_t* mix_dev, double* f_dev, int32_t* accepted_dev, int precision,
+                        void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* Soft-posterior mapping without MLPG (nnmnkwii MLPGBase.transform; the mlpg=False branch of
  * kwiiyatta/converter/gmm.py:30-31): out (total, dim_half) = sum_m p(m|x) (mu_y + S_yx S_xx^-1 (x - mu_x)).
  * `prepared_dev` comes from kw_convert_prepare with the same dim_half. */

@@ -3,7 +3,8 @@
 Public surface mirrors the reference's (kwiiyatta/__init__.py:1-22) for this path: ``align`` (the
 type-dispatching one, kwiiyatta/align.py:7-19), ``align_even``, the dataset chain
 (``ParallelDataset`` ... ``align_dataset``), ``MelCepstrumConverter`` with the converter back-end
-``B200GMMFeatureConverter``, a ``fastdtw`` module and ``MLPG``.  See INTEGRATION.md.
+``B200GMMFeatureConverter``, a ``fastdtw`` module and ``MLPG``, plus global-variance
+(GV) conversion: ``estimate_gv`` and the ``gv`` options of ``MLPG`` and the converter.  See INTEGRATION.md.
 """
 import collections.abc
 
@@ -18,6 +19,7 @@ from .dataset import (AlignedDataset, Dataset, DeltaFeatureDataset, MapDataset,
                       joint_array_from_pairs, make_dataset_to_array, map_dataset)
 from .delta import DELTA_WINDOWS, delta_features
 from .gmm import B200GMMFeatureConverter, FeatureConverter, GaussianMixture
+from .gv import GlobalVariance, estimate_gv
 from .mlpg import MLPG
 
 name = 'kwiiyatta_b200'
@@ -53,4 +55,5 @@ __all__ = ['fastdtw', 'hooks', 'align', 'align_even', 'align_even_many', 'align_
            'MelCepstrumConverter', 'MelCepstrumFeatureConverter', 'DeltaFeatureConverter',
            'MapFeatureConverter', 'B200GMMFeatureConverter', 'FeatureConverter',
            'save_converter', 'load_converter', 'mc2b', 'mc2b_many',
-           'GaussianMixture', 'MLPG', 'DELTA_WINDOWS', 'delta_features']
+           'GaussianMixture', 'MLPG', 'DELTA_WINDOWS', 'delta_features',
+           'GlobalVariance', 'estimate_gv']

@@ -20,8 +20,10 @@ _POWER_MODES = {'binalize': 0, 'raw': 1, None: 2}
 def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vuv='voiced',
                         power='binalize', strict=True, radius=32, vuv_weight=9.0,
                         power_weight=9.4, power_pivot='max', power_threshold=1.636, device=None,
-                        return_paths=False):
-    """(N, 2 * (3 or 1) * order) float64 CUDA tensor of joint frames for ``pairs``."""
+                        return_paths=False, return_offsets=False):
+    """(N, 2 * (3 or 1) * order) float64 CUDA tensor of joint frames for ``pairs``.
+    ``return_offsets``: also the int64 CUDA tensor of row offsets (n + 1) of each pair's rows
+    after the zero-frame removal."""
     torch = _lib.require_cuda()
     lib = _lib.lib()
     dev = torch.device('cuda' if device is None else device)
@@ -36,7 +38,8 @@ def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vu
         pairs = [(pad(a, pad_len), pad(b, pad_len)) for a, b in pairs]
     n = len(pairs)
     if n == 0:
-        return torch.zeros((0, 0), dtype=torch.float64, device=dev)
+        empty = torch.zeros((0, 0), dtype=torch.float64, device=dev)
+        return (empty, torch.zeros(1, dtype=torch.int64, device=dev)) if return_offsets else empty
     sides = []
     for which in (0, 1):
         mceps, flags, thr = [], [], []
@@ -96,8 +99,16 @@ def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vu
                                      xm.data_ptr(), ym.data_ptr(), width, int(bool(use_delta)),
                                      out.data_ptr(), zero.data_ptr(), stream)
             _lib.check(rc, 'kw_joint_frames')
+            row_off = out_off
             if bool(zero.any()):                    # rare: silent frames inside an utterance
                 out = out[~zero.bool()].contiguous()
+                dropped = torch.zeros(total + 1, dtype=torch.int64, device=dev)
+                dropped[1:] = torch.cumsum(zero.long(), dim=0)
+                row_off = out_off - dropped[out_off]
+        else:
+            row_off = out_off
     if return_paths:
         return out, (res, sel_len, out_off)
+    if return_offsets:
+        return out, row_off
     return out

@@ -7,6 +7,8 @@
 //   D_t = diag(S_yy[m]) - diag(S_yx[m]) / diag(S_xx[m]) * diag(S_xy[m])   (per mixture table)
 //   y[:, d] = solve( W^T D^-1 W , W^T D^-1 E )  per static dim d, pentadiagonal SPD system,
 //   windows = kwiiyatta DELTA_WINDOWS (kwiiyatta/converter/delta.py:8-12).
+// Beyond the reference: global-variance (GV) statistics and GV-considered generation on the same
+// normal equations (kw_gv_estimate, kw_convert_gv_batch; restated in oracle/gv_ref.py).
 #include "common.cuh"
 
 namespace kw {
@@ -403,6 +405,269 @@ convert_mlpg_kernel(int n_utts, const int64_t* __restrict__ off, int sd, double*
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// Global variance (Toda, Black & Tokuda, IEEE TASLP 15(8), 2007; restated in oracle/gv_ref.py).
+//
+// kw_gv_estimate, one warp per (utterance, column): v = (1/T) sum_t (x_t - mean)^2 by two passes
+// (mean, then squared deviations), lane-strided partial sums and an xor-butterfly, so every sum
+// has one fixed order.  gv_reduce_kernel, one thread per column: mu_v, sigma^2_v over the
+// utterances with T >= 1 in utterance order, plus [sum v | sum v^2 | count] for an all-reduce.
+// (warp_sum's xor-butterfly leaves the same bits on every lane, so every lane takes the same
+// accept / reject branch below.)
+constexpr double GV_VAR_FLOOR = 1e-12;  // sigma^2_v floor: p = 1 / sigma^2_v stays finite
+
+__global__ void gv_utt_var_kernel(int n_utts, const int64_t* __restrict__ off, int ld, int col0,
+                                  int ncols, const double* __restrict__ x,
+                                  double* __restrict__ utt_var) {
+    const int warp = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (warp >= n_utts * ncols) return;
+    const int u = warp / ncols, c = warp - u * ncols;
+    const long long t0 = off[u];
+    const int T = (int)(off[u + 1] - t0);
+    const double* p = x + (size_t)t0 * ld + col0 + c;
+    double s = 0.0;
+    for (int t = lane; t < T; t += 32) s += p[(size_t)t * ld];
+    const double mean = T > 0 ? warp_sum(s) / T : 0.0;
+    double q = 0.0;
+    for (int t = lane; t < T; t += 32) {
+        const double e = p[(size_t)t * ld] - mean;
+        q += e * e;
+    }
+    q = warp_sum(q);
+    if (lane == 0) utt_var[(size_t)u * ncols + c] = T > 0 ? q / T : 0.0;
+}
+
+__global__ void gv_reduce_kernel(int n_utts, const int64_t* __restrict__ off, int ncols,
+                                 const double* __restrict__ utt_var, double* __restrict__ sums,
+                                 double* __restrict__ mean, double* __restrict__ var) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= ncols) return;
+    double s = 0.0, s2 = 0.0;
+    int n = 0;
+    for (int u = 0; u < n_utts; ++u) {
+        if (off[u + 1] <= off[u]) continue;
+        const double v = utt_var[(size_t)u * ncols + c];
+        s += v;
+        s2 += v * v;
+        ++n;
+    }
+    const double mu = n > 0 ? s / n : 0.0;
+    double q = 0.0;
+    for (int u = 0; u < n_utts; ++u) {
+        if (off[u + 1] <= off[u]) continue;
+        const double e = utt_var[(size_t)u * ncols + c] - mu;
+        q += e * e;
+    }
+    if (sums != nullptr) {
+        sums[c] = s;
+        sums[ncols + c] = s2;
+        if (c == 0) sums[2 * ncols] = n;
+    }
+    mean[c] = mu;
+    var[c] = fmax(n > 0 ? q / n : 0.0, GV_VAR_FLOOR);
+}
+
+// mu_v, sigma^2_v from [sum v | sum v^2 | count] summed over ranks.
+__global__ void gv_from_sums_kernel(int ncols, const double* __restrict__ sums,
+                                    double* __restrict__ mean, double* __restrict__ var) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= ncols) return;
+    const double n = sums[2 * ncols];
+    const double mu = n > 0 ? sums[c] / n : 0.0;
+    mean[c] = mu;
+    var[c] = fmax(n > 0 ? sums[ncols + c] / n - mu * mu : 0.0, GV_VAR_FLOOR);
+}
+
+// GV-considered generation, one warp per (utterance, static dim), on the normal equations the
+// band kernel built (R y = r: a = R[t][t], b = R[t][t+1], c = R[t][t+2]; the planes hold values
+// past the utterance's end for b and c, which are masked here) and the ML solution y0 in `out`:
+//   F(y) = w_traj (-1/2 y^T R y + y^T r) - w_gv 1/2 p (v(y) - mu_v)^2,   p = 1 / sigma^2_v
+//   y <- mean(y0) + sqrt(mu_v / v(y0)) (y0 - mean(y0))     (unless T < 2 or v(y0) = 0)
+//   gv_iter times: g = w_traj (r - R y) - w_gv p (v - mu_v) (2/T) (y - ybar),
+//     delta_t = w_traj R_tt + w_gv (2p/T^2) max(0, (T-1)(v - mu_v) + 2 (y_t - ybar)^2),
+//     d = step g / delta;  accept y + d (step *= 1.2) iff F(y + d) >= F(y), else step *= 0.5.
+// The test takes dF = F(y + d) - F(y) in closed form from d rather than as the difference of two
+// rounded values of F:
+//   dF = w_traj (d^T (r - R y) - 1/2 d^T R d) - w_gv 1/2 p dv (2 (v - mu_v) + dv),
+//   dv = (2/T) sum (y_t - ybar) d_t + (1/T) sum (d_t - dbar)^2,
+// and "dF >= 0" is read up to the rounding of the gradient it rests on:
+//   dF >= -tol,  tol = GV_ROUND (w_traj sum |d_t| (|r_t| + (|R| |y|)_t)
+//                                + w_gv p (v + mu_v) (2/T) sum |d_t| |y_t - ybar|).
+// Where y is stationary to rounding (T = 1 from the start: y0 is the optimum) r - R y is noise
+// of either sign or exactly zero, depending on the order of the operations; the tolerance makes
+// every such step F-neutral and accepted, so two correct implementations count the same steps.  Diff mode: the problem in z = s + y (r' = r + R s, z0 = y0 + s), y = z - s.
+// The arrays a, b, c, r, y and the step d live in shared memory when T <= GV_SMEM_FRAMES
+// (stride 1), otherwise in the band workspace, `out` and a step plane (stride sd).
+constexpr int GV_SMEM_FRAMES = 1024;  // 6 arrays x 1024 doubles = 48 KB per warp
+constexpr double GV_ROUND = 8.0 * 2.220446049250313e-16;  // 8 ulp-units of the gradient terms
+
+struct GvArgs {
+    const int64_t* off;
+    int n_utts, sd, gv_iter, smem_frames;
+    const double* mu;
+    const double* var;
+    double w_traj, w_gv;
+    const double* s;  // diff mode: static source, row stride s_ld; else nullptr
+    int s_ld;
+    double* band;     // [a | b | c | rhs], (total, sd) each
+    double* step;     // (total, sd) step plane for the global-memory branch
+    double* out;      // (total, sd): y0 in, y out
+    long long total;
+    double* f_out;    // (n_utts, sd) or nullptr
+    int32_t* acc_out; // (n_utts, sd) or nullptr
+};
+
+template <int STRIDE>  // 1: shared memory; 0: global memory, stride sd
+__device__ void gv_solve(const GvArgs& g, int u, int d, int T, double* A, double* B, double* C,
+                         double* R, double* Y, double* D, int gs) {
+    const int st = STRIDE == 1 ? 1 : gs;
+    const int lane = threadIdx.x & 31;
+    auto Ry = [&](const double* v, int t, double* mag = nullptr) {  // (R v)_t [, (|R| |v|)_t]
+        double p0 = A[(size_t)t * st] * v[(size_t)t * st];
+        double s = p0, m = fabs(p0);
+        auto add = [&](double r, double x) { s = fma(r, x, s); m = fma(fabs(r), fabs(x), m); };
+        if (t >= 1) add(B[(size_t)(t - 1) * st], v[(size_t)(t - 1) * st]);
+        if (t >= 2) add(C[(size_t)(t - 2) * st], v[(size_t)(t - 2) * st]);
+        if (t + 1 < T) add(B[(size_t)t * st], v[(size_t)(t + 1) * st]);
+        if (t + 2 < T) add(C[(size_t)t * st], v[(size_t)(t + 2) * st]);
+        if (mag != nullptr) *mag = m;
+        return s;
+    };
+    const double mu = g.mu[d], p = 1.0 / g.var[d], wt = g.w_traj, wg = g.w_gv;
+    const double invT = 1.0 / T;
+    if (g.s != nullptr) {  // r' = r + R s, z0 = y0 + s; D holds s meanwhile
+        const double* s = g.s + (size_t)g.off[u] * g.s_ld + d;
+        for (int t = lane; t < T; t += 32) D[(size_t)t * st] = s[(size_t)t * g.s_ld];
+        __syncwarp();
+        for (int t = lane; t < T; t += 32) {
+            R[(size_t)t * st] += Ry(D, t);
+            Y[(size_t)t * st] += D[(size_t)t * st];
+        }
+        __syncwarp();
+    }
+    auto moments = [&](double& mean, double& v) {
+        double s = 0.0;
+        for (int t = lane; t < T; t += 32) s += Y[(size_t)t * st];
+        mean = warp_sum(s) * invT;
+        double q = 0.0;
+        for (int t = lane; t < T; t += 32) {
+            const double e = Y[(size_t)t * st] - mean;
+            q = fma(e, e, q);
+        }
+        v = warp_sum(q) * invT;
+    };
+    double ybar, v;
+    moments(ybar, v);
+    if (T >= 2 && v > 0.0) {  // variance scaling: the postfilter and the start point
+        const double k = sqrt(mu / v);
+        for (int t = lane; t < T; t += 32) Y[(size_t)t * st] = ybar + k * (Y[(size_t)t * st] - ybar);
+        __syncwarp();
+        moments(ybar, v);
+    }
+    double step = 0.1;
+    int accepted = 0;
+    for (int it = 0; it < g.gv_iter; ++it) {
+        const double gvc = wg * p * (v - mu);          // w_gv p (v - mu)
+        double s_d = 0.0, s_dg = 0.0, s_yd = 0.0, s_et = 0.0, s_eg = 0.0;
+        for (int t = lane; t < T; t += 32) {
+            const double y = Y[(size_t)t * st], e = y - ybar;
+            double mag;
+            const double rt = R[(size_t)t * st];
+            const double gt = wt * (rt - Ry(Y, t, &mag));
+            const double grad = gt - gvc * (2.0 * invT) * e;
+            const double curv = wt * A[(size_t)t * st] +
+                                wg * (2.0 * p * invT * invT) * fmax(0.0, (T - 1) * (v - mu) + 2.0 * e * e);
+            const double dt = step * grad / curv;
+            D[(size_t)t * st] = dt;
+            s_d += dt;
+            s_dg = fma(dt, gt, s_dg);
+            s_yd = fma(e, dt, s_yd);
+            s_et = fma(fabs(dt), fabs(rt) + mag, s_et);
+            s_eg = fma(fabs(dt), fabs(e), s_eg);
+        }
+        s_d = warp_sum(s_d);
+        s_dg = warp_sum(s_dg);
+        s_yd = warp_sum(s_yd);
+        s_et = warp_sum(s_et);
+        s_eg = warp_sum(s_eg);
+        __syncwarp();
+        const double dbar = s_d * invT;
+        double s_dRd = 0.0, s_dd = 0.0;
+        for (int t = lane; t < T; t += 32) {
+            const double dt = D[(size_t)t * st], e = dt - dbar;
+            s_dRd = fma(dt, Ry(D, t), s_dRd);
+            s_dd = fma(e, e, s_dd);
+        }
+        s_dRd = warp_sum(s_dRd);
+        s_dd = warp_sum(s_dd);
+        const double dv = 2.0 * invT * s_yd + invT * s_dd;
+        const double dF = s_dg - 0.5 * wt * s_dRd - 0.5 * wg * p * dv * (2.0 * (v - mu) + dv);
+        const double tol = GV_ROUND * (wt * s_et + wg * p * (v + mu) * 2.0 * invT * s_eg);
+        if (dF >= -tol) {
+            for (int t = lane; t < T; t += 32) Y[(size_t)t * st] += D[(size_t)t * st];
+            __syncwarp();
+            moments(ybar, v);
+            step *= 1.2;
+            ++accepted;
+        } else {
+            step *= 0.5;
+        }
+        __syncwarp();
+    }
+    if (g.f_out != nullptr || g.acc_out != nullptr) {
+        double s_f = 0.0;
+        for (int t = lane; t < T; t += 32) {
+            const double y = Y[(size_t)t * st];
+            s_f = fma(y, R[(size_t)t * st] - 0.5 * Ry(Y, t), s_f);
+        }
+        s_f = warp_sum(s_f);
+        if (lane == 0) {
+            const double e = v - mu;
+            if (g.f_out != nullptr) g.f_out[(size_t)u * g.sd + d] = wt * s_f - 0.5 * wg * p * e * e;
+            if (g.acc_out != nullptr) g.acc_out[(size_t)u * g.sd + d] = accepted;
+        }
+    }
+    __syncwarp();
+    if (STRIDE == 1 || g.s != nullptr) {
+        const double* s = g.s != nullptr ? g.s + (size_t)g.off[u] * g.s_ld + d : nullptr;
+        double* o = g.out + (size_t)g.off[u] * g.sd + d;
+        for (int t = lane; t < T; t += 32)
+            o[(size_t)t * g.sd] = Y[(size_t)t * st] - (s != nullptr ? s[(size_t)t * g.s_ld] : 0.0);
+    }
+}
+
+__global__ void __launch_bounds__(32)
+convert_gv_kernel(GvArgs g) {
+    extern __shared__ double gsm[];
+    const int u = blockIdx.x / g.sd, d = blockIdx.x - u * g.sd;
+    const long long t0 = g.off[u];
+    const int T = (int)(g.off[u + 1] - t0);
+    if (T <= 0) return;
+    const int lane = threadIdx.x;
+    const size_t plane = (size_t)g.total * g.sd;
+    double* a = g.band + (size_t)t0 * g.sd + d;
+    if (T <= g.smem_frames) {
+        double* A = gsm;
+        double* B = A + T;
+        double* C = B + T;
+        double* R = C + T;
+        double* Y = R + T;
+        double* D = Y + T;
+        const double* y0 = g.out + (size_t)t0 * g.sd + d;
+        for (int t = lane; t < T; t += 32) {
+            const size_t o = (size_t)t * g.sd;
+            A[t] = a[o]; B[t] = a[plane + o]; C[t] = a[2 * plane + o]; R[t] = a[3 * plane + o];
+            Y[t] = y0[o];
+        }
+        __syncwarp();
+        gv_solve<1>(g, u, d, T, A, B, C, R, Y, D, 1);
+    } else {
+        gv_solve<0>(g, u, d, T, a, a + plane, a + 2 * plane, a + 3 * plane,
+                    g.out + (size_t)t0 * g.sd + d, g.step + (size_t)t0 * g.sd + d, g.sd);
+    }
+}
+
 struct ConvertWorkspace {
     int32_t* mix;
     int* counts;      // K
@@ -497,13 +762,30 @@ extern "C" size_t kw_convert_workspace_bytes(int64_t total_frames, int K, int Dh
     return b;
 }
 
+// Posterior, conditional means, normal equations and their solve into out_dev; `*wout` (may be
+// NULL) receives the workspace layout, whose E / mix / flags / band stay valid after the call.
+static int convert_run(int n_utts, const int64_t* off_dev, int64_t total, const double* src_dev,
+                       int K, int Dh, const double* prepared_dev, double* out_dev,
+                       int32_t* mix_dev, int precision, void* workspace_dev,
+                       size_t workspace_bytes, cudaStream_t st, ConvertWorkspace* wout);
+
+static const Windows kDeltaWindows = {{{0.0, 1.0, 0.0}, {-0.5, 0.0, 0.5}, {1.0, -2.0, 1.0}}};
+
 extern "C" int kw_convert_batch(int n_utts, const int64_t* off_dev, int64_t total, int max_frames,
                                 const double* src_dev, int K, int Dh, const double* prepared_dev,
                                 double* out_dev, int32_t* mix_dev, int precision,
                                 void* workspace_dev, size_t workspace_bytes, void* stream) {
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     (void)max_frames;
     if (n_utts == 0 || total == 0) return KW_OK;
+    return convert_run(n_utts, off_dev, total, src_dev, K, Dh, prepared_dev, out_dev, mix_dev,
+                       precision, workspace_dev, workspace_bytes,
+                       static_cast<cudaStream_t>(stream), nullptr);
+}
+
+static int convert_run(int n_utts, const int64_t* off_dev, int64_t total, const double* src_dev,
+                       int K, int Dh, const double* prepared_dev, double* out_dev,
+                       int32_t* mix_dev, int precision, void* workspace_dev,
+                       size_t workspace_bytes, cudaStream_t st, ConvertWorkspace* wout) {
     KW_REQUIRE(n_utts > 0 && total > 0 && K > 0, "kw_convert_batch: bad sizes");
     KW_REQUIRE(Dh % 3 == 0, "dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
     KW_REQUIRE(precision == 0 || precision == 1, "convert precision must be 0 or 1");
@@ -549,7 +831,7 @@ extern "C" int kw_convert_batch(int n_utts, const int64_t* off_dev, int64_t tota
         KW_CUDA_CHECK(cudaGetLastError());
     }
     {
-        Windows win = {{{0.0, 1.0, 0.0}, {-0.5, 0.0, 0.5}, {1.0, -2.0, 1.0}}};
+        const Windows win = kDeltaWindows;
         KW_CUDA_CHECK(cudaMemsetAsync(w.flags, 0, (size_t)total, st));
         convert_flags_kernel<<<(n_utts + 127) / 128, 128, 0, st>>>(n_utts, off_dev, w.flags);
         KW_CUDA_CHECK(cudaGetLastError());
@@ -565,5 +847,104 @@ extern "C" int kw_convert_batch(int n_utts, const int64_t* off_dev, int64_t tota
     if (mix_dev != nullptr)
         KW_CUDA_CHECK(cudaMemcpyAsync(mix_dev, w.mix, sizeof(int32_t) * total,
                                       cudaMemcpyDeviceToDevice, st));
+    if (wout != nullptr) *wout = w;
+    return KW_OK;
+}
+
+extern "C" int kw_gv_estimate(int n_utts, const int64_t* off_dev, int64_t total_rows, int ld,
+                              int col0, int ncols, const double* x_dev, double* utt_var_dev,
+                              double* sums_dev, double* mean_dev, double* var_dev, void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    KW_REQUIRE(n_utts > 0 && ncols > 0 && col0 >= 0 && col0 + ncols <= ld && total_rows >= 0,
+               "kw_gv_estimate: bad sizes");
+    KW_REQUIRE((long long)n_utts * ncols < (1LL << 26), "kw_gv_estimate: too many utterances");
+    const long long threads = 32LL * n_utts * ncols;
+    gv_utt_var_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(
+        n_utts, off_dev, ld, col0, ncols, x_dev, utt_var_dev);
+    KW_CUDA_CHECK(cudaGetLastError());
+    gv_reduce_kernel<<<(ncols + 63) / 64, 64, 0, st>>>(n_utts, off_dev, ncols, utt_var_dev,
+                                                      sums_dev, mean_dev, var_dev);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+extern "C" int kw_gv_from_sums(int ncols, const double* sums_dev, double* mean_dev,
+                               double* var_dev, void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    KW_REQUIRE(ncols > 0, "kw_gv_from_sums: bad sizes");
+    gv_from_sums_kernel<<<(ncols + 63) / 64, 64, 0, st>>>(ncols, sums_dev, mean_dev, var_dev);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+// GV workspace: [ step plane (total, sd) | the kw_convert_batch workspace ].
+static size_t gv_step_bytes(int64_t total, int sd) {
+    return align_up(sizeof(double) * (size_t)total * sd, 256);
+}
+
+extern "C" size_t kw_convert_gv_workspace_bytes(int64_t total_frames, int K, int Dh,
+                                                int precision) {
+    return gv_step_bytes(total_frames, Dh / 3) +
+           kw_convert_workspace_bytes(total_frames, K, Dh, precision);
+}
+
+extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t total,
+                                   int max_frames, const double* src_dev, int K, int Dh,
+                                   const double* prepared_dev, const double* gv_mean_dev,
+                                   const double* gv_var_dev, int gv_iter, double w_traj,
+                                   double w_gv, const double* static_src_dev, int static_ld,
+                                   double* out_dev, int32_t* mix_dev, double* f_dev,
+                                   int32_t* accepted_dev, int precision, void* workspace_dev,
+                                   size_t workspace_bytes, void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (n_utts == 0 || total == 0) return KW_OK;
+    KW_REQUIRE(Dh % 3 == 0, "dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
+    KW_REQUIRE(gv_iter >= 0 && w_traj > 0.0 && w_gv >= 0.0,
+               "kw_convert_gv_batch: need gv_iter >= 0, w_traj > 0, w_gv >= 0");
+    const int sd = Dh / 3;
+    KW_REQUIRE(static_src_dev == nullptr || static_ld >= sd, "static_ld %d < static_dim %d",
+               static_ld, sd);
+    KW_REQUIRE((long long)n_utts * sd < 2147483647LL, "too many utterances for one batch");
+    const size_t sbytes = gv_step_bytes(total, sd);
+    if (kw_convert_gv_workspace_bytes(total, K, Dh, precision) > workspace_bytes) {
+        set_error("GV convert workspace too small");
+        return KW_ERR_WORKSPACE;
+    }
+    ConvertWorkspace w;
+    int rc = convert_run(n_utts, off_dev, total, src_dev, K, Dh, prepared_dev, out_dev, mix_dev,
+                         precision, static_cast<char*>(workspace_dev) + sbytes,
+                         workspace_bytes - sbytes, st, &w);
+    if (rc != KW_OK) return rc;
+    // convert_mlpg_kernel factored the bands in place: rebuild them (the band kernel is a pure
+    // function of E, the mixture sequence and the flags, all still in the workspace), which moves
+    // the same bytes as a saved copy would and keeps the workspace at one band set
+    PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    const long long cells = total * sd;
+    convert_band_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
+        total, sd, Dh, w.E, w.mix, v.var, w.flags, kDeltaWindows, w.band);
+    KW_CUDA_CHECK(cudaGetLastError());
+    GvArgs g;
+    g.off = off_dev;
+    g.n_utts = n_utts;
+    g.sd = sd;
+    g.gv_iter = gv_iter;
+    g.smem_frames = max(1, min(max_frames, GV_SMEM_FRAMES));
+    g.mu = gv_mean_dev;
+    g.var = gv_var_dev;
+    g.w_traj = w_traj;
+    g.w_gv = w_gv;
+    g.s = static_src_dev;
+    g.s_ld = static_ld;
+    g.band = w.band;
+    g.step = static_cast<double*>(workspace_dev);
+    g.out = out_dev;
+    g.total = total;
+    g.f_out = f_dev;
+    g.acc_out = accepted_dev;
+    const size_t smem = sizeof(double) * 6 * (size_t)g.smem_frames;
+    KW_CUDA_CHECK(cudaFuncSetAttribute(convert_gv_kernel,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    convert_gv_kernel<<<(unsigned)(n_utts * sd), 32, smem, st>>>(g);
+    KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }

@@ -280,11 +280,33 @@ def _assemble_on_device(chain, keys):
              'power_weight', 'power_pivot', 'power_threshold')
     if any(k not in known for k in aligned.kwargs):
         return None
-    x = assemble.joint_frames_device(pairs, use_delta=delta is not None, **aligned.kwargs)
+    x, offsets = assemble.joint_frames_device(pairs, use_delta=delta is not None,
+                                              return_offsets=True, **aligned.kwargs)
     mcep.order, mcep.fs = order, fs               # what the per-item path would have recorded
     if delta is not None:
         delta.frame_period = next(iter(periods))
-    return x
+    return x, offsets
+
+
+def _dataset_to_array_with_offsets(dataset, keys=None, device_resident=False):
+    """``make_dataset_to_array`` plus the int64 row offsets (n_keys + 1) of each key's rows in
+    it: a numpy array with the host matrix, a CUDA tensor with the device-assembled one."""
+    if keys is None:
+        keys = sorted(dataset.keys())
+    keys = list(keys)
+    if device_resident and keys:
+        chain = _device_chain(dataset)
+        if chain is not None:
+            res = _assemble_on_device(chain, keys)
+            if res is not None:
+                return res
+    if hasattr(dataset, 'get_many'):
+        items = dataset.get_many(keys)
+    else:
+        items = [dataset[key] for key in keys]
+    rows = [remove_zeros_frames(np.hstack(d) if isinstance(d, tuple) else d) for d in items]
+    offsets = np.concatenate(([0], np.cumsum([len(r) for r in rows]))).astype(np.int64)
+    return (np.concatenate(rows) if rows else None), offsets
 
 
 def make_dataset_to_array(dataset, keys=None, device_resident=False):
@@ -293,21 +315,7 @@ def make_dataset_to_array(dataset, keys=None, device_resident=False):
     key list goes down the chain in one request.  ``device_resident``: for the standard training
     chain return the matrix as a CUDA tensor assembled on the device
     (kwiiyatta_b200.assemble), bit-identical to the host result."""
-    if keys is None:
-        keys = sorted(dataset.keys())
-    keys = list(keys)
-    if device_resident and keys:
-        chain = _device_chain(dataset)
-        if chain is not None:
-            x = _assemble_on_device(chain, keys)
-            if x is not None:
-                return x
-    if hasattr(dataset, 'get_many'):
-        items = dataset.get_many(keys)
-    else:
-        items = [dataset[key] for key in keys]
-    rows = [remove_zeros_frames(np.hstack(d) if isinstance(d, tuple) else d) for d in items]
-    return np.concatenate(rows) if rows else None
+    return _dataset_to_array_with_offsets(dataset, keys, device_resident)[0]
 
 
 def joint_array_from_pairs(pairs, use_delta=True, pad_silence=True, pad_len=100,

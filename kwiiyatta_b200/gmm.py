@@ -500,9 +500,49 @@ class B200GMMFeatureConverter(FeatureConverter):
     """Drop-in for GMMFeatureConverter (kwiiyatta/converter/gmm.py:8-34)."""
     accepts_device_array = True
 
-    def __init__(self, components=64, max_iter=100, random_state=None, **kwargs):
+    def __init__(self, components=64, max_iter=100, random_state=None, gv=False, **kwargs):
+        """``gv=True``: ``train`` also estimates the global-variance (GV) statistics that
+        ``convert(..., gv=True)`` uses (see ``train``)."""
         super().__init__()
+        self.train_gv = bool(gv)
+        self._gv = None
         self.init_gmm(components, max_iter, random_state, **kwargs)
+
+    @property
+    def gv(self):
+        """GV statistics (kwiiyatta_b200.gv.GlobalVariance) or None.  Assign the result of
+        ``kwiiyatta_b200.estimate_gv`` to use statistics of other data, e.g. of natural target
+        utterances."""
+        return self._gv
+
+    @gv.setter
+    def gv(self, value):
+        from .gv import as_gv
+        self._gv = None if value is None else as_gv(value)
+        self._paramgen = {k: p for k, p in self._paramgen.items() if not k[2]}
+
+    def train(self, dataset, keys, **kwargs):
+        """With ``gv=True`` at construction, the GV statistics come from the TARGET static
+        columns [Dh, Dh + static_dim) of each key's rows of the training matrix: the aligned
+        target frames without zero frames, exactly what the model is trained on (estimated on the
+        device before the fit)."""
+        if not self.train_gv:
+            return super().train(dataset, keys, **kwargs)
+        from . import dataset as ds
+        from .gv import estimate_gv
+        x, offsets = ds._dataset_to_array_with_offsets(dataset, keys, device_resident=True)
+        if x is None:
+            raise ValueError('no training data')
+        dh = x.shape[1] // 2
+        gv = estimate_gv((_as_device(x, _lib.require_cuda(), self._gv_device()), offsets),
+                         columns=(dh, dh // len(DELTA_WINDOWS)),
+                         process_group=self.gmm.process_group)
+        self._train(x, **kwargs)
+        self.gv = gv
+
+    def _gv_device(self):
+        torch = _lib.require_cuda()
+        return torch.device('cuda' if self.gmm.device is None else self.gmm.device)
 
     def init_gmm(self, components, max_iter=100, random_state=None, **kwargs):
         if 'verbose' not in kwargs:
@@ -527,7 +567,8 @@ class B200GMMFeatureConverter(FeatureConverter):
                 'reg_covar': g.reg_covar,
                 'random_state': -1 if g.random_state is None else g.random_state,
                 'n_iter': getattr(g, 'n_iter_', 0), 'converged': getattr(g, 'converged_', False),
-                'lower_bound': getattr(g, 'lower_bound_', float('nan'))}
+                'lower_bound': getattr(g, 'lower_bound_', float('nan')),
+                **({} if self._gv is None else {'gv_mean': self._gv.mean, 'gv_var': self._gv.var})}
 
     def load_state_dict(self, state):
         g = self.gmm
@@ -540,6 +581,7 @@ class B200GMMFeatureConverter(FeatureConverter):
         g.n_iter_, g.converged_ = int(state['n_iter']), bool(state['converged'])
         g.lower_bound_ = float(state['lower_bound'])
         self._paramgen = {}
+        self.gv = (state['gv_mean'], state['gv_var']) if 'gv_mean' in state else None
         return self
 
     def save(self, path):
@@ -552,20 +594,28 @@ class B200GMMFeatureConverter(FeatureConverter):
         conv = cls(components=int(state['n_components']), verbose=0, **kwargs)
         return conv.load_state_dict(state)
 
-    def _mlpg(self, diff, mlpg=True):
+    def _mlpg(self, diff, mlpg=True, gv=False):
         from .mlpg import MLPG
-        key = (bool(diff), bool(mlpg))
+        key = (bool(diff), bool(mlpg), bool(gv))
+        if gv and not mlpg:
+            raise ValueError('GV is defined for MLPG conversion only (mlpg=True)')
+        if gv and self._gv is None:
+            raise ValueError('gv=True needs GV statistics: construct with gv=True and train, '
+                             'or assign estimate_gv(...) to .gv')
         if key not in self._paramgen:
             windows = DELTA_WINDOWS if mlpg else DELTA_WINDOWS[0:1]   # gmm.py:29-31
             # 'auto': the tensor-core posterior re-checks near-ties in FP64, so the mixture
             # sequence (and with it the FP64 MLPG output) is the FP64 one at any size
             self._paramgen[key] = MLPG(self.gmm, windows=windows, diff=diff,
-                                       precision=self.gmm.precision_request)
+                                       precision=self.gmm.precision_request,
+                                       gv=self._gv if gv else None)
         return self._paramgen[key]
 
-    def convert(self, feature, mlpg=True, diff=False):
-        return self._mlpg(diff, mlpg).transform(feature)
+    def convert(self, feature, mlpg=True, diff=False, gv=False):
+        """``gv=True``: GV-considered MLPG with the statistics in ``.gv`` (in diff mode the GV
+        is that of source + output, which is what the MLSA filter makes heard)."""
+        return self._mlpg(diff, mlpg, gv).transform(feature)
 
-    def convert_many(self, features, diff=False):
+    def convert_many(self, features, diff=False, gv=False):
         """Batched ``convert`` over a list of (T_i, 72) arrays."""
-        return self._mlpg(diff).transform_many(features)
+        return self._mlpg(diff, True, gv).transform_many(features)

@@ -1,5 +1,5 @@
 """Posterior + MLPG on the B200 (nnmnkwii.baseline.gmm.MLPG as used at
-kwiiyatta/converter/gmm.py:28-34)."""
+kwiiyatta/converter/gmm.py:28-34), optionally with global variance (``gv=``; kwiiyatta_b200.gv)."""
 import numpy as np
 
 from . import _lib
@@ -16,14 +16,41 @@ class MLPG:
     here; the reference rebuilds it on every convert call (kwiiyatta/converter/gmm.py:32)."""
 
     def __init__(self, gmm, windows=None, swap=False, diff=False, precision='auto',
-                 device=None):
+                 device=None, gv=None, gv_iter=20, gv_weights=(1.0, 1.0)):
         torch = _lib.require_cuda()
         self._dev = torch.device('cuda' if device is None else device)
         if self._dev.index is not None:
             with torch.cuda.device(self._dev):
                 self._setup(torch, gmm, windows, swap, diff, precision)
+                self._setup_gv(torch, gv, gv_iter, gv_weights)
         else:
             self._setup(torch, gmm, windows, swap, diff, precision)
+            self._setup_gv(torch, gv, gv_iter, gv_weights)
+
+    def _setup_gv(self, torch, gv, gv_iter, gv_weights):
+        """``gv``: GV statistics (a kwiiyatta_b200.gv.GlobalVariance, a dict with ``mean`` /
+        ``var`` or a (mean, var) pair, one value per static dimension) -> every transform
+        generates the GV-considered trajectory: the ML trajectory scaled to the GV mean, then
+        ``gv_iter`` ascent steps on w_traj * (trajectory log-likelihood) + w_gv * (GV
+        log-likelihood), ``gv_weights = (w_traj, w_gv)``.  ``gv_iter = 0`` is the
+        variance-scaling postfilter.  In diff mode the GV is that of source + output."""
+        self.gv = None
+        if gv is None:
+            return
+        from .gv import as_gv
+        if len(self.windows) == 1:
+            raise ValueError('GV is defined for MLPG trajectories only (not with a single '
+                             'static window)')
+        gv = as_gv(gv)
+        if len(gv) != self.static_dim:
+            raise ValueError(f'GV statistics have {len(gv)} dimensions, expected '
+                             f'{self.static_dim}')
+        w_traj, w_gv = (float(w) for w in gv_weights)
+        if int(gv_iter) < 0 or not w_traj > 0 or not w_gv >= 0:
+            raise ValueError('need gv_iter >= 0, w_traj > 0 and w_gv >= 0')
+        self.gv, self.gv_iter, self.gv_weights = gv, int(gv_iter), (w_traj, w_gv)
+        self._gv_mean = torch.from_numpy(gv.mean).to(self._dev)
+        self._gv_var = torch.from_numpy(gv.var).to(self._dev)
 
     def _setup(self, torch, gmm, windows, swap, diff, precision):
         if windows is None:
@@ -65,24 +92,53 @@ class MLPG:
             raise np.linalg.LinAlgError('source covariance of some mixture is not positive '
                                         'definite')
 
-    @_on_own_device
-    def transform_device(self, src_dev, offsets_dev, n_utts, max_frames, return_mix=False):
-        """src_dev (sum T, dim_half) float64 CUDA tensor, offsets int64 (n_utts + 1)."""
-        torch = _lib.require_cuda()
+    def _launch(self, torch, n_utts, off_dev, total, max_frames, src, out, mix, stream,
+                gv_f=None, gv_accepted=None):
+        """kw_convert_batch, or kw_convert_gv_batch when GV statistics are set, on device
+        tensors (``src`` (total, dim_half), ``out`` (total, static_dim))."""
         lib = _lib.lib()
+        k, dh = self.num_mixtures, self.dim_half
+        if self.gv is None:
+            ws_bytes = lib.kw_convert_workspace_bytes(total, k, dh, self.precision)
+            ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=src.device)
+            rc = lib.kw_convert_batch(n_utts, off_dev.data_ptr(), total, int(max_frames),
+                                      src.data_ptr(), k, dh, self._prepared.data_ptr(),
+                                      out.data_ptr(), _lib.ptr(mix), self.precision,
+                                      ws.data_ptr(), ws_bytes, stream)
+            _lib.check(rc, 'kw_convert_batch')
+            return
+        ws_bytes = lib.kw_convert_gv_workspace_bytes(total, k, dh, self.precision)
+        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=src.device)
+        rc = lib.kw_convert_gv_batch(
+            n_utts, off_dev.data_ptr(), total, int(max_frames), src.data_ptr(), k, dh,
+            self._prepared.data_ptr(), self._gv_mean.data_ptr(), self._gv_var.data_ptr(),
+            self.gv_iter, self.gv_weights[0], self.gv_weights[1],
+            src.data_ptr() if self.diff else None, dh, out.data_ptr(), _lib.ptr(mix),
+            _lib.ptr(gv_f), _lib.ptr(gv_accepted), self.precision, ws.data_ptr(), ws_bytes,
+            stream)
+        _lib.check(rc, 'kw_convert_gv_batch')
+
+    @_on_own_device
+    def transform_device(self, src_dev, offsets_dev, n_utts, max_frames, return_mix=False,
+                         return_gv_info=False):
+        """src_dev (sum T, dim_half) float64 CUDA tensor, offsets int64 (n_utts + 1).
+        ``return_gv_info`` (with GV): also the final objective F and the number of accepted
+        ascent steps per (utterance, static dim), as (n_utts, static_dim) tensors."""
+        torch = _lib.require_cuda()
         total = src_dev.shape[0]
-        out = torch.empty((total, self.static_dim), dtype=torch.float64, device=src_dev.device)
-        mix = torch.empty(total, dtype=torch.int32, device=src_dev.device) if return_mix else None
-        ws_bytes = lib.kw_convert_workspace_bytes(total, self.num_mixtures, self.dim_half,
-                                                  self.precision)
-        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=src_dev.device)
-        rc = lib.kw_convert_batch(n_utts, offsets_dev.data_ptr(), total, int(max_frames),
-                                  src_dev.data_ptr(), self.num_mixtures, self.dim_half,
-                                  self._prepared.data_ptr(), out.data_ptr(), _lib.ptr(mix),
-                                  self.precision, ws.data_ptr(), ws_bytes,
-                                  _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_convert_batch')
-        return (out, mix) if return_mix else out
+        dev = src_dev.device
+        out = torch.empty((total, self.static_dim), dtype=torch.float64, device=dev)
+        mix = torch.empty(total, dtype=torch.int32, device=dev) if return_mix else None
+        info = None
+        if return_gv_info:
+            if self.gv is None:
+                raise ValueError('return_gv_info needs GV statistics')
+            info = (torch.zeros((n_utts, self.static_dim), dtype=torch.float64, device=dev),
+                    torch.zeros((n_utts, self.static_dim), dtype=torch.int32, device=dev))
+        self._launch(torch, n_utts, offsets_dev, total, max_frames, src_dev, out, mix,
+                     _lib.stream_ptr(torch), *(info or ()))
+        res = (out,) + ((mix,) if return_mix else ()) + ((info,) if return_gv_info else ())
+        return res if len(res) > 1 else out
 
     CHUNK_FRAMES = 65536       # frames per pipeline chunk (36 MB in, 12 MB out at Dh = 72)
 
@@ -164,7 +220,6 @@ class MLPG:
         s_in.wait_event(start)            # buffers may still be in use by the previous call
         s_out.wait_event(start)
         ev_comp, ev_d2h = {}, {}
-        lib = _lib.lib()
         keep = []
         for c, (a, b) in enumerate(chunks):
             r0, r1 = int(rows[a]), int(rows[b])
@@ -181,14 +236,8 @@ class MLPG:
             if c >= 2:
                 compute.wait_event(ev_d2h[c - 2])        # device output buffer copied down
             chunk_in, chunk_out = bufs['din'][c & 1][:n_c], bufs['dout'][c & 1][:n_c]
-            ws_bytes = lib.kw_convert_workspace_bytes(n_c, self.num_mixtures, dh, self.precision)
-            ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
-            rc = lib.kw_convert_batch(b - a, off_dev.data_ptr(), n_c, int(lens[a:b].max()),
-                                      chunk_in.data_ptr(), self.num_mixtures, dh,
-                                      self._prepared.data_ptr(), chunk_out.data_ptr(), None,
-                                      self.precision, ws.data_ptr(), ws_bytes,
-                                      compute.cuda_stream)
-            _lib.check(rc, 'kw_convert_batch')
+            self._launch(torch, b - a, off_dev, n_c, int(lens[a:b].max()), chunk_in, chunk_out,
+                         None, compute.cuda_stream)
             off_dev.record_stream(compute)
             keep.append(off)
             ev_comp[c] = torch.cuda.Event()
