@@ -2,9 +2,10 @@
 
 There is no CPU fallback: if the library is missing or a call fails, this raises."""
 import ctypes
+import math
+import os
 
 import numpy as np
-import os
 
 from . import build as _build
 
@@ -112,6 +113,23 @@ def stream_ptr(torch):
     return torch.cuda.current_stream().cuda_stream
 
 
+def call(name, *args):
+    """``lib().<name>(*args)`` for an entry point that returns a status: torch tensors, numpy
+    arrays and None go in as pointers (``ptr``), everything else as it is, for ctypes to convert
+    and range-check; a non-zero status raises (``check``).  The size queries
+    (``kw_*_len``, ``kw_*_workspace_bytes``) return sizes and are called on ``lib()``."""
+    rc = getattr(lib(), name)(*[
+        ptr(a) if a is None or isinstance(a, np.ndarray) or hasattr(a, 'data_ptr') else a
+        for a in args])
+    check(rc, name)
+
+
+def workspace(nbytes, device):
+    """Device workspace of ``nbytes`` bytes (at least one, so that it has an address)."""
+    import torch
+    return torch.empty(max(nbytes, 1), dtype=torch.uint8, device=device)
+
+
 def device_guard(device_of):
     """Decorator: run the call with the CUDA device of its data current, so the C-ABI launches
     (which go to ``torch.cuda.current_stream()`` of the CURRENT device) land on the GPU that
@@ -135,14 +153,53 @@ def device_guard(device_of):
     return wrap
 
 
-# Pinned staging buffers (and the side streams of the packed host APIs) kept between calls: pinning
-# is far more expensive than the copy, and the caching allocator keeps one pool per stream.  This
-# is a per-process cache of the Python host layer (the C ABI itself keeps no state); calls that
-# share a slot must not run concurrently from several host threads.
-# slot -> (tensor, event of the last copy that read it) or a dict of buffers
+# Host buffers and side streams of the host APIs, kept between calls per (slot, device): pinning
+# costs far more than the copies, and the caching allocator keeps one pool per stream.  This is a
+# per-process cache of the Python host layer (the C ABI itself keeps no state); calls that share
+# a slot must not run concurrently from several host threads.
+# (slot, device) -> (pinned tensor, event of the last copy that read it) or a dict (``staging``)
 _STAGING = {}
 _GATHER_THREADS = max(4, min(32, os.cpu_count() or 8))
 _POOL = None
+
+
+def pinned(slot, dev, shape, dtype):
+    """Pinned host tensor of ``shape`` and ``dtype``, kept for (``slot``, ``dev``) between calls
+    and reallocated only when too small.  The next call for the slot hands out the same memory,
+    so every caller keeps one of these rules:
+
+    * an asynchronous copy that may still read the buffer when the caller returns is recorded
+      with ``pinned_in_flight``; the next call for the slot waits for it (``gather_to_device``);
+    * what the caller returns from the buffer is copied out of it, never a view of it
+      (``fastdtw_batch_packed``);
+    * the caller synchronises before it returns (``MLPG.transform_many``, whose
+      ``transform_packed`` does)."""
+    key = (slot, str(dev))
+    numel = math.prod(shape)
+    buf, ev = _STAGING.get(key, (None, None))
+    if buf is None or buf.numel() < numel or buf.dtype != dtype:
+        import torch
+        buf, ev = torch.empty(max(numel, 1), dtype=dtype).pin_memory(), None
+    if ev is not None:
+        ev.synchronize()
+    _STAGING[key] = (buf, None)
+    return buf[:numel].view(shape)
+
+
+def pinned_in_flight(slot, dev, stream):
+    """Record that the work queued so far on ``stream`` reads the ``pinned`` buffer of
+    (``slot``, ``dev``)."""
+    import torch
+    key = (slot, str(dev))
+    ev = torch.cuda.Event()
+    ev.record(stream)
+    _STAGING[key] = (_STAGING[key][0], ev)
+
+
+def staging(slot, dev):
+    """The dict kept for (``slot``, ``dev``) between calls, for the device buffers and side
+    streams of the packed host APIs."""
+    return _STAGING.setdefault((slot, str(dev)), {})
 
 
 def copy_pool():
@@ -155,7 +212,8 @@ def copy_pool():
 
 
 def parallel_copy(jobs):
-    """``jobs``: list of (dst_view, src_array) pairs, copied by the pool; blocks until done."""
+    """``jobs``: list of (dst_view, src_array) pairs, copied by the pool; blocks until done.
+    Below 2 MB in all, or for a single pair, the calling thread copies alone."""
     if not jobs:
         return
     total = sum(src.nbytes for _, src in jobs)
@@ -172,66 +230,12 @@ def parallel_copy(jobs):
 
 
 def gather_to_device(torch, arrays, dev, slot):
-    """Row-concatenate ``arrays`` into a pinned buffer (several threads; numpy releases the
-    GIL while copying) and start one asynchronous copy to ``dev``."""
-    from concurrent.futures import ThreadPoolExecutor
-    rows = np.array([len(a) for a in arrays], dtype=np.int64)
-    f = arrays[0].shape[1]
-    total = int(rows.sum())
-    key = (slot, str(dev))
-    buf, ev = _STAGING.get(key, (None, None))
-    if buf is None or buf.numel() < total * f:
-        buf = torch.empty(max(total * f, 1), dtype=torch.float64).pin_memory()
-        ev = None
-    if ev is not None:
-        ev.synchronize()            # the previous batch's copy has left the buffer
-    view = buf[:total * f].view(total, f)
-    host = view.numpy()
-    off = np.concatenate(([0], np.cumsum(rows)))
-    n = len(arrays)
-    step = max(1, (n + 4 * _GATHER_THREADS - 1) // (4 * _GATHER_THREADS))
-
-    def copy(lo):
-        for i in range(lo, min(n, lo + step)):
-            host[off[i]:off[i + 1]] = arrays[i]
-
-    if total * f * 8 < (1 << 22) or n == 1:
-        copy(0) if n == 1 else [copy(lo) for lo in range(0, n, step)]
-    else:
-        list(copy_pool().map(copy, range(0, n, step)))
-    out = view.to(dev, non_blocking=True)
-    ev = torch.cuda.Event()
-    ev.record(torch.cuda.current_stream(dev))
-    _STAGING[key] = (buf, ev)
-    return out
-
-
-def scatter_to_host(torch, tensor, offsets, slot):
-    """Device (rows, F) tensor -> list of freshly allocated host arrays, rows
-    ``offsets[i]:offsets[i + 1]`` each: one copy into a pinned buffer kept between calls, then
-    the per-segment copies on several threads."""
-    from concurrent.futures import ThreadPoolExecutor
-    total, f = tensor.shape
-    key = (slot, str(tensor.device))
-    buf, _ = _STAGING.get(key, (None, None))
-    if buf is None or buf.numel() < total * f or buf.dtype != tensor.dtype:
-        buf = torch.empty(max(total * f, 1), dtype=tensor.dtype).pin_memory()
-    _STAGING[key] = (buf, None)
-    view = buf[:total * f].view(total, f)
-    view.copy_(tensor, non_blocking=True)
-    torch.cuda.current_stream(tensor.device).synchronize()
-    host = view.numpy()
-    n = len(offsets) - 1
-    out = [None] * n
-    step = max(1, (n + _GATHER_THREADS - 1) // _GATHER_THREADS)
-
-    def copy(lo):
-        for i in range(lo, min(n, lo + step)):
-            out[i] = host[offsets[i]:offsets[i + 1]].copy()
-
-    if total * f * tensor.element_size() < (1 << 22) or n == 1:
-        for lo in range(0, n, step):
-            copy(lo)
-    else:
-        list(copy_pool().map(copy, range(0, n, step)))
+    """Row-concatenate ``arrays`` into the pinned buffer of ``slot`` (``parallel_copy``) and start
+    one asynchronous copy to ``dev``."""
+    off = np.concatenate(([0], np.cumsum([len(a) for a in arrays])))
+    buf = pinned(slot, dev, (int(off[-1]), arrays[0].shape[1]), torch.float64)
+    host = buf.numpy()
+    parallel_copy([(host[off[i]:off[i + 1]], a) for i, a in enumerate(arrays)])
+    out = buf.to(dev, non_blocking=True)
+    pinned_in_flight(slot, dev, torch.cuda.current_stream(dev))
     return out

@@ -25,7 +25,6 @@ def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vu
     ``return_offsets``: also the int64 CUDA tensor of row offsets (n + 1) of each pair's rows
     after the zero-frame removal."""
     torch = _lib.require_cuda()
-    lib = _lib.lib()
     dev = torch.device('cuda' if device is None else device)
     if power not in _POWER_MODES:
         raise ValueError(f'Unknown power parameter: {power!r}')
@@ -67,11 +66,8 @@ def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vu
             t_dev = torch.from_numpy(thr).to(dev) if len(thr) else None
             off_dev = torch.from_numpy(off).to(dev)
             feat = torch.empty((int(off[-1]), width + 1), dtype=torch.float64, device=dev)
-            rc = lib.kw_dtw_features(n, off_dev.data_ptr(), int(off[-1]), width, m_dev.data_ptr(),
-                                     _lib.ptr(v_dev), _lib.ptr(t_dev), _POWER_MODES[power],
-                                     float(power_weight), float(vuv_weight), feat.data_ptr(),
-                                     stream)
-            _lib.check(rc, 'kw_dtw_features')
+            _lib.call('kw_dtw_features', n, off_dev, int(off[-1]), width, m_dev, v_dev, t_dev,
+                      _POWER_MODES[power], float(power_weight), float(vuv_weight), feat, stream)
             dev_side.append((m_dev, feat, off_dev, lens))
         (xm, xf, xoff, tx), (ym, yf, yoff, ty) = dev_side
         res = fastdtw_batch_device(xf, yf, tx.astype(np.int32), ty.astype(np.int32),
@@ -80,13 +76,10 @@ def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vu
         tx_dev = torch.from_numpy(tx.astype(np.int32)).to(dev)
         ty_dev = torch.from_numpy(ty.astype(np.int32)).to(dev)
         sel_len = torch.empty(n, dtype=torch.int32, device=dev)
-        rc = lib.kw_path_select(n, region_off.data_ptr(), res.path_begin.data_ptr(),
-                                res.path_len.data_ptr(), tx_dev.data_ptr(), ty_dev.data_ptr(),
-                                xoff.data_ptr(), yoff.data_ptr(), xf.data_ptr(), yf.data_ptr(),
-                                width + 1, int(bool(strict)), int(power == 'binalize'),
-                                int(vuv is not None), int(bool(pad_silence)), int(pad_len),
-                                res.path.data_ptr(), sel_len.data_ptr(), stream)
-        _lib.check(rc, 'kw_path_select')
+        _lib.call('kw_path_select', n, region_off, res.path_begin, res.path_len, tx_dev, ty_dev,
+                  xoff, yoff, xf, yf, width + 1, int(bool(strict)), int(power == 'binalize'),
+                  int(vuv is not None), int(bool(pad_silence)), int(pad_len), res.path, sel_len,
+                  stream)
         out_off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
         out_off[1:] = torch.cumsum(sel_len.long(), dim=0)
         total = int(out_off[-1].item())             # the one read-back: N, for the allocation
@@ -94,11 +87,8 @@ def joint_frames_device(pairs, use_delta=True, pad_silence=True, pad_len=100, vu
         out = torch.empty((total, cols), dtype=torch.float64, device=dev)
         if total:
             zero = torch.empty(total, dtype=torch.uint8, device=dev)
-            rc = lib.kw_joint_frames(n, out_off.data_ptr(), total, region_off.data_ptr(),
-                                     res.path.data_ptr(), xoff.data_ptr(), yoff.data_ptr(),
-                                     xm.data_ptr(), ym.data_ptr(), width, int(bool(use_delta)),
-                                     out.data_ptr(), zero.data_ptr(), stream)
-            _lib.check(rc, 'kw_joint_frames')
+            _lib.call('kw_joint_frames', n, out_off, total, region_off, res.path, xoff, yoff, xm,
+                      ym, width, int(bool(use_delta)), out, zero, stream)
             row_off = out_off
             if bool(zero.any()):                    # rare: silent frames inside an utterance
                 out = out[~zero.bool()].contiguous()

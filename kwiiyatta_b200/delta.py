@@ -24,10 +24,8 @@ def delta_features_device(x_dev, offsets_dev, n_utts):
     torch = _lib.require_cuda()
     total, dim = x_dev.shape
     out = torch.empty((total, 3 * dim), dtype=torch.float64, device=x_dev.device)
-    rc = _lib.lib().kw_delta_features(n_utts, offsets_dev.data_ptr(), total, dim,
-                                      x_dev.data_ptr(), out.data_ptr(),
-                                      _lib.stream_ptr(torch))
-    _lib.check(rc, 'kw_delta_features')
+    _lib.call('kw_delta_features', n_utts, offsets_dev, total, dim, x_dev, out,
+              _lib.stream_ptr(torch))
     return out
 
 

@@ -72,7 +72,6 @@ def fastdtw_batch_device(x_dev, y_dev, tx, ty, radius=1, dist=2, precision=0, ti
     return the smallest decision margin on each path (``result.margin``, (n, 2): the returned
     path, all resolution levels).  Returns a DtwBatchResult (device tensors)."""
     torch = _lib.require_cuda()
-    lib = _lib.lib()
     tx = np.ascontiguousarray(tx, dtype=np.int32)
     ty = np.ascontiguousarray(ty, dtype=np.int32)
     n = len(tx)
@@ -81,8 +80,7 @@ def fastdtw_batch_device(x_dev, y_dev, tx, ty, radius=1, dist=2, precision=0, ti
         raise ValueError('second dimension of x and y must be the same')
     p_norm = _norm_from_dist(dist, 2)
     dev = x_dev.device
-    ws_bytes = lib.kw_dtw_workspace_bytes(n, tx.ctypes.data, ty.ctypes.data, f, int(radius))
-    ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+    ws_bytes = _lib.lib().kw_dtw_workspace_bytes(n, _lib.ptr(tx), _lib.ptr(ty), f, int(radius))
     total_pts = int(tx.astype(np.int64).sum() + ty.astype(np.int64).sum())
     cost = torch.empty(n, dtype=torch.float64, device=dev)
     path = torch.empty((total_pts, 2), dtype=torch.int32, device=dev)
@@ -90,12 +88,9 @@ def fastdtw_batch_device(x_dev, y_dev, tx, ty, radius=1, dist=2, precision=0, ti
     length = torch.empty(n, dtype=torch.int32, device=dev)
     cells = torch.empty(n, dtype=torch.int64, device=dev)
     margin = torch.empty((n, 2), dtype=torch.float64, device=dev) if with_margin else None
-    rc = lib.kw_dtw_batch(n, x_dev.data_ptr(), y_dev.data_ptr(), tx.ctypes.data,
-                          ty.ctypes.data, f, int(radius), p_norm, int(precision),
-                          TIE_MODES[tie_mode], cost.data_ptr(), path.data_ptr(),
-                          begin.data_ptr(), length.data_ptr(), cells.data_ptr(),
-                          _lib.ptr(margin), ws.data_ptr(), ws_bytes, _lib.stream_ptr(torch))
-    _lib.check(rc, 'kw_dtw_batch')
+    _lib.call('kw_dtw_batch', n, x_dev, y_dev, tx, ty, f, int(radius), p_norm, int(precision),
+              TIE_MODES[tie_mode], cost, path, begin, length, cells, margin,
+              _lib.workspace(ws_bytes, dev), ws_bytes, _lib.stream_ptr(torch))
     return DtwBatchResult(cost, path, begin, length, cells, tx, ty, margin)
 
 
@@ -152,20 +147,10 @@ def fastdtw_batch_packed(x_host, y_host, tx, ty, radius=1, dist=2, precision=0,
     results = []
     with torch.cuda.device(dev):
         main = torch.cuda.current_stream(dev)
-        # streams and pinned result buffers live across calls: the caching allocator keeps one
-        # pool per stream, and pinning is far more expensive than the copies
-        key = ('dtw_packed', str(dev))
-        cache = _lib._STAGING.setdefault(key, {'streams': [], 'host': {}})
-        while len(cache['streams']) < n_chunks:
-            cache['streams'].append(torch.cuda.Stream(dev))
-        streams = cache['streams'][:n_chunks] if n_chunks > 1 else [main]
-
-        def pinned(slot, name, like):
-            buf = cache['host'].get((slot, name))
-            if buf is None or buf.numel() < like.numel() or buf.dtype != like.dtype:
-                buf = torch.empty(max(like.numel(), 1), dtype=like.dtype).pin_memory()
-                cache['host'][(slot, name)] = buf
-            return buf[:like.numel()].view(like.shape)
+        streams = _lib.staging('dtw_packed', dev).setdefault('streams', [])
+        while len(streams) < n_chunks:
+            streams.append(torch.cuda.Stream(dev))
+        streams = streams[:n_chunks] if n_chunks > 1 else [main]
         start = torch.cuda.Event()
         start.record(main)
         parts = []
@@ -178,7 +163,7 @@ def fastdtw_batch_packed(x_host, y_host, tx, ty, radius=1, dist=2, precision=0,
                 yd = y_host[int(yrow[a]):int(yrow[b])].to(dev, non_blocking=True)
                 res = fastdtw_batch_device(xd, yd, tx[a:b], ty[a:b], radius, dist, precision,
                                            tie_mode)
-                host = {k: pinned(c, k, t)
+                host = {k: _lib.pinned(('dtw_packed', c, k), dev, t.shape, t.dtype)
                         for k, t in (('cost', res.cost), ('path', res.path),
                                      ('begin', res.path_begin), ('len', res.path_len))}
                 host['cost'].copy_(res.cost, non_blocking=True)
@@ -192,7 +177,7 @@ def fastdtw_batch_packed(x_host, y_host, tx, ty, radius=1, dist=2, precision=0,
             done.synchronize()
             main.wait_event(done)
             cost = host['cost'].tolist()
-            path = host['path'].numpy().copy()       # the pinned buffer is reused by the next call
+            path = host['path'].numpy().copy()
             first = (res.region_off[:-1] + host['begin'].numpy()).tolist()
             length = host['len'].tolist()
             results.extend((cost[p], path[first[p]:first[p] + length[p]])

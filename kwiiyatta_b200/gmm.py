@@ -121,7 +121,7 @@ class GaussianMixture:
         self._npad = lib.kw_gmm_resp_len(n, k) // k
         self._resp = torch.zeros((k, self._npad), **f64)   # component-major
         self._ws_bytes = lib.kw_gmm_workspace_bytes(n, k, d, self.precision)
-        self._ws = torch.empty(max(self._ws_bytes, 1), dtype=torch.uint8, device=dev)
+        self._ws = _lib.workspace(self._ws_bytes, dev)
         # two slots of pinned host memory for the per-iteration scalars (sum log p, n) and the
         # finalisation flags: copied asynchronously, read half an iteration later
         self._host_tail = torch.empty((2, 2), dtype=torch.float64).pin_memory()
@@ -130,10 +130,8 @@ class GaussianMixture:
 
     def _pack(self, torch, x):
         n, d = x.shape
-        rc = _lib.lib().kw_gmm_pack_frames(n, x.data_ptr(), self.n_components, d,
-                                           self.precision, self._ws.data_ptr(), self._ws_bytes,
-                                           _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_pack_frames')
+        _lib.call('kw_gmm_pack_frames', n, x, self.n_components, d, self.precision, self._ws,
+                  self._ws_bytes, _lib.stream_ptr(torch))
 
     def _frames(self, x):
         """The tensor the kernels read for the caller's ``x``: its reordered copy if one is
@@ -167,32 +165,25 @@ class GaussianMixture:
         n, d = x.shape
         self._resp_log = (bool(for_mstep) and self.precision == 1
                           and self.n_components <= RESP_FORM1_MAX_COMPONENTS)
-        rc = _lib.lib().kw_gmm_estep(
-            n, x.data_ptr(), self.n_components, d, self._means[self._cur].data_ptr(),
-            self._pc.data_ptr(), self._aux.data_ptr(), self._resp.data_ptr(),
-            self._stats.data_ptr(), self.precision, int(self._resp_log),
-            self._ws.data_ptr(), self._ws_bytes, _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_estep')
+        _lib.call('kw_gmm_estep', n, x, self.n_components, d, self._means[self._cur], self._pc,
+                  self._aux, self._resp, self._stats, self.precision, int(self._resp_log),
+                  self._ws, self._ws_bytes, _lib.stream_ptr(torch))
 
     def _normalize_resp(self, torch, x):
         """``_resp`` from log-probabilities to responsibilities, in place (no-op otherwise)."""
         if not self._resp_log:
             return
         n, d = self._frames(x).shape
-        rc = _lib.lib().kw_gmm_normalize_resp(
-            n, self.n_components, d, self._resp.data_ptr(), self._ws.data_ptr(), self._ws_bytes,
-            _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_normalize_resp')
+        _lib.call('kw_gmm_normalize_resp', n, self.n_components, d, self._resp, self._ws,
+                  self._ws_bytes, _lib.stream_ptr(torch))
         self._resp_log = False
 
     def _accumulate(self, torch, x, centres):
         x = self._frames(x)
         n, d = x.shape
-        rc = _lib.lib().kw_gmm_mstep_accumulate(
-            n, x.data_ptr(), self.n_components, d, self._resp.data_ptr(), centres.data_ptr(),
-            self._stats.data_ptr(), self.precision, int(self._resp_log),
-            self._ws.data_ptr(), self._ws_bytes, _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_mstep_accumulate')
+        _lib.call('kw_gmm_mstep_accumulate', n, x, self.n_components, d, self._resp, centres,
+                  self._stats, self.precision, int(self._resp_log), self._ws, self._ws_bytes,
+                  _lib.stream_ptr(torch))
 
     def _allreduce(self, torch):
         """The path's one exchange: sum of the statistics vector over the ranks."""
@@ -202,12 +193,9 @@ class GaussianMixture:
     def _finalize(self, torch, centres, weight_norm):
         k, d = centres.shape
         new = self._means[self._cur ^ 1]
-        rc = _lib.lib().kw_gmm_mstep_finalize(
-            k, d, float(self.reg_covar), weight_norm, self._stats.data_ptr(),
-            centres.data_ptr(), self._weights.data_ptr(), new.data_ptr(),
-            self._cov.data_ptr(), self._pc.data_ptr(), self._aux.data_ptr(),
-            self._info.data_ptr(), _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_mstep_finalize')
+        _lib.call('kw_gmm_mstep_finalize', k, d, float(self.reg_covar), weight_norm, self._stats,
+                  centres, self._weights, new, self._cov, self._pc, self._aux, self._info,
+                  _lib.stream_ptr(torch))
         self._cur ^= 1
 
     @staticmethod
@@ -403,11 +391,8 @@ class GaussianMixture:
         if self.means_init is not None:
             self._means[self._cur].copy_(_as_device(self.means_init, torch, dev))
         k, d = self._means[self._cur].shape
-        rc = _lib.lib().kw_gmm_precision_cholesky(
-            k, d, self._weights.data_ptr(), self._means[self._cur].data_ptr(),
-            self._cov.data_ptr(), self._pc.data_ptr(), self._aux.data_ptr(),
-            self._info.data_ptr(), _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_precision_cholesky')
+        _lib.call('kw_gmm_precision_cholesky', k, d, self._weights, self._means[self._cur],
+                  self._cov, self._pc, self._aux, self._info, _lib.stream_ptr(torch))
 
     def _publish(self):
         self.weights_ = self._weights.cpu().numpy()
@@ -436,11 +421,8 @@ class GaussianMixture:
         self._pc = torch.empty((k, d, d), **f64)
         self._aux = torch.empty((k, d + 2), **f64)
         self._info = torch.zeros(k, dtype=torch.int32, device=dev)
-        rc = _lib.lib().kw_gmm_precision_cholesky(
-            k, d, self._weights.data_ptr(), self._means[0].data_ptr(), self._cov.data_ptr(),
-            self._pc.data_ptr(), self._aux.data_ptr(), self._info.data_ptr(),
-            _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_gmm_precision_cholesky')
+        _lib.call('kw_gmm_precision_cholesky', k, d, self._weights, self._means[0], self._cov,
+                  self._pc, self._aux, self._info, _lib.stream_ptr(torch))
         self._check_info()
         self._publish()
         return self
@@ -459,7 +441,7 @@ class GaussianMixture:
         if self.precision < 0:      # 'auto' on a model that was loaded, not fitted: FP64 posteriors
             self.precision = 0
         self._ws_bytes = lib.kw_gmm_workspace_bytes(n, k, d, self.precision)
-        self._ws = torch.empty(max(self._ws_bytes, 1), dtype=torch.uint8, device=x.device)
+        self._ws = _lib.workspace(self._ws_bytes, x.device)
         self._pack(torch, x)
         self._estep(torch, x)
         resp, self._resp, self._ws = self._resp[:, :n].t(), None, None

@@ -75,7 +75,6 @@ def estimate_gv(features, columns=None, process_group=None, device=None):
         raise ValueError(f'bad utterance offsets or columns {columns} for width {width}')
     if int(off[-1].item()) != x.shape[0]:
         raise ValueError('offsets do not cover the rows of x')
-    lib = _lib.lib()
     f64 = dict(dtype=torch.float64, device=dev)
     utt_var = torch.empty((n_utts, ncols), **f64)
     sums = torch.empty(2 * ncols + 1, **f64)
@@ -83,18 +82,14 @@ def estimate_gv(features, columns=None, process_group=None, device=None):
     var = torch.empty(ncols, **f64)
     with torch.cuda.device(dev):
         stream = _lib.stream_ptr(torch)
-        rc = lib.kw_gv_estimate(n_utts, off.data_ptr(), int(x.shape[0]), width, col0, ncols,
-                                x.data_ptr(), utt_var.data_ptr(), sums.data_ptr(),
-                                mean.data_ptr(), var.data_ptr(), stream)
-        _lib.check(rc, 'kw_gv_estimate')
+        _lib.call('kw_gv_estimate', n_utts, off, int(x.shape[0]), width, col0, ncols, x, utt_var,
+                  sums, mean, var, stream)
         import torch.distributed as dist
         if dist.is_available() and dist.is_initialized() and \
                 dist.get_world_size(process_group) > 1:
             from . import dist as kdist
             kdist.allreduce_stats(sums, process_group)
-            rc = lib.kw_gv_from_sums(ncols, sums.data_ptr(), mean.data_ptr(), var.data_ptr(),
-                                     stream)
-            _lib.check(rc, 'kw_gv_from_sums')
+            _lib.call('kw_gv_from_sums', ncols, sums, mean, var, stream)
         if float(sums[-1].item()) < 1:
             raise ValueError('no utterance with frames to estimate the GV from')
     return GlobalVariance(mean.cpu().numpy(), var.cpu().numpy())

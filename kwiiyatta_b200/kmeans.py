@@ -63,12 +63,11 @@ def kmeans_labels(x, k, seed=None, group=None, n_lloyd=300, precision=0, tol=1e-
     aux = torch.zeros((k, d + 2), **f64)                         # [b = mu, log|L| = 0, log w = 0]
     labels = torch.empty(n, dtype=torch.int32, device=x.device)
     ws_bytes = lib.kw_gmm_workspace_bytes(n, k, d, precision)
-    ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=x.device)
+    ws = _lib.workspace(ws_bytes, x.device)
     npad = lib.kw_gmm_resp_len(n, k) // k
     resp = torch.zeros((k, npad), **f64)
     stream = _lib.stream_ptr(torch)
-    _lib.check(lib.kw_gmm_pack_frames(n, x.data_ptr(), k, d, precision, ws.data_ptr(), ws_bytes,
-                                      stream), 'kw_gmm_pack_frames')
+    _lib.call('kw_gmm_pack_frames', n, x, k, d, precision, ws, ws_bytes, stream)
     rows = torch.arange(n, device=x.device)
     prev = None
     # tolerance on the squared centre shift, relative to the data's mean variance (all ranks)
@@ -81,10 +80,8 @@ def kmeans_labels(x, k, seed=None, group=None, n_lloyd=300, precision=0, tol=1e-
     shift_tol = tol * var_mean
     for it in range(max(n_lloyd, 0) + 1):
         aux[:, :d] = centres
-        _lib.check(lib.kw_gmm_hard_labels(n, x.data_ptr(), k, d, centres.data_ptr(),
-                                          eye.data_ptr(), aux.data_ptr(), labels.data_ptr(),
-                                          precision, ws.data_ptr(), ws_bytes, stream),
-                   'kw_gmm_hard_labels')
+        _lib.call('kw_gmm_hard_labels', n, x, k, d, centres, eye, aux, labels, precision, ws,
+                  ws_bytes, stream)
         lab = labels.long()
         if it == n_lloyd:
             break
@@ -113,9 +110,7 @@ def kmeans_labels(x, k, seed=None, group=None, n_lloyd=300, precision=0, tol=1e-
         if n_lloyd > 0 and bool(shift <= shift_tol):
             # converged: one more assignment with the final centres, as sklearn does
             aux[:, :d] = centres
-            _lib.check(lib.kw_gmm_hard_labels(n, x.data_ptr(), k, d, centres.data_ptr(),
-                                              eye.data_ptr(), aux.data_ptr(), labels.data_ptr(),
-                                              precision, ws.data_ptr(), ws_bytes, stream),
-                       'kw_gmm_hard_labels')
+            _lib.call('kw_gmm_hard_labels', n, x, k, d, centres, eye, aux, labels, precision, ws,
+                      ws_bytes, stream)
             break
     return labels.long()

@@ -19,11 +19,7 @@ class MLPG:
                  device=None, gv=None, gv_iter=20, gv_weights=(1.0, 1.0)):
         torch = _lib.require_cuda()
         self._dev = torch.device('cuda' if device is None else device)
-        if self._dev.index is not None:
-            with torch.cuda.device(self._dev):
-                self._setup(torch, gmm, windows, swap, diff, precision)
-                self._setup_gv(torch, gv, gv_iter, gv_weights)
-        else:
+        with torch.cuda.device(self._dev):      # 'cuda' without an index: the current device
             self._setup(torch, gmm, windows, swap, diff, precision)
             self._setup_gv(torch, gv, gv_iter, gv_weights)
 
@@ -84,15 +80,13 @@ class MLPG:
         self._prepared = torch.empty(lib.kw_convert_prepared_len(k, dh), dtype=torch.float64,
                                      device=dev)
         info = torch.zeros(k, dtype=torch.int32, device=dev)
-        rc = lib.kw_convert_prepare(k, dh, int(self.diff), w.data_ptr(), m.data_ptr(),
-                                    c.data_ptr(), self._prepared.data_ptr(), info.data_ptr(),
-                                    _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_convert_prepare')
+        _lib.call('kw_convert_prepare', k, dh, int(self.diff), w, m, c, self._prepared, info,
+                  _lib.stream_ptr(torch))
         if info.cpu().numpy().any():
             raise np.linalg.LinAlgError('source covariance of some mixture is not positive '
                                         'definite')
 
-    def _launch(self, torch, n_utts, off_dev, total, max_frames, src, out, mix, stream,
+    def _launch(self, n_utts, off_dev, total, max_frames, src, out, mix, stream,
                 gv_f=None, gv_accepted=None):
         """kw_convert_batch, or kw_convert_gv_batch when GV statistics are set, on device
         tensors (``src`` (total, dim_half), ``out`` (total, static_dim))."""
@@ -100,23 +94,16 @@ class MLPG:
         k, dh = self.num_mixtures, self.dim_half
         if self.gv is None:
             ws_bytes = lib.kw_convert_workspace_bytes(total, k, dh, self.precision)
-            ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=src.device)
-            rc = lib.kw_convert_batch(n_utts, off_dev.data_ptr(), total, int(max_frames),
-                                      src.data_ptr(), k, dh, self._prepared.data_ptr(),
-                                      out.data_ptr(), _lib.ptr(mix), self.precision,
-                                      ws.data_ptr(), ws_bytes, stream)
-            _lib.check(rc, 'kw_convert_batch')
+            _lib.call('kw_convert_batch', n_utts, off_dev, total, int(max_frames), src, k, dh,
+                      self._prepared, out, mix, self.precision,
+                      _lib.workspace(ws_bytes, src.device), ws_bytes, stream)
             return
         ws_bytes = lib.kw_convert_gv_workspace_bytes(total, k, dh, self.precision)
-        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=src.device)
-        rc = lib.kw_convert_gv_batch(
-            n_utts, off_dev.data_ptr(), total, int(max_frames), src.data_ptr(), k, dh,
-            self._prepared.data_ptr(), self._gv_mean.data_ptr(), self._gv_var.data_ptr(),
-            self.gv_iter, self.gv_weights[0], self.gv_weights[1],
-            src.data_ptr() if self.diff else None, dh, out.data_ptr(), _lib.ptr(mix),
-            _lib.ptr(gv_f), _lib.ptr(gv_accepted), self.precision, ws.data_ptr(), ws_bytes,
-            stream)
-        _lib.check(rc, 'kw_convert_gv_batch')
+        _lib.call('kw_convert_gv_batch', n_utts, off_dev, total, int(max_frames), src, k, dh,
+                  self._prepared, self._gv_mean, self._gv_var, self.gv_iter, self.gv_weights[0],
+                  self.gv_weights[1], src if self.diff else None, dh, out, mix, gv_f,
+                  gv_accepted, self.precision, _lib.workspace(ws_bytes, src.device), ws_bytes,
+                  stream)
 
     @_on_own_device
     def transform_device(self, src_dev, offsets_dev, n_utts, max_frames, return_mix=False,
@@ -135,7 +122,7 @@ class MLPG:
                 raise ValueError('return_gv_info needs GV statistics')
             info = (torch.zeros((n_utts, self.static_dim), dtype=torch.float64, device=dev),
                     torch.zeros((n_utts, self.static_dim), dtype=torch.int32, device=dev))
-        self._launch(torch, n_utts, offsets_dev, total, max_frames, src_dev, out, mix,
+        self._launch(n_utts, offsets_dev, total, max_frames, src_dev, out, mix,
                      _lib.stream_ptr(torch), *(info or ()))
         res = (out,) + ((mix,) if return_mix else ()) + ((info,) if return_gv_info else ())
         return res if len(res) > 1 else out
@@ -158,14 +145,8 @@ class MLPG:
         if total == 0:
             return [np.zeros((0, self.static_dim)) for _ in feats]
         off = np.concatenate(([0], np.cumsum(lens)))
-        key = ('mlpg_many', str(self._dev))
-        bufs = _lib._STAGING.get(key)
-        if bufs is None or bufs[0].shape[0] < total or bufs[0].shape[1] != self.dim_half \
-                or bufs[1].shape[1] != self.static_dim:
-            bufs = (torch.empty((total, self.dim_half), dtype=torch.float64).pin_memory(),
-                    torch.empty((total, self.static_dim), dtype=torch.float64).pin_memory())
-            _lib._STAGING[key] = bufs
-        hin, hout = bufs[0][:total], bufs[1][:total]
+        hin = _lib.pinned('mlpg_in', self._dev, (total, self.dim_half), torch.float64)
+        hout = _lib.pinned('mlpg_out', self._dev, (total, self.static_dim), torch.float64)
         host = hin.numpy()
         _lib.parallel_copy([(host[off[i]:off[i + 1]], feats[i]) for i in range(len(feats))])
         self.transform_packed(hin, lens, out=hout)
@@ -203,16 +184,14 @@ class MLPG:
                 chunks.append((lo, i + 1))
                 lo, acc = i + 1, 0
         cap = max(int(rows[b] - rows[a]) for a, b in chunks)
-        key = ('mlpg_pipe', str(dev), dh, sd)
-        bufs = _lib._STAGING.get(key)
-        if bufs is None or bufs['cap'] < cap:
-            bufs = {'cap': cap,
-                    'din': [torch.empty((cap, dh), dtype=torch.float64, device=dev)
-                            for _ in range(2)],
-                    'dout': [torch.empty((cap, sd), dtype=torch.float64, device=dev)
+        bufs = _lib.staging(('mlpg_pipe', dh, sd), dev)
+        if bufs.get('cap', 0) < cap:
+            bufs.update(cap=cap,
+                        din=[torch.empty((cap, dh), dtype=torch.float64, device=dev)
                              for _ in range(2)],
-                    'streams': (torch.cuda.Stream(dev), torch.cuda.Stream(dev))}
-            _lib._STAGING[key] = bufs
+                        dout=[torch.empty((cap, sd), dtype=torch.float64, device=dev)
+                              for _ in range(2)],
+                        streams=(torch.cuda.Stream(dev), torch.cuda.Stream(dev)))
         s_in, s_out = bufs['streams']
         compute = torch.cuda.current_stream(dev)
         start = torch.cuda.Event()
@@ -236,7 +215,7 @@ class MLPG:
             if c >= 2:
                 compute.wait_event(ev_d2h[c - 2])        # device output buffer copied down
             chunk_in, chunk_out = bufs['din'][c & 1][:n_c], bufs['dout'][c & 1][:n_c]
-            self._launch(torch, b - a, off_dev, n_c, int(lens[a:b].max()), chunk_in, chunk_out,
+            self._launch(b - a, off_dev, n_c, int(lens[a:b].max()), chunk_in, chunk_out,
                          None, compute.cuda_stream)
             off_dev.record_stream(compute)
             keep.append(off)
@@ -255,7 +234,6 @@ class MLPG:
     def transform_soft(self, src):
         """MLPGBase.transform: per-frame soft-posterior conditional mean, (T, dim_half)."""
         torch = _lib.require_cuda()
-        lib = _lib.lib()
         src = np.ascontiguousarray(src, dtype=np.float64)
         if src.ndim != 2 or src.shape[1] != self.dim_half:
             raise ValueError(f'expected (T, {self.dim_half}) features, got {src.shape}')
@@ -264,12 +242,11 @@ class MLPG:
             return np.zeros((0, self.dim_half))
         x = torch.from_numpy(src).to(self._dev)
         out = torch.empty((total, self.dim_half), dtype=torch.float64, device=self._dev)
-        ws_bytes = lib.kw_convert_soft_workspace_bytes(total, self.num_mixtures, self.dim_half)
-        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=self._dev)
-        rc = lib.kw_convert_soft_batch(total, x.data_ptr(), self.num_mixtures, self.dim_half,
-                                       self._prepared.data_ptr(), out.data_ptr(), ws.data_ptr(),
-                                       ws_bytes, _lib.stream_ptr(torch))
-        _lib.check(rc, 'kw_convert_soft_batch')
+        ws_bytes = _lib.lib().kw_convert_soft_workspace_bytes(total, self.num_mixtures,
+                                                              self.dim_half)
+        _lib.call('kw_convert_soft_batch', total, x, self.num_mixtures, self.dim_half,
+                  self._prepared, out, _lib.workspace(ws_bytes, self._dev), ws_bytes,
+                  _lib.stream_ptr(torch))
         return out.cpu().numpy()
 
     def transform(self, src):

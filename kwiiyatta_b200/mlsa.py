@@ -21,9 +21,8 @@ def mc2b_many(mceps, alpha, zero_power=True):
     if any(m.ndim != 2 or m.shape[1] != width for m in mceps):
         raise ValueError('all mel-cepstra must be (T, order + 1) with the same order')
     x = torch.from_numpy(np.concatenate(mceps)).cuda()
-    rc = _lib.lib().kw_mc2b(x.shape[0], width, float(alpha), int(bool(zero_power)), x.data_ptr(),
-                            x.data_ptr(), _lib.stream_ptr(torch))
-    _lib.check(rc, 'kw_mc2b')
+    _lib.call('kw_mc2b', x.shape[0], width, float(alpha), int(bool(zero_power)), x, x,
+              _lib.stream_ptr(torch))
     out = x.cpu().numpy()
     off = np.concatenate(([0], np.cumsum(lens)))
     return [out[off[i]:off[i + 1]] for i in range(len(mceps))]
