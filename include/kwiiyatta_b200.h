@@ -240,6 +240,26 @@ int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t total_frames
                         int32_t* mix_dev, double* f_dev, int32_t* accepted_dev, int precision,
                         void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* Maximum-likelihood conversion over all mixture sequences (EM trajectory estimation; Toda, Black
+ * & Tokuda, IEEE TASLP 15(8), 2007; oracle/mlpg_em_ref.py).  kw_convert_em_batch starts from the
+ * kw_convert_batch output y0 and runs em_iter (>= 1) EM iterations on
+ *   L(y) = sum_t log sum_m w_m N(x_t; mu_x, S_xx) N((W y)_t; E_{m,t}, diag D_m)
+ * per utterance: E-step = the GMM E-step at dimension 2 * dim_half on [x_t ; (W y)_t] (precision
+ * 0: FP64, 1: tensor cores); M-step = the MLPG system (W^T P W) y = W^T q with per-frame
+ * P_t = sum_m gamma D_m^-1 and q_t = sum_m gamma D_m^-1 E_{m,t}, where posteriors gamma <= 1e-14
+ * contribute nothing.  No iteration decreases L (up to rounding).  Diff mode is the same
+ * iteration on a `prepared` block made with diff = 1.  out_dev (sum T, static_dim) receives y;
+ * loglik_dev (n_utts, em_iter + 1), may be NULL, receives L(y_k) for k = 0 .. em_iter (the last
+ * entry costs one more E-step), each summed in a fixed order.  Bitwise reproducible.  Needs
+ * dim_half a multiple of 3 and 2 * dim_half <= 144.  Workspace: kw_convert_em_workspace_bytes. */
+size_t kw_convert_em_workspace_bytes(int64_t total_frames, int n_components, int dim_half,
+                                     int precision);
+int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t total_frames,
+                        const double* src_dev, int n_components, int dim_half,
+                        const double* prepared_dev, int em_iter, double* out_dev,
+                        double* loglik_dev, int precision, void* workspace_dev,
+                        size_t workspace_bytes, void* stream);
+
 /* Soft-posterior mapping without MLPG (nnmnkwii MLPGBase.transform; the mlpg=False branch of
  * kwiiyatta/converter/gmm.py:30-31): out (total, dim_half) = sum_m p(m|x) (mu_y + S_yx S_xx^-1 (x - mu_x)).
  * `prepared_dev` comes from kw_convert_prepare with the same dim_half. */

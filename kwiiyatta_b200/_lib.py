@@ -55,6 +55,9 @@ SIGNATURES = {
     'kw_convert_gv_workspace_bytes': (_sz, [_i64, _i, _i, _i]),
     'kw_convert_gv_batch': (_i, [_i, _vp, _i64, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _dbl, _dbl,
                                  _vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _sz, _vp]),
+    'kw_convert_em_workspace_bytes': (_sz, [_i64, _i, _i, _i]),
+    'kw_convert_em_batch': (_i, [_i, _vp, _i64, _vp, _i, _i, _vp, _i, _vp, _vp, _i, _vp, _sz,
+                                 _vp]),
 }
 
 

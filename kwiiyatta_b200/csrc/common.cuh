@@ -52,8 +52,10 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // gmm.cu internals shared with convert.cu
+// lse_frame (mode 0, may be NULL): the per-frame log-normaliser logsumexp_k wlp[n, k]
 int estep_fp64(long long N, const double* X, int K, int D, const double* pc, const double* aux,
-               double* resp, double* lse_partial, int mode, int32_t* mix, cudaStream_t st);
+               double* resp, double* lse_partial, int mode, int32_t* mix, cudaStream_t st,
+               double* lse_frame = nullptr);
 long long resp_pad(long long n);
 void launch_reduce_fixed(const double* in, long long n, double extra, double* out, cudaStream_t st);
 // gmm_tc.cu
@@ -67,7 +69,8 @@ int normalize_resp_tc(long long N, int K, int D, double* resp, void* workspace,
                       size_t workspace_bytes, cudaStream_t st);
 int estep_tc(long long N, const double* X, int K, int D, const double* means, const double* pc,
              const double* aux, double* resp, double* lse_out, int mode, int32_t* mix,
-             void* workspace, size_t workspace_bytes, cudaStream_t st, int resp_form = 0);
+             void* workspace, size_t workspace_bytes, cudaStream_t st, int resp_form = 0,
+             double* lse_frame = nullptr);
 int mstats_fp64(long long N, const double* X, int K, int D, const double* resp,
                 const double* centres, double* partial, double* stats, double resp_floor,
                 cudaStream_t st);

@@ -8,7 +8,11 @@
 //   y[:, d] = solve( W^T D^-1 W , W^T D^-1 E )  per static dim d, pentadiagonal SPD system,
 //   windows = kwiiyatta DELTA_WINDOWS (kwiiyatta/converter/delta.py:8-12).
 // Beyond the reference: global-variance (GV) statistics and GV-considered generation on the same
-// normal equations (kw_gv_estimate, kw_convert_gv_batch; restated in oracle/gv_ref.py).
+// normal equations (kw_gv_estimate, kw_convert_gv_batch; restated in oracle/gv_ref.py), and
+// maximum-likelihood conversion over all mixture sequences by EM (kw_convert_em_batch; restated
+// in oracle/mlpg_em_ref.py).
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace kw {
@@ -210,11 +214,17 @@ convert_condmean_kernel(int K, int Dh, const double* __restrict__ src,
 // Soft-posterior mapping (nnmnkwii MLPGBase.transform, the mlpg=False branch of
 // kwiiyatta/converter/gmm.py:30-31):  y_t = sum_m p(m | x_t) (offset[m] + A[m] x_t).
 // CTA = 32 frames; thread r owns output dimension r for all 32 frames; mixtures whose posterior is
-// below 1e-14 for every frame of the tile are skipped.
+// not above SOFT_FLOOR for any frame of the tile are skipped.
+// PREC (the M-step of EM conversion): every term is also weighted by 1 / var[m][r] and terms with
+// p(m | x_t) <= SOFT_FLOOR are dropped, so out = q_t = sum_m p D_m^-1 E_{m,t} and prec_out =
+// P_t = sum_m p D_m^-1 (both (N, Dh)).
 constexpr int SOFT_FT = 32;
+constexpr double SOFT_FLOOR = 1e-14;
+template <bool PREC>
 __global__ void __launch_bounds__(96)
 convert_soft_kernel(long long N, long long Npad, int K, int Dh, const double* __restrict__ src,
-                    const double* __restrict__ respT, PreparedView v, double* __restrict__ out) {
+                    const double* __restrict__ respT, PreparedView v, double* __restrict__ out,
+                    double* __restrict__ prec_out) {
     extern __shared__ double xs[];          // SOFT_FT * Dh frames, then SOFT_FT responsibilities
     double* rs = xs + SOFT_FT * Dh;
     __shared__ int any_active;
@@ -224,9 +234,13 @@ convert_soft_kernel(long long N, long long Npad, int K, int Dh, const double* __
         xs[e] = (n < N) ? src[n * Dh + (e % Dh)] : 0.0;
     }
     const int r = threadIdx.x;
-    double acc[SOFT_FT];
+    double acc[SOFT_FT], pacc[PREC ? SOFT_FT : 1];
 #pragma unroll
     for (int f = 0; f < SOFT_FT; ++f) acc[f] = 0.0;
+    if (PREC) {
+#pragma unroll
+        for (int f = 0; f < SOFT_FT; ++f) pacc[f] = 0.0;
+    }
     for (int m = 0; m < K; ++m) {
         __syncthreads();
         if (threadIdx.x == 0) any_active = 0;
@@ -234,8 +248,8 @@ convert_soft_kernel(long long N, long long Npad, int K, int Dh, const double* __
         if (threadIdx.x < SOFT_FT) {
             const long long n = n0 + threadIdx.x;
             const double p = (n < N) ? respT[(size_t)m * Npad + n] : 0.0;
-            rs[threadIdx.x] = p;
-            if (p > 1e-14) any_active = 1;
+            rs[threadIdx.x] = (PREC && !(p > SOFT_FLOOR)) ? 0.0 : p;
+            if (p > SOFT_FLOOR) any_active = 1;
         }
         __syncthreads();
         if (!any_active || r >= Dh) continue;
@@ -249,13 +263,26 @@ convert_soft_kernel(long long N, long long Npad, int K, int Dh, const double* __
 #pragma unroll
             for (int f = 0; f < SOFT_FT; ++f) e[f] = fma(a, xs[f * Dh + c], e[f]);
         }
+        if (PREC) {
+            const double iv = 1.0 / v.var[(size_t)m * Dh + r];
 #pragma unroll
-        for (int f = 0; f < SOFT_FT; ++f) acc[f] = fma(rs[f], e[f], acc[f]);
+            for (int f = 0; f < SOFT_FT; ++f) {
+                const double g = rs[f] * iv;
+                pacc[f] += g;
+                acc[f] = fma(g, e[f], acc[f]);
+            }
+        } else {
+#pragma unroll
+            for (int f = 0; f < SOFT_FT; ++f) acc[f] = fma(rs[f], e[f], acc[f]);
+        }
     }
     if (r < Dh) {
 #pragma unroll
         for (int f = 0; f < SOFT_FT; ++f)
-            if (n0 + f < N) out[(n0 + f) * Dh + r] = acc[f];
+            if (n0 + f < N) {
+                out[(n0 + f) * Dh + r] = acc[f];
+                if (PREC) prec_out[(n0 + f) * Dh + r] = pacc[f];
+            }
     }
 }
 
@@ -263,7 +290,9 @@ convert_soft_kernel(long long N, long long Npad, int K, int Dh, const double* __
 //  1. convert_band_kernel, one thread per (frame, static dim): the pentadiagonal normal
 //     equations W^T P W y = W^T P mu of that dimension, row by row: a_i = P[i][i],
 //     b_i = P[i][i+1], c_i = P[i][i+2] and the right-hand side.  Fully parallel; this is where
-//     the per-frame gathers (mixture -> variance) and the divisions happen.
+//     the per-frame gathers (mixture -> variance) and the divisions happen.  FRAME_PREC (the
+//     M-step of EM conversion) reads the per-frame precision P_t from `var` and the
+//     precision-weighted mean P_t mu_t from `E`, both (total, Dh); `mix` is unused.
 //  2. convert_mlpg_kernel, one thread per (utterance, static dim): banded Cholesky
 //     (bandwidth 2) and the two substitutions, in place over the four arrays, reading four
 //     steps ahead of the recurrence.  The chain per frame is two fused multiply-adds and one
@@ -290,6 +319,7 @@ __global__ void convert_flags_kernel(int n_utts, const int64_t* __restrict__ off
     }
 }
 
+template <bool FRAME_PREC>
 __global__ void __launch_bounds__(256)
 convert_band_kernel(long long total, int sd, int Dh, const double* __restrict__ E,
                     const int32_t* __restrict__ mix, const double* __restrict__ var,
@@ -303,6 +333,14 @@ convert_band_kernel(long long total, int sd, int Dh, const double* __restrict__ 
     // p[w], bs[w] at frames n-1 (m), n (c), n+1 (x)
     double pm[3] = {0, 0, 0}, bm[3] = {0, 0, 0}, pc[3], bc[3], px[3] = {0, 0, 0}, bx[3] = {0, 0, 0};
     auto load = [&](long long t, double* p, double* b) {
+        if (FRAME_PREC) {
+#pragma unroll
+            for (int w = 0; w < 3; ++w) {
+                p[w] = var[t * Dh + w * sd + d];
+                b[w] = E[t * Dh + w * sd + d];
+            }
+            return;
+        }
         const int m = mix[t];
 #pragma unroll
         for (int w = 0; w < 3; ++w) {
@@ -668,6 +706,84 @@ convert_gv_kernel(GvArgs g) {
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// Maximum-likelihood conversion over all mixture sequences (EM trajectory estimation; Toda,
+// Black & Tokuda, IEEE TASLP 15(8), 2007; restated in oracle/mlpg_em_ref.py).  With the diagonal
+// conditional variance the hard-sequence MLPG already uses, the model of the joint vector
+// z_t = [x_t ; (W y)_t] under mixture m is ONE Gaussian of dimension 2 Dh:
+//   mean [mu_x ; mu_y],  precision Cholesky (upper)  L~ = [[Lx, -A^T D^-1/2], [0, D^-1/2]],
+//   log|L~| = log|Lx| - 1/2 sum_j log D_j,
+// so the E-step is the GMM E-step at D = 2 Dh on z, and its per-frame log-normaliser summed over
+// an utterance is the objective L(y) = sum_t log sum_m w_m N(x_t; mu_x, S_xx) N((W y)_t; E, D).
+// M-step: P_t = sum_m g D_m^-1, q_t = sum_m g D_m^-1 E_{m,t} (g = gamma above SOFT_FLOOR), then
+// (W^T P W) y = W^T q per static dimension, the MLPG system with per-frame precisions.
+
+// The derived joint model (means, L~, aux = [mu~ L~ | log|L~| | log w]) from the prepared block.
+// mu~ L~ = [mu_x Lx ; offset D^-1/2] (offset = mu_y - A mu_x).  One CTA per mixture.
+__global__ void convert_em_model_kernel(int Dh, PreparedView v, double* __restrict__ means,
+                                        double* __restrict__ pc, double* __restrict__ aux) {
+    const int k = blockIdx.x;
+    const int D = 2 * Dh;
+    const double* lx = v.px_prec_chol + (size_t)k * Dh * Dh;
+    const double* at = v.at + (size_t)k * Dh * Dh;
+    const double* var = v.var + (size_t)k * Dh;
+    double* L = pc + (size_t)k * D * D;
+    for (int e = threadIdx.x; e < D * D; e += blockDim.x) {
+        const int r = e / D, c = e - r * D;
+        double x = 0.0;
+        if (r < Dh && c < Dh) x = lx[r * Dh + c];
+        else if (r < Dh) x = -at[r * Dh + c - Dh] / sqrt(var[c - Dh]);   // -A^T[r][j] / sqrt(D_j)
+        else if (r == c) x = 1.0 / sqrt(var[r - Dh]);
+        L[e] = x;
+    }
+    const double* pa = v.px_aux + (size_t)k * (Dh + 2);
+    double* ak = aux + (size_t)k * (D + 2);
+    for (int j = threadIdx.x; j < Dh; j += blockDim.x) {
+        means[(size_t)k * D + j] = v.src_means[(size_t)k * Dh + j];
+        means[(size_t)k * D + Dh + j] = v.tgt_means[(size_t)k * Dh + j];
+        ak[j] = pa[j];
+        ak[Dh + j] = v.offset[(size_t)k * Dh + j] / sqrt(var[j]);
+    }
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int j = 0; j < Dh; ++j) s += log(var[j]);
+        ak[D] = pa[Dh] - 0.5 * s;
+        ak[D + 1] = pa[Dh + 1];
+    }
+}
+
+// (W y)_t into columns [col0, col0 + 3 sd) of the row-major (total, ld) joint frames: window w at
+// offsets -1, 0, +1, zero past the utterance's edges (flags), one thread per (frame, static dim).
+__global__ void convert_em_frames_kernel(long long total, int sd, const double* __restrict__ y,
+                                         const unsigned char* __restrict__ flags, Windows win,
+                                         int ld, int col0, double* __restrict__ z) {
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= total * sd) return;
+    const long long n = gid / sd;
+    const int d = (int)(gid - n * sd);
+    const unsigned fl = flags[n];
+    const double yc = y[gid];
+    const double ym = (fl & 1u) ? 0.0 : y[gid - sd];
+    const double yp = (fl & 2u) ? 0.0 : y[gid + sd];
+    double* o = z + n * ld + col0 + d;
+#pragma unroll
+    for (int w = 0; w < 3; ++w) o[w * sd] = win.c[w][0] * ym + win.c[w][1] * yc + win.c[w][2] * yp;
+}
+
+// out[u * stride + col] = sum of lse over the frames of utterance u: one warp per utterance,
+// lane-strided partial sums and an xor-butterfly (one fixed order).
+__global__ void convert_em_loglik_kernel(int n_utts, const int64_t* __restrict__ off,
+                                         const double* __restrict__ lse, int stride, int col,
+                                         double* __restrict__ out) {
+    const int u = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (u >= n_utts) return;
+    double s = 0.0;
+    for (long long t = off[u] + lane; t < off[u + 1]; t += 32) s += lse[t];
+    s = warp_sum(s);
+    if (lane == 0) out[(size_t)u * stride + col] = s;
+}
+
 struct ConvertWorkspace {
     int32_t* mix;
     int* counts;      // K
@@ -750,8 +866,8 @@ extern "C" int kw_convert_soft_batch(int64_t total, const double* src_dev, int K
     int rc = estep_fp64(total, src_dev, K, Dh, v.px_prec_chol, v.px_aux, resp, lse, 0, nullptr, st);
     if (rc != KW_OK) return rc;
     const size_t smem = sizeof(double) * ((size_t)SOFT_FT * Dh + SOFT_FT);
-    convert_soft_kernel<<<(unsigned)((total + SOFT_FT - 1) / SOFT_FT), 96, smem, st>>>(
-        total, resp_pad(total), K, Dh, src_dev, resp, v, out_dev);
+    convert_soft_kernel<false><<<(unsigned)((total + SOFT_FT - 1) / SOFT_FT), 96, smem, st>>>(
+        total, resp_pad(total), K, Dh, src_dev, resp, v, out_dev, nullptr);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }
@@ -836,7 +952,7 @@ static int convert_run(int n_utts, const int64_t* off_dev, int64_t total, const 
         convert_flags_kernel<<<(n_utts + 127) / 128, 128, 0, st>>>(n_utts, off_dev, w.flags);
         KW_CUDA_CHECK(cudaGetLastError());
         const long long cells = total * sd;
-        convert_band_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
+        convert_band_kernel<false><<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
             total, sd, Dh, w.E, w.mix, v.var, w.flags, win, w.band);
         KW_CUDA_CHECK(cudaGetLastError());
         const long long threads = (long long)n_utts * sd;
@@ -920,7 +1036,7 @@ extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t t
     // the same bytes as a saved copy would and keeps the workspace at one band set
     PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
     const long long cells = total * sd;
-    convert_band_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
+    convert_band_kernel<false><<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
         total, sd, Dh, w.E, w.mix, v.var, w.flags, kDeltaWindows, w.band);
     KW_CUDA_CHECK(cudaGetLastError());
     GvArgs g;
@@ -946,5 +1062,135 @@ extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t t
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     convert_gv_kernel<<<(unsigned)(n_utts * sd), 32, smem, st>>>(g);
     KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+// EM workspace: [ EmWorkspace | the kw_convert_batch workspace at precision 0 | the tensor-core
+// workspace of the larger of the two E-steps (precision 1) ].
+struct EmWorkspace {
+    double* z;      // (total, 2 Dh) joint frames [x | W y]
+    double* resp;   // (K, resp_pad(total))
+    double* lse;    // (total) per-frame log-normaliser
+    double* lsep;   // E-step partial sums (at most one per frame) + the two-value total
+    double* q;      // (total, Dh)
+    double* prec;   // (total, Dh)
+    double* means;  // (K, 2 Dh)
+    double* pc;     // (K, 2 Dh, 2 Dh)
+    double* aux;    // (K, 2 Dh + 2)
+    size_t bytes;
+};
+
+static EmWorkspace carve_em(long long total, int K, int Dh, void* base) {
+    Carver c(base);
+    EmWorkspace w;
+    const size_t D = 2 * (size_t)Dh;
+    w.z = c.take<double>((size_t)total * D);
+    w.resp = c.take<double>((size_t)K * (size_t)resp_pad(total));
+    w.lse = c.take<double>((size_t)total);
+    w.lsep = c.take<double>((size_t)total + 2);
+    w.q = c.take<double>((size_t)total * Dh);
+    w.prec = c.take<double>((size_t)total * Dh);
+    w.means = c.take<double>((size_t)K * D);
+    w.pc = c.take<double>((size_t)K * D * D);
+    w.aux = c.take<double>((size_t)K * (D + 2));
+    w.bytes = align_up(c.used, 256);
+    return w;
+}
+
+extern "C" size_t kw_convert_em_workspace_bytes(int64_t total_frames, int K, int Dh,
+                                                int precision) {
+    size_t b = carve_em(total_frames, K, Dh, nullptr).bytes +
+               carve_convert(total_frames, K, Dh, Dh / 3, nullptr).bytes;
+    if (precision == 1)
+        b += std::max(tc_workspace_bytes(total_frames, K, Dh),
+                      tc_workspace_bytes(total_frames, K, 2 * Dh));
+    return b;
+}
+
+extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t total,
+                                   const double* src_dev, int K, int Dh,
+                                   const double* prepared_dev, int em_iter, double* out_dev,
+                                   double* loglik_dev, int precision, void* workspace_dev,
+                                   size_t workspace_bytes, void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    KW_REQUIRE(em_iter >= 1, "kw_convert_em_batch: em_iter must be at least 1, got %d", em_iter);
+    KW_REQUIRE(Dh % 3 == 0, "dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
+    KW_REQUIRE(n_utts >= 0 && total >= 0 && K > 0, "kw_convert_em_batch: bad sizes");
+    if (n_utts == 0) return KW_OK;
+    if (total == 0) {
+        if (loglik_dev != nullptr)
+            KW_CUDA_CHECK(cudaMemsetAsync(loglik_dev, 0,
+                                          sizeof(double) * (size_t)n_utts * (em_iter + 1), st));
+        return KW_OK;
+    }
+    if (2 * Dh > 144) {
+        set_error("dim_half %d: the EM E-step runs at 2 * dim_half <= 144", Dh);
+        return KW_ERR_UNSUPPORTED;
+    }
+    KW_REQUIRE(precision == 0 || precision == 1, "convert precision must be 0 or 1");
+    if (kw_convert_em_workspace_bytes(total, K, Dh, precision) > workspace_bytes) {
+        set_error("EM convert workspace too small");
+        return KW_ERR_WORKSPACE;
+    }
+    const int sd = Dh / 3, D = 2 * Dh;
+    EmWorkspace em = carve_em(total, K, Dh, workspace_dev);
+    ConvertWorkspace w;
+    int rc = convert_run(n_utts, off_dev, total, src_dev, K, Dh, prepared_dev, out_dev, nullptr,
+                         precision, static_cast<char*>(workspace_dev) + em.bytes,
+                         workspace_bytes - em.bytes, st, &w);
+    if (rc != KW_OK) return rc;
+    // convert_run left the flags in its workspace; its tensor-core region follows it
+    char* tcw = static_cast<char*>(workspace_dev) + em.bytes + w.bytes;
+    const size_t tcb = workspace_bytes - em.bytes - w.bytes;
+    PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    convert_em_model_kernel<<<K, 256, 0, st>>>(Dh, v, em.means, em.pc, em.aux);
+    KW_CUDA_CHECK(cudaGetLastError());
+    KW_CUDA_CHECK(cudaMemcpy2DAsync(em.z, sizeof(double) * D, src_dev, sizeof(double) * Dh,
+                                    sizeof(double) * Dh, (size_t)total, cudaMemcpyDeviceToDevice,
+                                    st));
+    const long long cells = total * sd;
+    const unsigned cell_blocks = (unsigned)((cells + 255) / 256);
+    // E-step at y = out_dev: responsibilities into em.resp, log-normalisers into em.lse and, when
+    // asked, their per-utterance sums into column `col` of the trace
+    auto estep = [&](int col) -> int {
+        convert_em_frames_kernel<<<cell_blocks, 256, 0, st>>>(total, sd, out_dev, w.flags,
+                                                               kDeltaWindows, D, Dh, em.z);
+        KW_CUDA_CHECK(cudaGetLastError());
+        int r;
+        if (precision == 1) {
+            r = pack_frames_tc(total, em.z, K, D, tcw, tcb, st, /*mstep_parts=*/false);
+            if (r != KW_OK) return r;
+            r = estep_tc(total, em.z, K, D, em.means, em.pc, em.aux, em.resp, em.lsep, 0, nullptr,
+                         tcw, tcb, st, 0, em.lse);
+        } else {
+            r = estep_fp64(total, em.z, K, D, em.pc, em.aux, em.resp, em.lsep, 0, nullptr, st,
+                           em.lse);
+        }
+        if (r != KW_OK) return r;
+        if (loglik_dev != nullptr) {
+            convert_em_loglik_kernel<<<(unsigned)((32LL * n_utts + 255) / 256), 256, 0, st>>>(
+                n_utts, off_dev, em.lse, em_iter + 1, col, loglik_dev);
+            KW_CUDA_CHECK(cudaGetLastError());
+        }
+        return KW_OK;
+    };
+    const size_t soft_smem = sizeof(double) * ((size_t)SOFT_FT * Dh + SOFT_FT);
+    for (int it = 0; it < em_iter; ++it) {
+        rc = estep(it);
+        if (rc != KW_OK) return rc;
+        convert_soft_kernel<true><<<(unsigned)((total + SOFT_FT - 1) / SOFT_FT), 96, soft_smem,
+                                    st>>>(total, resp_pad(total), K, Dh, src_dev, em.resp, v, em.q,
+                                          em.prec);
+        KW_CUDA_CHECK(cudaGetLastError());
+        convert_band_kernel<true><<<cell_blocks, 256, 0, st>>>(total, sd, Dh, em.q, nullptr,
+                                                               em.prec, w.flags, kDeltaWindows,
+                                                               w.band);
+        KW_CUDA_CHECK(cudaGetLastError());
+        const long long threads = (long long)n_utts * sd;
+        convert_mlpg_kernel<<<(unsigned)((threads + 95) / 96), 96, 0, st>>>(
+            n_utts, off_dev, sd, w.band, total, out_dev);
+        KW_CUDA_CHECK(cudaGetLastError());
+    }
+    if (loglik_dev != nullptr) return estep(em_iter);
     return KW_OK;
 }

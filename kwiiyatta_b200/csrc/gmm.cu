@@ -27,14 +27,15 @@ __host__ __device__ static inline size_t stats_block(int D) { return 1 + (size_t
 // ---------------------------------------------------------------------------------------
 // E-step.  CTA = 64 frames x all K components.  256 threads = 16 frame groups (4 frames
 // each, interleaved) x 16 column groups (TN contiguous columns each).
-// mode 0: write resp + per-CTA sum of logsumexp.  mode 1: hard argmax (np.argmax: first max).
+// mode 0: write resp + per-CTA sum of logsumexp (and, when lse_frame is not NULL, the logsumexp
+// of every frame).  mode 1: hard argmax (np.argmax: first max).
 // ---------------------------------------------------------------------------------------
 template <int TN>
 __global__ void __launch_bounds__(256)
 gmm_estep_kernel(long long N, long long Npad, const double* __restrict__ X, int K, int D,
                  const double* __restrict__ prec_chol, const double* __restrict__ aux,
                  double* __restrict__ resp, double* __restrict__ lse_partial, int mode,
-                 int32_t* __restrict__ mix_out) {
+                 int32_t* __restrict__ mix_out, double* __restrict__ lse_frame) {
     constexpr int WT = 16 * TN;
     extern __shared__ double sm[];
     const int Dp = (D + E_KC - 1) / E_KC * E_KC;
@@ -160,6 +161,7 @@ gmm_estep_kernel(long long N, long long Npad, const double* __restrict__ X, int 
             lse = log(sum) + mx;
             for (int k = 0; k < K; ++k)
                 col[(size_t)k * Npad] = exp(__ldcg(col + (size_t)k * Npad) - lse);
+            if (lse_frame != nullptr) lse_frame[n] = lse;
         }
         frame_lse[tid] = lse;
     }
@@ -757,7 +759,7 @@ static GmmWorkspace carve_gmm(long long N, int K, int D, void* base) {
 template <int TN>
 static int launch_estep(long long N, const double* X, int K, int D, const double* pc,
                         const double* aux, double* resp, double* lse_partial, int mode,
-                        int32_t* mix, cudaStream_t st) {
+                        int32_t* mix, cudaStream_t st, double* lse_frame) {
     const int Dp = (D + E_KC - 1) / E_KC * E_KC;
     const size_t smem = sizeof(double) * ((size_t)E_FT * (Dp + 1) + 2 * E_KC * 16 * TN);
     auto kern = gmm_estep_kernel<TN>;
@@ -765,18 +767,24 @@ static int launch_estep(long long N, const double* X, int K, int D, const double
                                        (int)smem));
     const long long grid = (N + E_FT - 1) / E_FT;
     kern<<<(unsigned)grid, 256, smem, st>>>(N, resp_pad(N), X, K, D, pc, aux, resp, lse_partial,
-                                            mode, mix);
+                                            mode, mix, lse_frame);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }
 
 int estep_fp64(long long N, const double* X, int K, int D, const double* pc, const double* aux,
-               double* resp, double* lse_partial, int mode, int32_t* mix, cudaStream_t st) {
-    if (D <= 16) return launch_estep<1>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st);
-    if (D <= 32) return launch_estep<2>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st);
-    if (D <= 48) return launch_estep<3>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st);
-    if (D <= 80) return launch_estep<5>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st);
-    if (D <= 144) return launch_estep<9>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st);
+               double* resp, double* lse_partial, int mode, int32_t* mix, cudaStream_t st,
+               double* lse_frame) {
+    if (D <= 16) return launch_estep<1>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
+                                        lse_frame);
+    if (D <= 32) return launch_estep<2>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
+                                        lse_frame);
+    if (D <= 48) return launch_estep<3>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
+                                        lse_frame);
+    if (D <= 80) return launch_estep<5>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
+                                        lse_frame);
+    if (D <= 144) return launch_estep<9>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
+                                        lse_frame);
     set_error("dim %d > 144 is not supported by the E-step kernels", D);
     return KW_ERR_UNSUPPORTED;
 }

@@ -828,10 +828,10 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
 // below the maximum cannot change a double-precision sum and skip their exp), then
 // r = exp(wlp - lse) in place.  A thread walks K values a whole row pitch apart, so the loads are
 // issued eight at a time -- with one in flight per thread the kernel was bound by memory latency
-// (81 us for 90 MB), not by bandwidth.
+// (81 us for 90 MB), not by bandwidth.  lse_frame (may be NULL) receives each frame's lse.
 __global__ void __launch_bounds__(128)
 lse_kernel(long long N, long long Npad, int K, double* __restrict__ respT,
-           double* __restrict__ lse_partial) {
+           double* __restrict__ lse_partial, double* __restrict__ lse_frame) {
     __shared__ double sh[128];
     const long long n = (long long)blockIdx.x * 128 + threadIdx.x;
     double lse = 0.0;
@@ -866,6 +866,7 @@ lse_kernel(long long N, long long Npad, int K, double* __restrict__ respT,
             for (int j = 0; j < 8; ++j)
                 if (k0 + j < K) col[(size_t)(k0 + j) * Npad] = exp(v[j] - lse);
         }
+        if (lse_frame != nullptr) lse_frame[n] = lse;
     }
     sh[threadIdx.x] = lse;
     __syncthreads();
@@ -1950,10 +1951,12 @@ int pack_frames_tc(long long N, const double* X, int K, int D, void* workspace,
 
 // wlp (or resp, or argmax) through the tensor-core path; the frames must have been packed into
 // this workspace by pack_frames_tc.  mode 0: resp + sum of logsumexp into lse_out[0] and N into
-// lse_out[1];  mode 1: hard labels into mix (FP64 re-check of near ties).
+// lse_out[1] (with resp_form 0, each frame's logsumexp into lse_frame unless it is NULL);
+// mode 1: hard labels into mix (FP64 re-check of near ties).
 int estep_tc(long long N, const double* X, int K, int D, const double* means, const double* pc,
              const double* aux, double* resp, double* lse_out, int mode, int32_t* mix,
-             void* workspace, size_t workspace_bytes, cudaStream_t st, int resp_form) {
+             void* workspace, size_t workspace_bytes, cudaStream_t st, int resp_form,
+             double* lse_frame) {
     TcWorkspace w;
     int rc = tc_check(N, K, D, workspace, workspace_bytes, w);
     if (rc != KW_OK) return rc;
@@ -2012,7 +2015,7 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
             N, Npad, K, resp, w.lse_partial, n_mt_pad, w.tflags, w.wts, w.tsum,
             TC_TILE_FLOOR, w.tiles_per_chunk, w.item_count);
     } else {
-        tc::lse_kernel<<<lgrid, 128, 0, st>>>(N, Npad, K, resp, w.lse_partial);
+        tc::lse_kernel<<<lgrid, 128, 0, st>>>(N, Npad, K, resp, w.lse_partial, lse_frame);
     }
     KW_CUDA_CHECK(cudaGetLastError());
     launch_reduce_fixed(w.lse_partial, (long long)lgrid, (double)N, lse_out, st);
@@ -2027,7 +2030,7 @@ int normalize_resp_tc(long long N, int K, int D, double* resp, void* workspace,
     int rc = tc_check(N, K, D, workspace, workspace_bytes, w);
     if (rc != KW_OK) return rc;
     tc::lse_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(N, resp_pad(N), K, resp,
-                                                              w.lse_partial);
+                                                              w.lse_partial, nullptr);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }

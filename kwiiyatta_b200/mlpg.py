@@ -1,5 +1,6 @@
 """Posterior + MLPG on the B200 (nnmnkwii.baseline.gmm.MLPG as used at
-kwiiyatta/converter/gmm.py:28-34), optionally with global variance (``gv=``; kwiiyatta_b200.gv)."""
+kwiiyatta/converter/gmm.py:28-34), optionally with global variance (``gv=``; kwiiyatta_b200.gv)
+or maximum-likelihood conversion over all mixture sequences (``em_iter=``)."""
 import numpy as np
 
 from . import _lib
@@ -16,12 +17,31 @@ class MLPG:
     here; the reference rebuilds it on every convert call (kwiiyatta/converter/gmm.py:32)."""
 
     def __init__(self, gmm, windows=None, swap=False, diff=False, precision='auto',
-                 device=None, gv=None, gv_iter=20, gv_weights=(1.0, 1.0)):
+                 device=None, gv=None, gv_iter=20, gv_weights=(1.0, 1.0), em_iter=0):
         torch = _lib.require_cuda()
         self._dev = torch.device('cuda' if device is None else device)
         with torch.cuda.device(self._dev):      # 'cuda' without an index: the current device
             self._setup(torch, gmm, windows, swap, diff, precision)
             self._setup_gv(torch, gv, gv_iter, gv_weights)
+            self._setup_em(precision, em_iter)
+
+    def _setup_em(self, precision, em_iter):
+        """``em_iter > 0``: every transform runs ``em_iter`` EM iterations of maximum-likelihood
+        conversion over all mixture sequences (Toda, Black & Tokuda 2007), started from the
+        hard-sequence trajectory: E-step = posteriors of the joint model of [x_t ; (W y)_t],
+        M-step = MLPG with per-frame precisions.  ``em_iter = 0`` is the hard-sequence path."""
+        em_iter = int(em_iter)
+        if em_iter < 0:
+            raise ValueError(f'em_iter must be >= 0, got {em_iter}')
+        if em_iter and len(self.windows) == 1:
+            raise ValueError('EM conversion is defined for MLPG trajectories only (not with a '
+                             'single static window)')
+        if em_iter and self.gv is not None:
+            raise NotImplementedError('EM conversion together with GV is not built')
+        self.em_iter = em_iter
+        # 'auto' = the FP64 E-step for EM: soft posteriors feel the tensor-core E-step's error
+        # directly, with no FP64 re-check as the hard labels have (DESIGN.md, "Numerics")
+        self._em_precision = 0 if precision == 'auto' else self.precision
 
     def _setup_gv(self, torch, gv, gv_iter, gv_weights):
         """``gv``: GV statistics (a kwiiyatta_b200.gv.GlobalVariance, a dict with ``mean`` /
@@ -87,11 +107,18 @@ class MLPG:
                                         'definite')
 
     def _launch(self, n_utts, off_dev, total, max_frames, src, out, mix, stream,
-                gv_f=None, gv_accepted=None):
-        """kw_convert_batch, or kw_convert_gv_batch when GV statistics are set, on device
-        tensors (``src`` (total, dim_half), ``out`` (total, static_dim))."""
+                gv_f=None, gv_accepted=None, em_loglik=None):
+        """kw_convert_batch, kw_convert_gv_batch when GV statistics are set, or
+        kw_convert_em_batch when ``em_iter > 0``, on device tensors (``src`` (total, dim_half),
+        ``out`` (total, static_dim))."""
         lib = _lib.lib()
         k, dh = self.num_mixtures, self.dim_half
+        if self.em_iter:
+            ws_bytes = lib.kw_convert_em_workspace_bytes(total, k, dh, self._em_precision)
+            _lib.call('kw_convert_em_batch', n_utts, off_dev, total, src, k, dh, self._prepared,
+                      self.em_iter, out, em_loglik, self._em_precision,
+                      _lib.workspace(ws_bytes, src.device), ws_bytes, stream)
+            return
         if self.gv is None:
             ws_bytes = lib.kw_convert_workspace_bytes(total, k, dh, self.precision)
             _lib.call('kw_convert_batch', n_utts, off_dev, total, int(max_frames), src, k, dh,
@@ -107,11 +134,17 @@ class MLPG:
 
     @_on_own_device
     def transform_device(self, src_dev, offsets_dev, n_utts, max_frames, return_mix=False,
-                         return_gv_info=False):
+                         return_gv_info=False, return_em_info=False):
         """src_dev (sum T, dim_half) float64 CUDA tensor, offsets int64 (n_utts + 1).
         ``return_gv_info`` (with GV): also the final objective F and the number of accepted
-        ascent steps per (utterance, static dim), as (n_utts, static_dim) tensors."""
+        ascent steps per (utterance, static dim), as (n_utts, static_dim) tensors.
+        ``return_em_info`` (with ``em_iter > 0``): also the (n_utts, em_iter + 1) trace of the
+        objective L(y_k), k = 0 (the hard-sequence start) .. em_iter."""
         torch = _lib.require_cuda()
+        if return_mix and self.em_iter:
+            raise ValueError('return_mix: EM conversion has no single mixture sequence')
+        if return_em_info and not self.em_iter:
+            raise ValueError('return_em_info needs em_iter > 0')
         total = src_dev.shape[0]
         dev = src_dev.device
         out = torch.empty((total, self.static_dim), dtype=torch.float64, device=dev)
@@ -122,9 +155,12 @@ class MLPG:
                 raise ValueError('return_gv_info needs GV statistics')
             info = (torch.zeros((n_utts, self.static_dim), dtype=torch.float64, device=dev),
                     torch.zeros((n_utts, self.static_dim), dtype=torch.int32, device=dev))
+        loglik = (torch.zeros((n_utts, self.em_iter + 1), dtype=torch.float64, device=dev)
+                  if return_em_info else None)
         self._launch(n_utts, offsets_dev, total, max_frames, src_dev, out, mix,
-                     _lib.stream_ptr(torch), *(info or ()))
-        res = (out,) + ((mix,) if return_mix else ()) + ((info,) if return_gv_info else ())
+                     _lib.stream_ptr(torch), *(info or (None, None)), em_loglik=loglik)
+        res = (out,) + ((mix,) if return_mix else ()) + ((info,) if return_gv_info else ()) + \
+            ((loglik,) if return_em_info else ())
         return res if len(res) > 1 else out
 
     CHUNK_FRAMES = 65536       # frames per pipeline chunk (36 MB in, 12 MB out at Dh = 72)
