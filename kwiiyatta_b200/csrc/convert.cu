@@ -784,22 +784,46 @@ __global__ void convert_em_loglik_kernel(int n_utts, const int64_t* __restrict__
     if (lane == 0) out[(size_t)u * stride + col] = s;
 }
 
+// ------------------------------------------------------------------------------------------
+// Host side of the hard-sequence conversions (kw_convert_batch, kw_convert_gv_batch,
+// kw_convert_em_batch): one workspace layout, one argument check and the stages they share.
+
+enum ConvertKind { CONVERT_PLAIN, CONVERT_GV, CONVERT_EM };
+
+// The workspace of one conversion call, in this order: the hard-sequence buffers every kind uses,
+// then the GV step plane or the EM buffers, then the tensor-core region of the E-steps the call
+// runs (precision 1 only: the hard-sequence E-step at dim_half, and for EM also the E-step at
+// 2 * dim_half).
 struct ConvertWorkspace {
-    int32_t* mix;
-    int* counts;      // K
-    int* offsets;     // K + 1
-    int* blockstart;  // K + 1
-    int* cursor;      // K
-    int* order;       // total
-    double* E;
-    double* band;
-    unsigned char* flags;
+    int32_t* mix;          // (total) hard mixture sequence
+    int* counts;           // K      (counting sort of the frames by mixture)
+    int* offsets;          // K + 1
+    int* blockstart;       // K + 1
+    int* cursor;           // K
+    int* order;            // total
+    double* E;             // (total, Dh) conditional means
+    double* band;          // [a | b | c | rhs], (total, sd) each
+    unsigned char* flags;  // (total) utterance edges
+    double* step;          // GV: (total, sd) step plane
+    double* z;             // EM: (total, 2 Dh) joint frames [x | W y]
+    double* resp;          // EM: (K, resp_pad(total))
+    double* lse;           // EM: (total) per-frame log-normaliser
+    double* lsep;          // EM: E-step partial sums (at most one per frame) + the two-value total
+    double* q;             // EM: (total, Dh)
+    double* prec;          // EM: (total, Dh)
+    double* means;         // EM: (K, 2 Dh)
+    double* pc;            // EM: (K, 2 Dh, 2 Dh)
+    double* aux;           // EM: (K, 2 Dh + 2)
+    char* tc;              // tensor-core region of tc_bytes (0 at precision 0)
+    size_t tc_bytes;
     size_t bytes;
 };
 
-static ConvertWorkspace carve_convert(long long total, int K, int Dh, int sd, void* base) {
+static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, int Dh,
+                                      int precision, void* base) {
+    const int sd = Dh / 3;
     Carver c(base);
-    ConvertWorkspace w;
+    ConvertWorkspace w = {};
     w.mix = c.take<int32_t>((size_t)total);
     w.counts = c.take<int>((size_t)K);
     w.offsets = c.take<int>((size_t)K + 1);
@@ -809,8 +833,118 @@ static ConvertWorkspace carve_convert(long long total, int K, int Dh, int sd, vo
     w.E = c.take<double>((size_t)total * Dh);
     w.band = c.take<double>(4 * (size_t)total * sd);
     w.flags = c.take<unsigned char>((size_t)total);
+    if (kind == CONVERT_GV) w.step = c.take<double>((size_t)total * sd);
+    if (kind == CONVERT_EM) {
+        const size_t D = 2 * (size_t)Dh;
+        w.z = c.take<double>((size_t)total * D);
+        w.resp = c.take<double>((size_t)K * (size_t)resp_pad(total));
+        w.lse = c.take<double>((size_t)total);
+        w.lsep = c.take<double>((size_t)total + 2);
+        w.q = c.take<double>((size_t)total * Dh);
+        w.prec = c.take<double>((size_t)total * Dh);
+        w.means = c.take<double>((size_t)K * D);
+        w.pc = c.take<double>((size_t)K * D * D);
+        w.aux = c.take<double>((size_t)K * (D + 2));
+    }
+    if (precision == 1) {
+        w.tc_bytes = tc_workspace_bytes(total, K, Dh);
+        if (kind == CONVERT_EM)
+            w.tc_bytes = std::max(w.tc_bytes, tc_workspace_bytes(total, K, 2 * Dh));
+    }
+    w.tc = c.take<char>(w.tc_bytes);
     w.bytes = align_up(c.used, 256);
     return w;
+}
+
+// The arguments every conversion kind shares (the caller has returned early on an empty batch).
+// estep_dim: the largest dimension an E-step of the call runs at.
+static int check_convert(const char* fn, int n_utts, long long total, int K, int Dh, int precision,
+                         int estep_dim) {
+    KW_REQUIRE(n_utts > 0 && total > 0 && K > 0, "%s: bad sizes", fn);
+    KW_REQUIRE(Dh % 3 == 0, "%s: dim_half %d is not static+delta+delta2 (multiple of 3)", fn, Dh);
+    KW_REQUIRE(precision == 0 || precision == 1, "%s: precision must be 0 or 1", fn);
+    if (estep_dim > 144) {
+        set_error("%s: dim_half %d: the E-step at dimension %d > 144 is not supported", fn, Dh,
+                  estep_dim);
+        return KW_ERR_UNSUPPORTED;
+    }
+    KW_REQUIRE(Dh <= 80, "%s: dim_half %d > 80 unsupported", fn, Dh);
+    KW_REQUIRE(total < 2147483647LL, "%s: too many frames for one conversion batch", fn);
+    return KW_OK;
+}
+
+static int workspace_too_small(const char* fn, size_t need, size_t got) {
+    set_error("%s: workspace too small: need %zu bytes, got %zu", fn, need, got);
+    return KW_ERR_WORKSPACE;
+}
+
+static const Windows kDeltaWindows = {{{0.0, 1.0, 0.0}, {-0.5, 0.0, 0.5}, {1.0, -2.0, 1.0}}};
+
+// The hard mixture sequence (the E-step in label mode) into w.mix, then the conditional means of
+// the frames under it into w.E: a counting sort of the frames by mixture (histogram, scan,
+// scatter) and one pass per mixture.
+static int hard_sequence(long long total, const double* src, int K, int Dh, int precision,
+                         const PreparedView& v, const ConvertWorkspace& w, cudaStream_t st) {
+    int rc;
+    if (precision == 1) {
+        rc = pack_frames_tc(total, src, K, Dh, w.tc, w.tc_bytes, st, /*mstep_parts=*/false);
+        if (rc != KW_OK) return rc;
+        rc = estep_tc(total, src, K, Dh, v.src_means, v.px_prec_chol, v.px_aux, nullptr, nullptr,
+                      1, w.mix, w.tc, w.tc_bytes, st);
+    } else {
+        rc = estep_fp64(total, src, K, Dh, v.px_prec_chol, v.px_aux, nullptr, nullptr, 1, w.mix,
+                        st);
+    }
+    if (rc != KW_OK) return rc;
+    KW_CUDA_CHECK(cudaMemsetAsync(w.counts, 0, sizeof(int) * K, st));
+    convert_hist_kernel<<<296, 256, sizeof(int) * K, st>>>(total, K, w.mix, w.counts);
+    KW_CUDA_CHECK(cudaGetLastError());
+    convert_scan_kernel<<<1, 32, 0, st>>>(K, w.counts, w.offsets, w.blockstart, w.cursor);
+    KW_CUDA_CHECK(cudaGetLastError());
+    convert_scatter_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
+        total, w.mix, w.offsets, w.cursor, w.order);
+    KW_CUDA_CHECK(cudaGetLastError());
+    const size_t smem = sizeof(double) * ((size_t)Dh * Dh + (size_t)CM_FT * (Dh + 1));
+    KW_CUDA_CHECK(cudaFuncSetAttribute(convert_condmean_kernel,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const long long max_blocks = (total + CM_FT - 1) / CM_FT + K;
+    convert_condmean_kernel<<<(unsigned)max_blocks, 256, smem, st>>>(
+        K, Dh, src, w.offsets, w.blockstart, w.order, v, w.E);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+static int utterance_flags(int n_utts, const int64_t* off, long long total,
+                           const ConvertWorkspace& w, cudaStream_t st) {
+    KW_CUDA_CHECK(cudaMemsetAsync(w.flags, 0, (size_t)total, st));
+    convert_flags_kernel<<<(n_utts + 127) / 128, 128, 0, st>>>(n_utts, off, w.flags);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+// The MLPG normal equations into w.band: from the conditional means w.E under the mixture
+// sequence w.mix (FRAME_PREC false), or from the EM M-step's per-frame w.q and w.prec (true).
+template <bool FRAME_PREC>
+static int build_band(long long total, int Dh, const PreparedView& v, const ConvertWorkspace& w,
+                      cudaStream_t st) {
+    const int sd = Dh / 3;
+    const long long cells = total * sd;
+    convert_band_kernel<FRAME_PREC><<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
+        total, sd, Dh, FRAME_PREC ? w.q : w.E, FRAME_PREC ? nullptr : w.mix,
+        FRAME_PREC ? w.prec : v.var, w.flags, kDeltaWindows, w.band);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+// Solves the equations in w.band (factoring them in place) into out.
+static int solve_mlpg(int n_utts, const int64_t* off, long long total, int Dh,
+                      const ConvertWorkspace& w, double* out, cudaStream_t st) {
+    const int sd = Dh / 3;
+    const long long threads = (long long)n_utts * sd;
+    convert_mlpg_kernel<<<(unsigned)((threads + 95) / 96), 96, 0, st>>>(n_utts, off, sd, w.band,
+                                                                        total, out);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
 }
 
 }  // namespace kw
@@ -873,97 +1007,31 @@ extern "C" int kw_convert_soft_batch(int64_t total, const double* src_dev, int K
 }
 
 extern "C" size_t kw_convert_workspace_bytes(int64_t total_frames, int K, int Dh, int precision) {
-    size_t b = carve_convert(total_frames, K, Dh, Dh / 3, nullptr).bytes;
-    if (precision == 1) b += tc_workspace_bytes(total_frames, K, Dh);
-    return b;
+    return carve_convert(CONVERT_PLAIN, total_frames, K, Dh, precision, nullptr).bytes;
 }
-
-// Posterior, conditional means, normal equations and their solve into out_dev; `*wout` (may be
-// NULL) receives the workspace layout, whose E / mix / flags / band stay valid after the call.
-static int convert_run(int n_utts, const int64_t* off_dev, int64_t total, const double* src_dev,
-                       int K, int Dh, const double* prepared_dev, double* out_dev,
-                       int32_t* mix_dev, int precision, void* workspace_dev,
-                       size_t workspace_bytes, cudaStream_t st, ConvertWorkspace* wout);
-
-static const Windows kDeltaWindows = {{{0.0, 1.0, 0.0}, {-0.5, 0.0, 0.5}, {1.0, -2.0, 1.0}}};
 
 extern "C" int kw_convert_batch(int n_utts, const int64_t* off_dev, int64_t total, int max_frames,
                                 const double* src_dev, int K, int Dh, const double* prepared_dev,
                                 double* out_dev, int32_t* mix_dev, int precision,
                                 void* workspace_dev, size_t workspace_bytes, void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
     (void)max_frames;
     if (n_utts == 0 || total == 0) return KW_OK;
-    return convert_run(n_utts, off_dev, total, src_dev, K, Dh, prepared_dev, out_dev, mix_dev,
-                       precision, workspace_dev, workspace_bytes,
-                       static_cast<cudaStream_t>(stream), nullptr);
-}
-
-static int convert_run(int n_utts, const int64_t* off_dev, int64_t total, const double* src_dev,
-                       int K, int Dh, const double* prepared_dev, double* out_dev,
-                       int32_t* mix_dev, int precision, void* workspace_dev,
-                       size_t workspace_bytes, cudaStream_t st, ConvertWorkspace* wout) {
-    KW_REQUIRE(n_utts > 0 && total > 0 && K > 0, "kw_convert_batch: bad sizes");
-    KW_REQUIRE(Dh % 3 == 0, "dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
-    KW_REQUIRE(precision == 0 || precision == 1, "convert precision must be 0 or 1");
-    const int sd = Dh / 3;
-    ConvertWorkspace w = carve_convert(total, K, Dh, sd, workspace_dev);
-    if (w.bytes > workspace_bytes) {
-        set_error("convert workspace too small: need %zu bytes, got %zu", w.bytes,
-                  workspace_bytes);
-        return KW_ERR_WORKSPACE;
-    }
-    PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
-    int rc;
-    if (precision == 1) {
-        rc = pack_frames_tc(total, src_dev, K, Dh, static_cast<char*>(workspace_dev) + w.bytes,
-                            workspace_bytes - w.bytes, st, /*mstep_parts=*/false);
-        if (rc != KW_OK) return rc;
-    }
-    if (precision == 1)
-        rc = estep_tc(total, src_dev, K, Dh, v.src_means, v.px_prec_chol, v.px_aux, nullptr,
-                      nullptr, 1, w.mix, static_cast<char*>(workspace_dev) + w.bytes,
-                      workspace_bytes - w.bytes, st);
-    else
-        rc = estep_fp64(total, src_dev, K, Dh, v.px_prec_chol, v.px_aux, nullptr, nullptr, 1,
-                        w.mix, st);
+    int rc = check_convert("kw_convert_batch", n_utts, total, K, Dh, precision, Dh);
     if (rc != KW_OK) return rc;
-    {
-        KW_REQUIRE(Dh <= 80, "dim_half %d > 80 unsupported", Dh);
-        KW_REQUIRE(total < 2147483647LL, "too many frames for one conversion batch");
-        KW_CUDA_CHECK(cudaMemsetAsync(w.counts, 0, sizeof(int) * K, st));
-        convert_hist_kernel<<<296, 256, sizeof(int) * K, st>>>(total, K, w.mix, w.counts);
-        KW_CUDA_CHECK(cudaGetLastError());
-        convert_scan_kernel<<<1, 32, 0, st>>>(K, w.counts, w.offsets, w.blockstart, w.cursor);
-        KW_CUDA_CHECK(cudaGetLastError());
-        convert_scatter_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
-            total, w.mix, w.offsets, w.cursor, w.order);
-        KW_CUDA_CHECK(cudaGetLastError());
-        const size_t smem = sizeof(double) * ((size_t)Dh * Dh + (size_t)CM_FT * (Dh + 1));
-        KW_CUDA_CHECK(cudaFuncSetAttribute(convert_condmean_kernel,
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        const long long max_blocks = (total + CM_FT - 1) / CM_FT + K;
-        convert_condmean_kernel<<<(unsigned)max_blocks, 256, smem, st>>>(
-            K, Dh, src_dev, w.offsets, w.blockstart, w.order, v, w.E);
-        KW_CUDA_CHECK(cudaGetLastError());
-    }
-    {
-        const Windows win = kDeltaWindows;
-        KW_CUDA_CHECK(cudaMemsetAsync(w.flags, 0, (size_t)total, st));
-        convert_flags_kernel<<<(n_utts + 127) / 128, 128, 0, st>>>(n_utts, off_dev, w.flags);
-        KW_CUDA_CHECK(cudaGetLastError());
-        const long long cells = total * sd;
-        convert_band_kernel<false><<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
-            total, sd, Dh, w.E, w.mix, v.var, w.flags, win, w.band);
-        KW_CUDA_CHECK(cudaGetLastError());
-        const long long threads = (long long)n_utts * sd;
-        convert_mlpg_kernel<<<(unsigned)((threads + 95) / 96), 96, 0, st>>>(
-            n_utts, off_dev, sd, w.band, total, out_dev);
-        KW_CUDA_CHECK(cudaGetLastError());
-    }
+    const ConvertWorkspace w =
+        carve_convert(CONVERT_PLAIN, total, K, Dh, precision, workspace_dev);
+    if (w.bytes > workspace_bytes)
+        return workspace_too_small("kw_convert_batch", w.bytes, workspace_bytes);
+    const PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    rc = hard_sequence(total, src_dev, K, Dh, precision, v, w, st);
+    if (rc == KW_OK) rc = utterance_flags(n_utts, off_dev, total, w, st);
+    if (rc == KW_OK) rc = build_band<false>(total, Dh, v, w, st);
+    if (rc == KW_OK) rc = solve_mlpg(n_utts, off_dev, total, Dh, w, out_dev, st);
+    if (rc != KW_OK) return rc;
     if (mix_dev != nullptr)
         KW_CUDA_CHECK(cudaMemcpyAsync(mix_dev, w.mix, sizeof(int32_t) * total,
                                       cudaMemcpyDeviceToDevice, st));
-    if (wout != nullptr) *wout = w;
     return KW_OK;
 }
 
@@ -993,15 +1061,9 @@ extern "C" int kw_gv_from_sums(int ncols, const double* sums_dev, double* mean_d
     return KW_OK;
 }
 
-// GV workspace: [ step plane (total, sd) | the kw_convert_batch workspace ].
-static size_t gv_step_bytes(int64_t total, int sd) {
-    return align_up(sizeof(double) * (size_t)total * sd, 256);
-}
-
 extern "C" size_t kw_convert_gv_workspace_bytes(int64_t total_frames, int K, int Dh,
                                                 int precision) {
-    return gv_step_bytes(total_frames, Dh / 3) +
-           kw_convert_workspace_bytes(total_frames, K, Dh, precision);
+    return carve_convert(CONVERT_GV, total_frames, K, Dh, precision, nullptr).bytes;
 }
 
 extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t total,
@@ -1014,31 +1076,32 @@ extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t t
                                    size_t workspace_bytes, void* stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (n_utts == 0 || total == 0) return KW_OK;
-    KW_REQUIRE(Dh % 3 == 0, "dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
+    int rc = check_convert("kw_convert_gv_batch", n_utts, total, K, Dh, precision, Dh);
+    if (rc != KW_OK) return rc;
     KW_REQUIRE(gv_iter >= 0 && w_traj > 0.0 && w_gv >= 0.0,
                "kw_convert_gv_batch: need gv_iter >= 0, w_traj > 0, w_gv >= 0");
     const int sd = Dh / 3;
-    KW_REQUIRE(static_src_dev == nullptr || static_ld >= sd, "static_ld %d < static_dim %d",
-               static_ld, sd);
-    KW_REQUIRE((long long)n_utts * sd < 2147483647LL, "too many utterances for one batch");
-    const size_t sbytes = gv_step_bytes(total, sd);
-    if (kw_convert_gv_workspace_bytes(total, K, Dh, precision) > workspace_bytes) {
-        set_error("GV convert workspace too small");
-        return KW_ERR_WORKSPACE;
-    }
-    ConvertWorkspace w;
-    int rc = convert_run(n_utts, off_dev, total, src_dev, K, Dh, prepared_dev, out_dev, mix_dev,
-                         precision, static_cast<char*>(workspace_dev) + sbytes,
-                         workspace_bytes - sbytes, st, &w);
+    KW_REQUIRE(static_src_dev == nullptr || static_ld >= sd,
+               "kw_convert_gv_batch: static_ld %d < static_dim %d", static_ld, sd);
+    KW_REQUIRE((long long)n_utts * sd < 2147483647LL,
+               "kw_convert_gv_batch: too many utterances for one batch");
+    const ConvertWorkspace w = carve_convert(CONVERT_GV, total, K, Dh, precision, workspace_dev);
+    if (w.bytes > workspace_bytes)
+        return workspace_too_small("kw_convert_gv_batch", w.bytes, workspace_bytes);
+    const PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    rc = hard_sequence(total, src_dev, K, Dh, precision, v, w, st);
+    if (rc == KW_OK) rc = utterance_flags(n_utts, off_dev, total, w, st);
+    if (rc == KW_OK) rc = build_band<false>(total, Dh, v, w, st);
+    if (rc == KW_OK) rc = solve_mlpg(n_utts, off_dev, total, Dh, w, out_dev, st);
     if (rc != KW_OK) return rc;
-    // convert_mlpg_kernel factored the bands in place: rebuild them (the band kernel is a pure
-    // function of E, the mixture sequence and the flags, all still in the workspace), which moves
-    // the same bytes as a saved copy would and keeps the workspace at one band set
-    PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
-    const long long cells = total * sd;
-    convert_band_kernel<false><<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
-        total, sd, Dh, w.E, w.mix, v.var, w.flags, kDeltaWindows, w.band);
-    KW_CUDA_CHECK(cudaGetLastError());
+    if (mix_dev != nullptr)
+        KW_CUDA_CHECK(cudaMemcpyAsync(mix_dev, w.mix, sizeof(int32_t) * total,
+                                      cudaMemcpyDeviceToDevice, st));
+    // the solve factored the bands in place: rebuild them (the band kernel is a pure function of
+    // E, the mixture sequence and the flags, all still in the workspace), which moves the same
+    // bytes as a saved copy would and keeps the workspace at one band set
+    rc = build_band<false>(total, Dh, v, w, st);
+    if (rc != KW_OK) return rc;
     GvArgs g;
     g.off = off_dev;
     g.n_utts = n_utts;
@@ -1052,7 +1115,7 @@ extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t t
     g.s = static_src_dev;
     g.s_ld = static_ld;
     g.band = w.band;
-    g.step = static_cast<double*>(workspace_dev);
+    g.step = w.step;
     g.out = out_dev;
     g.total = total;
     g.f_out = f_dev;
@@ -1065,46 +1128,9 @@ extern "C" int kw_convert_gv_batch(int n_utts, const int64_t* off_dev, int64_t t
     return KW_OK;
 }
 
-// EM workspace: [ EmWorkspace | the kw_convert_batch workspace at precision 0 | the tensor-core
-// workspace of the larger of the two E-steps (precision 1) ].
-struct EmWorkspace {
-    double* z;      // (total, 2 Dh) joint frames [x | W y]
-    double* resp;   // (K, resp_pad(total))
-    double* lse;    // (total) per-frame log-normaliser
-    double* lsep;   // E-step partial sums (at most one per frame) + the two-value total
-    double* q;      // (total, Dh)
-    double* prec;   // (total, Dh)
-    double* means;  // (K, 2 Dh)
-    double* pc;     // (K, 2 Dh, 2 Dh)
-    double* aux;    // (K, 2 Dh + 2)
-    size_t bytes;
-};
-
-static EmWorkspace carve_em(long long total, int K, int Dh, void* base) {
-    Carver c(base);
-    EmWorkspace w;
-    const size_t D = 2 * (size_t)Dh;
-    w.z = c.take<double>((size_t)total * D);
-    w.resp = c.take<double>((size_t)K * (size_t)resp_pad(total));
-    w.lse = c.take<double>((size_t)total);
-    w.lsep = c.take<double>((size_t)total + 2);
-    w.q = c.take<double>((size_t)total * Dh);
-    w.prec = c.take<double>((size_t)total * Dh);
-    w.means = c.take<double>((size_t)K * D);
-    w.pc = c.take<double>((size_t)K * D * D);
-    w.aux = c.take<double>((size_t)K * (D + 2));
-    w.bytes = align_up(c.used, 256);
-    return w;
-}
-
 extern "C" size_t kw_convert_em_workspace_bytes(int64_t total_frames, int K, int Dh,
                                                 int precision) {
-    size_t b = carve_em(total_frames, K, Dh, nullptr).bytes +
-               carve_convert(total_frames, K, Dh, Dh / 3, nullptr).bytes;
-    if (precision == 1)
-        b += std::max(tc_workspace_bytes(total_frames, K, Dh),
-                      tc_workspace_bytes(total_frames, K, 2 * Dh));
-    return b;
+    return carve_convert(CONVERT_EM, total_frames, K, Dh, precision, nullptr).bytes;
 }
 
 extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t total,
@@ -1114,7 +1140,8 @@ extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t t
                                    size_t workspace_bytes, void* stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     KW_REQUIRE(em_iter >= 1, "kw_convert_em_batch: em_iter must be at least 1, got %d", em_iter);
-    KW_REQUIRE(Dh % 3 == 0, "dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
+    KW_REQUIRE(Dh % 3 == 0,
+               "kw_convert_em_batch: dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
     KW_REQUIRE(n_utts >= 0 && total >= 0 && K > 0, "kw_convert_em_batch: bad sizes");
     if (n_utts == 0) return KW_OK;
     if (total == 0) {
@@ -1123,53 +1150,43 @@ extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t t
                                           sizeof(double) * (size_t)n_utts * (em_iter + 1), st));
         return KW_OK;
     }
-    if (2 * Dh > 144) {
-        set_error("dim_half %d: the EM E-step runs at 2 * dim_half <= 144", Dh);
-        return KW_ERR_UNSUPPORTED;
-    }
-    KW_REQUIRE(precision == 0 || precision == 1, "convert precision must be 0 or 1");
-    if (kw_convert_em_workspace_bytes(total, K, Dh, precision) > workspace_bytes) {
-        set_error("EM convert workspace too small");
-        return KW_ERR_WORKSPACE;
-    }
-    const int sd = Dh / 3, D = 2 * Dh;
-    EmWorkspace em = carve_em(total, K, Dh, workspace_dev);
-    ConvertWorkspace w;
-    int rc = convert_run(n_utts, off_dev, total, src_dev, K, Dh, prepared_dev, out_dev, nullptr,
-                         precision, static_cast<char*>(workspace_dev) + em.bytes,
-                         workspace_bytes - em.bytes, st, &w);
+    int rc = check_convert("kw_convert_em_batch", n_utts, total, K, Dh, precision, 2 * Dh);
     if (rc != KW_OK) return rc;
-    // convert_run left the flags in its workspace; its tensor-core region follows it
-    char* tcw = static_cast<char*>(workspace_dev) + em.bytes + w.bytes;
-    const size_t tcb = workspace_bytes - em.bytes - w.bytes;
-    PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
-    convert_em_model_kernel<<<K, 256, 0, st>>>(Dh, v, em.means, em.pc, em.aux);
+    const ConvertWorkspace w = carve_convert(CONVERT_EM, total, K, Dh, precision, workspace_dev);
+    if (w.bytes > workspace_bytes)
+        return workspace_too_small("kw_convert_em_batch", w.bytes, workspace_bytes);
+    const PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    rc = hard_sequence(total, src_dev, K, Dh, precision, v, w, st);
+    if (rc == KW_OK) rc = utterance_flags(n_utts, off_dev, total, w, st);
+    if (rc == KW_OK) rc = build_band<false>(total, Dh, v, w, st);
+    if (rc == KW_OK) rc = solve_mlpg(n_utts, off_dev, total, Dh, w, out_dev, st);
+    if (rc != KW_OK) return rc;
+    const int sd = Dh / 3, D = 2 * Dh;
+    convert_em_model_kernel<<<K, 256, 0, st>>>(Dh, v, w.means, w.pc, w.aux);
     KW_CUDA_CHECK(cudaGetLastError());
-    KW_CUDA_CHECK(cudaMemcpy2DAsync(em.z, sizeof(double) * D, src_dev, sizeof(double) * Dh,
+    KW_CUDA_CHECK(cudaMemcpy2DAsync(w.z, sizeof(double) * D, src_dev, sizeof(double) * Dh,
                                     sizeof(double) * Dh, (size_t)total, cudaMemcpyDeviceToDevice,
                                     st));
     const long long cells = total * sd;
-    const unsigned cell_blocks = (unsigned)((cells + 255) / 256);
-    // E-step at y = out_dev: responsibilities into em.resp, log-normalisers into em.lse and, when
+    // E-step at y = out_dev: responsibilities into w.resp, log-normalisers into w.lse and, when
     // asked, their per-utterance sums into column `col` of the trace
     auto estep = [&](int col) -> int {
-        convert_em_frames_kernel<<<cell_blocks, 256, 0, st>>>(total, sd, out_dev, w.flags,
-                                                               kDeltaWindows, D, Dh, em.z);
+        convert_em_frames_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
+            total, sd, out_dev, w.flags, kDeltaWindows, D, Dh, w.z);
         KW_CUDA_CHECK(cudaGetLastError());
         int r;
         if (precision == 1) {
-            r = pack_frames_tc(total, em.z, K, D, tcw, tcb, st, /*mstep_parts=*/false);
+            r = pack_frames_tc(total, w.z, K, D, w.tc, w.tc_bytes, st, /*mstep_parts=*/false);
             if (r != KW_OK) return r;
-            r = estep_tc(total, em.z, K, D, em.means, em.pc, em.aux, em.resp, em.lsep, 0, nullptr,
-                         tcw, tcb, st, 0, em.lse);
+            r = estep_tc(total, w.z, K, D, w.means, w.pc, w.aux, w.resp, w.lsep, 0, nullptr, w.tc,
+                         w.tc_bytes, st, 0, w.lse);
         } else {
-            r = estep_fp64(total, em.z, K, D, em.pc, em.aux, em.resp, em.lsep, 0, nullptr, st,
-                           em.lse);
+            r = estep_fp64(total, w.z, K, D, w.pc, w.aux, w.resp, w.lsep, 0, nullptr, st, w.lse);
         }
         if (r != KW_OK) return r;
         if (loglik_dev != nullptr) {
             convert_em_loglik_kernel<<<(unsigned)((32LL * n_utts + 255) / 256), 256, 0, st>>>(
-                n_utts, off_dev, em.lse, em_iter + 1, col, loglik_dev);
+                n_utts, off_dev, w.lse, em_iter + 1, col, loglik_dev);
             KW_CUDA_CHECK(cudaGetLastError());
         }
         return KW_OK;
@@ -1179,17 +1196,12 @@ extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t t
         rc = estep(it);
         if (rc != KW_OK) return rc;
         convert_soft_kernel<true><<<(unsigned)((total + SOFT_FT - 1) / SOFT_FT), 96, soft_smem,
-                                    st>>>(total, resp_pad(total), K, Dh, src_dev, em.resp, v, em.q,
-                                          em.prec);
+                                    st>>>(total, resp_pad(total), K, Dh, src_dev, w.resp, v, w.q,
+                                          w.prec);
         KW_CUDA_CHECK(cudaGetLastError());
-        convert_band_kernel<true><<<cell_blocks, 256, 0, st>>>(total, sd, Dh, em.q, nullptr,
-                                                               em.prec, w.flags, kDeltaWindows,
-                                                               w.band);
-        KW_CUDA_CHECK(cudaGetLastError());
-        const long long threads = (long long)n_utts * sd;
-        convert_mlpg_kernel<<<(unsigned)((threads + 95) / 96), 96, 0, st>>>(
-            n_utts, off_dev, sd, w.band, total, out_dev);
-        KW_CUDA_CHECK(cudaGetLastError());
+        rc = build_band<true>(total, Dh, v, w, st);
+        if (rc == KW_OK) rc = solve_mlpg(n_utts, off_dev, total, Dh, w, out_dev, st);
+        if (rc != KW_OK) return rc;
     }
     if (loglik_dev != nullptr) return estep(em_iter);
     return KW_OK;

@@ -112,6 +112,34 @@ def test_errors(cuda):
         MLPG(_Model(w, m, c)).transform(np.zeros((5, 71)))
 
 
+@pytest.mark.parametrize('precision', [0, 1])
+@pytest.mark.parametrize('entry', ['kw_convert_batch', 'kw_convert_gv_batch'])
+def test_rejected_call_enqueues_nothing(cuda, entry, precision):
+    """dim_half 84 is past what the conditional-mean kernel holds (80) but within the E-step's
+    limit (144): the call raises before it queues any work, so the workspace keeps its bytes."""
+    from kwiiyatta_b200 import _lib
+    torch = cuda
+    k, dh, sd, total = 4, 84, 28, 40
+    w, m, c = synth.make_joint_gmm(k, dim_half=dh, seed=5, static_dim=sd)
+    paramgen = MLPG(_Model(w, m, c), precision=precision)
+    x = torch.from_numpy(np.random.default_rng(5).standard_normal((total, dh))).cuda()
+    off = torch.tensor([0, 15, total], dtype=torch.int64, device='cuda')
+    out = torch.zeros((total, sd), dtype=torch.float64, device='cuda')
+    ones = torch.ones(sd, dtype=torch.float64, device='cuda')
+    nbytes = getattr(_lib.lib(), entry.replace('_batch', '_workspace_bytes'))(total, k, dh,
+                                                                             precision)
+    ws = torch.full((nbytes,), 0xA5, dtype=torch.uint8, device='cuda')
+    head = (2, off, total, 25, x, k, dh, paramgen._prepared)
+    tail = (precision, ws, nbytes, _lib.stream_ptr(torch))
+    args = {'kw_convert_batch': head + (out, None) + tail,
+            'kw_convert_gv_batch': head + (ones, ones, 20, 1.0, 1.0, None, dh, out, None, None,
+                                           None) + tail}[entry]
+    with pytest.raises(ValueError, match='dim_half 84 > 80'):
+        _lib.call(entry, *args)
+    torch.cuda.synchronize()
+    assert bool((ws == 0xA5).all())
+
+
 def test_mc2b_hand_off_to_the_mlsa_filter(cuda):
     """pysptk.mc2b as called at kwiiyatta/filter/mlsa.py:23-29 (power coefficient zeroed first)."""
     import kwiiyatta_b200 as kw
