@@ -260,6 +260,41 @@ int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t total_frames
                         double* loglik_dev, int precision, void* workspace_dev,
                         size_t workspace_bytes, void* stream);
 
+/* Full conditional covariance (the ML trajectory of Toda, Black & Tokuda, IEEE TASLP 15(8), 2007;
+ * oracle/mlpg_full_ref.py).  The hard-sequence conversion of kw_convert_batch with the full
+ * conditional covariance Sigma_m = S_yy - A_m S_xy of each mixture (after the diff rewrite) in place
+ * of the diagonal table `var`: y = argmax sum_t log N((W y)_t; E_{m_t,t}, Sigma_{m_t}), the
+ * block-pentadiagonal SPD system R y = r with static_dim x static_dim blocks (static dimensions
+ * coupled), solved per utterance by a block Cholesky factorisation.
+ *
+ * kw_convert_fullcov_prepare derives the `fullcov` block (device, float64, length
+ * kw_convert_fullcov_prepared_len) from the covariances and a `prepared` block made by
+ * kw_convert_prepare with the same dim_half and diff (neither is changed):
+ *   [ G (K, 6, sd, sd): the six distinct blocks sum_{w,v} c[w][a+1] c[v][b+1] P^(w,v) of
+ *     P = Sigma^-1 | B^T (K,Dh,Dh), B = P A | h (K,Dh) = P offset ]
+ * Sigma and its factorisation live in a workspace of kw_convert_fullcov_prepare_workspace_bytes
+ * that the call no longer needs once it has completed on `stream`.  info_dev (K) int32 is
+ * non-zero where Sigma_k is not positive definite.  dim_half a multiple of 3 and <= 80.
+ * kw_convert_fullcov_batch takes kw_convert_batch's arguments plus that block and writes the same
+ * outputs (mix_dev may be NULL); max_frames is unused, as in kw_convert_batch, and bounds
+ * nothing.  Workspace (kw_convert_fullcov_workspace_bytes): the block
+ * factors kept between the forward and the backward sweep, 8 (3 sd^2 + sd) bytes per frame
+ * (14 KB at sd = 24, where the diagonal path's band takes 768 B), plus what kw_convert_batch
+ * needs besides its band. */
+size_t kw_convert_fullcov_prepared_len(int n_components, int dim_half);
+size_t kw_convert_fullcov_prepare_workspace_bytes(int n_components, int dim_half);
+int kw_convert_fullcov_prepare(int n_components, int dim_half, int diff,
+                               const double* covariances_dev, const double* prepared_dev,
+                               double* fullcov_dev, int32_t* info_dev, void* workspace_dev,
+                               size_t workspace_bytes, void* stream);
+size_t kw_convert_fullcov_workspace_bytes(int64_t total_frames, int n_components, int dim_half,
+                                          int precision);
+int kw_convert_fullcov_batch(int n_utts, const int64_t* off_dev, int64_t total_frames,
+                             int max_frames, const double* src_dev, int n_components,
+                             int dim_half, const double* prepared_dev, const double* fullcov_dev,
+                             double* out_dev, int32_t* mix_dev, int precision,
+                             void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* Soft-posterior mapping without MLPG (nnmnkwii MLPGBase.transform; the mlpg=False branch of
  * kwiiyatta/converter/gmm.py:30-31): out (total, dim_half) = sum_m p(m|x) (mu_y + S_yx S_xx^-1 (x - mu_x)).
  * `prepared_dev` comes from kw_convert_prepare with the same dim_half. */

@@ -58,6 +58,12 @@ SIGNATURES = {
     'kw_convert_em_workspace_bytes': (_sz, [_i64, _i, _i, _i]),
     'kw_convert_em_batch': (_i, [_i, _vp, _i64, _vp, _i, _i, _vp, _i, _vp, _vp, _i, _vp, _sz,
                                  _vp]),
+    'kw_convert_fullcov_prepared_len': (_sz, [_i, _i]),
+    'kw_convert_fullcov_prepare_workspace_bytes': (_sz, [_i, _i]),
+    'kw_convert_fullcov_prepare': (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kw_convert_fullcov_workspace_bytes': (_sz, [_i64, _i, _i, _i]),
+    'kw_convert_fullcov_batch': (_i, [_i, _vp, _i64, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _i,
+                                      _vp, _sz, _vp]),
 }
 
 

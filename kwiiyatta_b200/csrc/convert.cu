@@ -8,9 +8,14 @@
 //   y[:, d] = solve( W^T D^-1 W , W^T D^-1 E )  per static dim d, pentadiagonal SPD system,
 //   windows = kwiiyatta DELTA_WINDOWS (kwiiyatta/converter/delta.py:8-12).
 // Beyond the reference: global-variance (GV) statistics and GV-considered generation on the same
-// normal equations (kw_gv_estimate, kw_convert_gv_batch; restated in oracle/gv_ref.py), and
+// normal equations (kw_gv_estimate, kw_convert_gv_batch; restated in oracle/gv_ref.py),
 // maximum-likelihood conversion over all mixture sequences by EM (kw_convert_em_batch; restated
-// in oracle/mlpg_em_ref.py).
+// in oracle/mlpg_em_ref.py), and the ML trajectory under the full conditional covariance
+//   Sigma_m = S_yy - A_m S_xy  (Dh x Dh) in place of D_m, a block-pentadiagonal system with
+// sd x sd blocks solved by a block Cholesky sweep per utterance (kw_convert_fullcov_batch;
+// restated in oracle/mlpg_full_ref.py).  Its workspace keeps the block factors between the
+// forward and the backward sweep: (3 sd^2 + sd) doubles per frame, 14 KB at sd = 24, where the
+// diagonal path's band takes 768 B.
 #include <algorithm>
 
 #include "common.cuh"
@@ -785,15 +790,310 @@ __global__ void convert_em_loglik_kernel(int n_utts, const int64_t* __restrict__
 }
 
 // ------------------------------------------------------------------------------------------
+// Full conditional covariance (the ML trajectory of Toda, Black & Tokuda, IEEE TASLP 15(8), 2007;
+// restated in oracle/mlpg_full_ref.py).  Per mixture Sigma_m = S_yy - A_m S_xy (Dh x Dh, after
+// the diff rewrite), P_m = Sigma_m^-1 in 3 x 3 blocks P^(w,v) of sd x sd, and
+//   G_m[a][b] = sum_{w,v} c[w][a+1] c[v][b+1] P^(w,v),   a, b in {-1, 0, 1}
+// frame t adds G_{m_t}[a][b] to block (t+a, t+b) of R and sum_w c[w][a+1] g_t^(w) to block row
+// t+a of r, g_t = P E_t = h_m + B_m x_t (B = P A, h = P offset); blocks outside [0, T) are
+// dropped.  R y = r is block-pentadiagonal SPD with sd x sd blocks and couples the static
+// dimensions, which the diagonal path (convert_band_kernel / convert_mlpg_kernel) solves apart.
+
+// The fullcov block (kw_convert_fullcov_prepare), separate from the prepared block.
+struct FullcovView {
+    double* g;       // (K, FC_NG, sd, sd) G blocks, each column-major: [l * sd + k] = G[k][l]
+    double* bt;      // (K, Dh, Dh) B^T, the layout of PreparedView::at
+    double* h;       // (K, Dh)
+    size_t len;
+};
+
+// The workspace of kw_convert_fullcov_prepare.
+struct FullcovScratch {
+    double* sigma;   // (K, Dh, Dh) Sigma
+    double* pc;      // (K, Dh, Dh) precision Cholesky of Sigma (upper, P = pc pc^T)
+    double* aux;     // (K, Dh + 2) by-product of the factorisation, unused
+    double* ones;    // (K) unit weights for the factorisation
+    size_t bytes;
+};
+
+static FullcovScratch carve_fullcov_scratch(int K, int Dh, void* base) {
+    Carver c(base);
+    FullcovScratch w;
+    w.sigma = c.take<double>((size_t)K * Dh * Dh);
+    w.pc = c.take<double>((size_t)K * Dh * Dh);
+    w.aux = c.take<double>((size_t)K * (Dh + 2));
+    w.ones = c.take<double>((size_t)K);
+    w.bytes = align_up(c.used, 256);
+    return w;
+}
+
+// The six distinct G blocks (G[b][a] = G[a][b]^T) in the order a frame's solve step reads them.
+enum { FC_GMM, FC_G00, FC_GPP, FC_GP0, FC_G0M, FC_GPM, FC_NG };
+
+static FullcovView view_fullcov(double* base, int K, int Dh) {
+    FullcovView f;
+    const int sd = Dh / 3;
+    const size_t kdd = (size_t)K * Dh * Dh;
+    size_t o = 0;
+    f.g = base + o;     o += (size_t)K * FC_NG * sd * sd;
+    f.bt = base + o;    o += kdd;
+    f.h = base + o;     o += (size_t)K * Dh;
+    f.len = o;
+    return f;
+}
+
+// Sigma = S_yy - A S_xy, with the diff rewrite S_yy <- S_xx + S_yy - S_xy - S_yx,
+// S_xy <- S_xy - S_xx.  One CTA per mixture.
+__global__ void convert_fullcov_sigma_kernel(int Dh, int diff, const double* __restrict__ cov,
+                                             PreparedView v, FullcovScratch w) {
+    const int k = blockIdx.x;
+    const int D = 2 * Dh;
+    const double* C = cov + (size_t)k * D * D;
+    const double* at = v.at + (size_t)k * Dh * Dh;
+    for (int e = threadIdx.x; e < Dh * Dh; e += blockDim.x) {
+        const int r = e / Dh, c = e - r * Dh;
+        double s = C[(size_t)(Dh + r) * D + Dh + c];
+        if (diff) s = C[(size_t)r * D + c] + s - C[(size_t)r * D + Dh + c] - C[(size_t)(Dh + r) * D + c];
+        for (int q = 0; q < Dh; ++q) {
+            double sxy = C[(size_t)q * D + Dh + c];
+            if (diff) sxy -= C[(size_t)q * D + c];
+            s = fma(-at[(size_t)q * Dh + r], sxy, s);
+        }
+        w.sigma[(size_t)k * Dh * Dh + e] = s;
+    }
+    if (threadIdx.x == 0) w.ones[k] = 1.0;
+}
+
+// P = pc pc^T, then the G blocks, B^T and h of one mixture.  One CTA per mixture, P in shared
+// memory.
+__global__ void convert_fullcov_tables_kernel(int Dh, PreparedView v, const double* __restrict__ pc,
+                                              FullcovView f, Windows win) {
+    extern __shared__ double P[];  // Dh * Dh
+    const int k = blockIdx.x;
+    const int sd = Dh / 3;
+    const double* U = pc + (size_t)k * Dh * Dh;
+    for (int e = threadIdx.x; e < Dh * Dh; e += blockDim.x) {
+        const int r = e / Dh, c = e - r * Dh;
+        double s = 0.0;
+        for (int q = max(r, c); q < Dh; ++q) s = fma(U[(size_t)r * Dh + q], U[(size_t)c * Dh + q], s);
+        P[e] = s;
+    }
+    __syncthreads();
+    const int ss = sd * sd;
+    for (int e = threadIdx.x; e < FC_NG * ss; e += blockDim.x) {
+        const int blk = e / ss, rem = e - blk * ss;
+        const int l = rem / sd, r = rem - l * sd;  // column-major: element G[r][l]
+        const int a = blk == FC_GMM ? -1 : (blk == FC_G00 || blk == FC_G0M) ? 0 : 1;
+        const int b = (blk == FC_GMM || blk == FC_G0M || blk == FC_GPM) ? -1 : blk == FC_GPP ? 1 : 0;
+        double ca[3], cb[3];  // c[w][a + 1], c[w][b + 1] by selects: no dynamic index into win
+#pragma unroll
+        for (int w = 0; w < 3; ++w) {
+            ca[w] = a < 0 ? win.c[w][0] : a == 0 ? win.c[w][1] : win.c[w][2];
+            cb[w] = b < 0 ? win.c[w][0] : b == 0 ? win.c[w][1] : win.c[w][2];
+        }
+        double s = 0.0;
+#pragma unroll
+        for (int w = 0; w < 3; ++w)
+#pragma unroll
+            for (int u = 0; u < 3; ++u)
+                s = fma(ca[w] * cb[u], P[(w * sd + r) * Dh + u * sd + l], s);
+        f.g[(size_t)k * FC_NG * ss + e] = s;
+    }
+    const double* at = v.at + (size_t)k * Dh * Dh;
+    for (int e = threadIdx.x; e < Dh * Dh; e += blockDim.x) {
+        const int c = e / Dh, r = e - c * Dh;  // B^T[c][r] = B[r][c] = sum_q P[r][q] A[q][c]
+        double s = 0.0;
+        for (int q = 0; q < Dh; ++q) s = fma(P[r * Dh + q], at[(size_t)c * Dh + q], s);
+        f.bt[(size_t)k * Dh * Dh + e] = s;
+    }
+    const double* offset = v.offset + (size_t)k * Dh;
+    for (int r = threadIdx.x; r < Dh; r += blockDim.x) {
+        double s = 0.0;
+        for (int q = 0; q < Dh; ++q) s = fma(P[r * Dh + q], offset[q], s);
+        f.h[(size_t)k * Dh + r] = s;
+    }
+}
+
+// The block solve, one warp per utterance; lane k owns row k of every sd x sd block.  Forward,
+// block row i (right-looking block Cholesky):
+//   A0 = R_ii + (updates of steps i-2, i-1),  A1 = R_{i+1,i} + (update of step i-1),  A2 = R_{i+2,i}
+//   L_ii = chol(A0), L1 = A1 L_ii^-T, L2 = A2 L_ii^-T, z_i = L_ii^-1 (r_i + carried terms)
+// as ONE column sweep over the 3 sd x sd panel [A0; A1; A2] and the right-hand side (lane k keeps
+// its rows of A0, A1, A2 in registers; column j of L_ii is broadcast through shared memory), then
+//   R~_{i+1,i+1} -= L1 L1^T,  R~_{i+2,i+2} = -L2 L2^T,  R~_{i+2,i+1} = -L2 L1^T
+// (rows in registers / shared memory), and L_ii (diagonal stored as 1 / L_kk), L1, L2 and z_i go
+// to the chain workspace, (3 sd^2 + sd) doubles per frame, column-major so the lanes store
+// coalesced.  Back:  y_i = L_ii^-T (z_i - L1^T y_{i+1} - L2^T y_{i+2}).
+// SDM: the largest static dimension the instantiation holds; EXACT: sd == SDM (no guards).
+constexpr int FC_MAXSD = 26;  // dim_half <= 80, a multiple of 3
+
+template <int SDM, bool EXACT>
+__global__ void __launch_bounds__(32)
+convert_fullcov_solve_kernel(const int64_t* __restrict__ off, int sd_arg,
+                             const int32_t* __restrict__ mix, const double* __restrict__ g,
+                             const double* __restrict__ gtab, Windows win,
+                             double* __restrict__ chain, double* __restrict__ out) {
+    constexpr int LD = SDM + 1;
+    constexpr unsigned FULL = 0xffffffffu;
+    __shared__ double Ls[SDM * LD];    // [l * LD + k]: L_ii[k][l] (back: the staged frame)
+    __shared__ double L1s[SDM * LD];   // L1[k][l]
+    __shared__ double L2s[SDM * LD];   // L2[k][l]
+    __shared__ double accN[SDM * LD];  // lane k's row of the update of R_{i+1,i+1} (own row only)
+    __shared__ double accO[SDM * LD];  // lane k's row of the update of R_{i+1,i}
+    const int sd = EXACT ? SDM : sd_arg;
+    const int u = blockIdx.x, k = threadIdx.x;
+    const long long t0 = off[u];
+    const int T = (int)(off[u + 1] - t0);
+    if (T <= 0) return;
+    const bool row = k < sd;
+    const int Dh = 3 * sd;
+    const size_t ss = (size_t)sd * sd, fs = 3 * ss + sd;
+    double a0[SDM], a1[SDM], a2[SDM];
+#pragma unroll
+    for (int l = 0; l < SDM; ++l) {
+        a0[l] = 0.0;
+        if (row && l < sd) accN[l * LD + k] = accO[l * LD + k] = 0.0;
+    }
+    double rN = 0.0, rNN = 0.0;  // carried right-hand-side terms of rows i+1, i+2
+    for (int i = 0; i < T; ++i) {
+        const long long n = t0 + i;
+        const bool hm = i >= 1, hp = i + 1 < T, hpp = i + 2 < T;
+        double b = 0.0;
+        if (row) {
+            const double* G0 = gtab + (size_t)mix[n] * FC_NG * ss + k;
+            const double* Gm = gtab + (size_t)(hm ? mix[n - 1] : 0) * FC_NG * ss + k;
+            const double* Gp = gtab + (size_t)(hp ? mix[n + 1] : 0) * FC_NG * ss + k;
+#pragma unroll
+            for (int l = 0; l < SDM; ++l) {
+                if (!EXACT && l >= sd) continue;
+                const size_t o = (size_t)l * sd;
+                double x = a0[l] + G0[FC_G00 * ss + o];
+                if (hm) x += Gm[FC_GPP * ss + o];
+                if (hp) x += Gp[FC_GMM * ss + o];
+                a0[l] = x;
+                a1[l] = hp ? accO[l * LD + k] + G0[FC_GP0 * ss + o] + Gp[FC_G0M * ss + o] : 0.0;
+                a2[l] = hpp ? Gp[FC_GPM * ss + o] : 0.0;
+            }
+            const double* gc = g + (size_t)n * Dh + k;
+            b = rN;
+#pragma unroll
+            for (int w = 0; w < 3; ++w) {
+                b = fma(win.c[w][1], gc[w * sd], b);
+                if (hm) b = fma(win.c[w][2], gc[w * sd - Dh], b);
+                if (hp) b = fma(win.c[w][0], gc[w * sd + Dh], b);
+            }
+        } else {
+#pragma unroll
+            for (int l = 0; l < SDM; ++l) a0[l] = a1[l] = a2[l] = 0.0;
+        }
+        // column sweep: POTRF of A0, the two TRSMs and the forward substitution
+        double inv_k = 0.0, z_k = 0.0, rN_next = rNN, rNN_next = 0.0;
+#pragma unroll
+        for (int j = 0; j < SDM; ++j) {
+            if (!EXACT && j >= sd) continue;
+            const double inv = rsqrt(__shfl_sync(FULL, a0[j], j));  // 1 / L_jj
+            const double l0 = k >= j ? a0[j] * inv : 0.0;
+            const double l1 = a1[j] * inv, l2 = a2[j] * inv;
+            const double zj = __shfl_sync(FULL, b, j) * inv;
+            if (k == j) { inv_k = inv; z_k = zj; }
+            a0[j] = l0;
+            a1[j] = l1;
+            a2[j] = l2;
+            if (k > j) b = fma(-l0, zj, b);
+            rN_next = fma(-l1, zj, rN_next);
+            rNN_next = fma(-l2, zj, rNN_next);
+            if (row) Ls[j * LD + k] = l0;
+            __syncwarp();
+#pragma unroll
+            for (int l = j + 1; l < SDM; ++l) {
+                if (!EXACT && l >= sd) continue;
+                const double L = Ls[j * LD + l];
+                a0[l] = fma(-l0, L, a0[l]);
+                a1[l] = fma(-l1, L, a1[l]);
+                a2[l] = fma(-l2, L, a2[l]);
+            }
+        }
+        rN = rN_next;
+        rNN = rNN_next;
+        if (row) {
+            double* cf = chain + (size_t)n * fs + k;
+#pragma unroll
+            for (int l = 0; l < SDM; ++l) {
+                if (!EXACT && l >= sd) continue;
+                cf[(size_t)l * sd] = l == k ? inv_k : a0[l];
+                cf[ss + (size_t)l * sd] = a1[l];
+                cf[2 * ss + (size_t)l * sd] = a2[l];
+                L1s[l * LD + k] = a1[l];
+                L2s[l * LD + k] = a2[l];
+            }
+            cf[3 * ss] = z_k;
+        }
+        __syncwarp();
+        // the SYRK / GEMM updates; a0 becomes the next step's update of its diagonal block
+        if (row) {
+#pragma unroll
+            for (int j = 0; j < SDM; ++j) {
+                if (!EXACT && j >= sd) continue;
+                double d1 = 0.0, d2 = 0.0, d3 = 0.0;
+#pragma unroll
+                for (int l = 0; l < SDM; ++l) {
+                    if (!EXACT && l >= sd) continue;
+                    const double p = L1s[l * LD + j], q = L2s[l * LD + j];
+                    d1 = fma(a1[l], p, d1);
+                    d2 = fma(a2[l], q, d2);
+                    d3 = fma(a2[l], p, d3);
+                }
+                a0[j] = accN[j * LD + k] - d1;
+                accN[j * LD + k] = -d2;
+                accO[j * LD + k] = -d3;
+            }
+        }
+    }
+    __syncwarp();
+    double y1 = 0.0, y2 = 0.0;  // lane k: y_{i+1}[k], y_{i+2}[k]
+    for (int i = T - 1; i >= 0; --i) {
+        const double* cf = chain + (size_t)(t0 + i) * fs;
+        for (int e = k; e < (int)ss; e += 32) {
+            const int l = e / sd, r = e - l * sd;
+            Ls[l * LD + r] = cf[e];
+            L1s[l * LD + r] = cf[ss + e];
+            L2s[l * LD + r] = cf[2 * ss + e];
+        }
+        __syncwarp();
+        double b = row ? cf[3 * ss + k] : 0.0;
+#pragma unroll
+        for (int l = 0; l < SDM; ++l) {
+            if (!EXACT && l >= sd) continue;
+            const double p = __shfl_sync(FULL, y1, l), q = __shfl_sync(FULL, y2, l);
+            if (row) b = fma(-L1s[k * LD + l], p, fma(-L2s[k * LD + l], q, b));  // L1[l][k], L2[l][k]
+        }
+        double y_k = 0.0;
+#pragma unroll
+        for (int j = SDM - 1; j >= 0; --j) {
+            if (!EXACT && j >= sd) continue;
+            const double yj = __shfl_sync(FULL, b, j) * Ls[j * LD + j];
+            if (k == j) y_k = yj;
+            if (k < j) b = fma(-Ls[k * LD + j], yj, b);  // L_ii[j][k]
+        }
+        if (row) out[(size_t)(t0 + i) * sd + k] = y_k;
+        y2 = y1;
+        y1 = y_k;
+        __syncwarp();
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // Host side of the hard-sequence conversions (kw_convert_batch, kw_convert_gv_batch,
-// kw_convert_em_batch): one workspace layout, one argument check and the stages they share.
+// kw_convert_em_batch, kw_convert_fullcov_batch): one workspace layout, one argument check and
+// the stages they share.
 
-enum ConvertKind { CONVERT_PLAIN, CONVERT_GV, CONVERT_EM };
+enum ConvertKind { CONVERT_PLAIN, CONVERT_GV, CONVERT_EM, CONVERT_FULLCOV };
 
-// The workspace of one conversion call, in this order: the hard-sequence buffers every kind uses,
-// then the GV step plane or the EM buffers, then the tensor-core region of the E-steps the call
-// runs (precision 1 only: the hard-sequence E-step at dim_half, and for EM also the E-step at
-// 2 * dim_half).
+// The workspace of one conversion call, in this order: the hard-sequence buffers every kind uses
+// (the band set and the utterance flags except for the full-covariance kind, whose block solve
+// takes neither), then the GV step plane, the EM buffers or the block-solve chain, then the
+// tensor-core region of the E-steps the call runs (precision 1 only: the hard-sequence E-step at
+// dim_half, and for EM also the E-step at 2 * dim_half).
 struct ConvertWorkspace {
     int32_t* mix;          // (total) hard mixture sequence
     int* counts;           // K      (counting sort of the frames by mixture)
@@ -814,6 +1114,7 @@ struct ConvertWorkspace {
     double* means;         // EM: (K, 2 Dh)
     double* pc;            // EM: (K, 2 Dh, 2 Dh)
     double* aux;           // EM: (K, 2 Dh + 2)
+    double* chain;         // full covariance: (total, 3 sd^2 + sd) block-Cholesky factors and z
     char* tc;              // tensor-core region of tc_bytes (0 at precision 0)
     size_t tc_bytes;
     size_t bytes;
@@ -831,8 +1132,10 @@ static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, 
     w.cursor = c.take<int>((size_t)K);
     w.order = c.take<int>((size_t)total);
     w.E = c.take<double>((size_t)total * Dh);
-    w.band = c.take<double>(4 * (size_t)total * sd);
-    w.flags = c.take<unsigned char>((size_t)total);
+    if (kind != CONVERT_FULLCOV) {
+        w.band = c.take<double>(4 * (size_t)total * sd);
+        w.flags = c.take<unsigned char>((size_t)total);
+    }
     if (kind == CONVERT_GV) w.step = c.take<double>((size_t)total * sd);
     if (kind == CONVERT_EM) {
         const size_t D = 2 * (size_t)Dh;
@@ -846,6 +1149,7 @@ static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, 
         w.pc = c.take<double>((size_t)K * D * D);
         w.aux = c.take<double>((size_t)K * (D + 2));
     }
+    if (kind == CONVERT_FULLCOV) w.chain = c.take<double>((size_t)total * (3 * (size_t)sd * sd + sd));
     if (precision == 1) {
         w.tc_bytes = tc_workspace_bytes(total, K, Dh);
         if (kind == CONVERT_EM)
@@ -943,6 +1247,21 @@ static int solve_mlpg(int n_utts, const int64_t* off, long long total, int Dh,
     const long long threads = (long long)n_utts * sd;
     convert_mlpg_kernel<<<(unsigned)((threads + 95) / 96), 96, 0, st>>>(n_utts, off, sd, w.band,
                                                                         total, out);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+// The block solve of the full-covariance system from the right-hand sides g_t in w.E under the
+// mixture sequence w.mix, into out.
+static int solve_fullcov(int n_utts, const int64_t* off, int Dh, const FullcovView& f,
+                         const ConvertWorkspace& w, double* out, cudaStream_t st) {
+    const int sd = Dh / 3;
+    if (sd == 24)
+        convert_fullcov_solve_kernel<24, true><<<n_utts, 32, 0, st>>>(
+            off, sd, w.mix, w.E, f.g, kDeltaWindows, w.chain, out);
+    else
+        convert_fullcov_solve_kernel<FC_MAXSD, false><<<n_utts, 32, 0, st>>>(
+            off, sd, w.mix, w.E, f.g, kDeltaWindows, w.chain, out);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }
@@ -1204,5 +1523,76 @@ extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t t
         if (rc != KW_OK) return rc;
     }
     if (loglik_dev != nullptr) return estep(em_iter);
+    return KW_OK;
+}
+
+extern "C" size_t kw_convert_fullcov_prepared_len(int K, int Dh) {
+    return view_fullcov(nullptr, K, Dh).len;
+}
+
+extern "C" size_t kw_convert_fullcov_prepare_workspace_bytes(int K, int Dh) {
+    return carve_fullcov_scratch(K, Dh, nullptr).bytes;
+}
+
+extern "C" int kw_convert_fullcov_prepare(int K, int Dh, int diff, const double* covariances_dev,
+                                          const double* prepared_dev, double* fullcov_dev,
+                                          int32_t* info_dev, void* workspace_dev,
+                                          size_t workspace_bytes, void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    KW_REQUIRE(K > 0 && Dh > 0, "kw_convert_fullcov_prepare: K, dim_half must be positive");
+    KW_REQUIRE(Dh % 3 == 0,
+               "kw_convert_fullcov_prepare: dim_half %d is not static+delta+delta2 (multiple of 3)",
+               Dh);
+    KW_REQUIRE(Dh <= 80, "kw_convert_fullcov_prepare: dim_half %d > 80 unsupported", Dh);
+    const PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    const FullcovScratch w = carve_fullcov_scratch(K, Dh, workspace_dev);
+    if (w.bytes > workspace_bytes)
+        return workspace_too_small("kw_convert_fullcov_prepare", w.bytes, workspace_bytes);
+    const FullcovView f = view_fullcov(fullcov_dev, K, Dh);
+    convert_fullcov_sigma_kernel<<<K, 256, 0, st>>>(Dh, diff, covariances_dev, v, w);
+    KW_CUDA_CHECK(cudaGetLastError());
+    // the precision Cholesky factor of Sigma (info[k] != 0: Sigma_k not positive definite)
+    int rc = finalize_launch(K, Dh, 0.0, 0, 0, nullptr, nullptr, w.ones, v.tgt_means, w.sigma,
+                             w.pc, w.aux, info_dev, st);
+    if (rc != KW_OK) return rc;
+    const size_t smem = sizeof(double) * (size_t)Dh * Dh;
+    KW_CUDA_CHECK(cudaFuncSetAttribute(convert_fullcov_tables_kernel,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    convert_fullcov_tables_kernel<<<K, 256, smem, st>>>(Dh, v, w.pc, f, kDeltaWindows);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+extern "C" size_t kw_convert_fullcov_workspace_bytes(int64_t total_frames, int K, int Dh,
+                                                     int precision) {
+    return carve_convert(CONVERT_FULLCOV, total_frames, K, Dh, precision, nullptr).bytes;
+}
+
+extern "C" int kw_convert_fullcov_batch(int n_utts, const int64_t* off_dev, int64_t total,
+                                        int max_frames, const double* src_dev, int K, int Dh,
+                                        const double* prepared_dev, const double* fullcov_dev,
+                                        double* out_dev, int32_t* mix_dev, int precision,
+                                        void* workspace_dev, size_t workspace_bytes,
+                                        void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    (void)max_frames;
+    if (n_utts == 0 || total == 0) return KW_OK;
+    int rc = check_convert("kw_convert_fullcov_batch", n_utts, total, K, Dh, precision, Dh);
+    if (rc != KW_OK) return rc;
+    const ConvertWorkspace w =
+        carve_convert(CONVERT_FULLCOV, total, K, Dh, precision, workspace_dev);
+    if (w.bytes > workspace_bytes)
+        return workspace_too_small("kw_convert_fullcov_batch", w.bytes, workspace_bytes);
+    const FullcovView f = view_fullcov(const_cast<double*>(fullcov_dev), K, Dh);
+    // the conditional-mean pass on B^T and h in place of A^T and offset yields g_t = P E_t
+    PreparedView vg = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    vg.at = f.bt;
+    vg.offset = f.h;
+    rc = hard_sequence(total, src_dev, K, Dh, precision, vg, w, st);
+    if (rc == KW_OK) rc = solve_fullcov(n_utts, off_dev, Dh, f, w, out_dev, st);
+    if (rc != KW_OK) return rc;
+    if (mix_dev != nullptr)
+        KW_CUDA_CHECK(cudaMemcpyAsync(mix_dev, w.mix, sizeof(int32_t) * total,
+                                      cudaMemcpyDeviceToDevice, st));
     return KW_OK;
 }

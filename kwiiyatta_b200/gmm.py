@@ -576,11 +576,14 @@ class B200GMMFeatureConverter(FeatureConverter):
         conv = cls(components=int(state['n_components']), verbose=0, **kwargs)
         return conv.load_state_dict(state)
 
-    def _mlpg(self, diff, mlpg=True, gv=False, em_iter=0):
+    def _mlpg(self, diff, mlpg=True, gv=False, em_iter=0, conditional_covariance='diagonal'):
         from .mlpg import MLPG
-        key = (bool(diff), bool(mlpg), bool(gv), int(em_iter))
+        key = (bool(diff), bool(mlpg), bool(gv), int(em_iter), conditional_covariance)
         if gv and not mlpg:
             raise ValueError('GV is defined for MLPG conversion only (mlpg=True)')
+        if conditional_covariance != 'diagonal' and not mlpg:
+            raise ValueError('conditional_covariance is defined for MLPG conversion only '
+                             '(mlpg=True)')
         if gv and self._gv is None:
             raise ValueError('gv=True needs GV statistics: construct with gv=True and train, '
                              'or assign estimate_gv(...) to .gv')
@@ -590,16 +593,22 @@ class B200GMMFeatureConverter(FeatureConverter):
             # sequence (and with it the FP64 MLPG output) is the FP64 one at any size
             self._paramgen[key] = MLPG(self.gmm, windows=windows, diff=diff,
                                        precision=self.gmm.precision_request,
-                                       gv=self._gv if gv else None, em_iter=em_iter)
+                                       gv=self._gv if gv else None, em_iter=em_iter,
+                                       conditional_covariance=conditional_covariance)
         return self._paramgen[key]
 
-    def convert(self, feature, mlpg=True, diff=False, gv=False, em_iter=0):
+    def convert(self, feature, mlpg=True, diff=False, gv=False, em_iter=0,
+                conditional_covariance='diagonal'):
         """``gv=True``: GV-considered MLPG with the statistics in ``.gv`` (in diff mode the GV
         is that of source + output, which is what the MLSA filter makes heard).
         ``em_iter > 0``: maximum-likelihood conversion over all mixture sequences, ``em_iter``
-        EM iterations from the hard-sequence trajectory (``MLPG(em_iter=)``)."""
-        return self._mlpg(diff, mlpg, gv, em_iter).transform(feature)
+        EM iterations from the hard-sequence trajectory (``MLPG(em_iter=)``).
+        ``conditional_covariance='full'``: the ML trajectory under each mixture's full
+        conditional covariance (``MLPG(conditional_covariance=)``)."""
+        return self._mlpg(diff, mlpg, gv, em_iter, conditional_covariance).transform(feature)
 
-    def convert_many(self, features, diff=False, gv=False, em_iter=0):
+    def convert_many(self, features, diff=False, gv=False, em_iter=0,
+                     conditional_covariance='diagonal'):
         """Batched ``convert`` over a list of (T_i, 72) arrays."""
-        return self._mlpg(diff, True, gv, em_iter).transform_many(features)
+        return self._mlpg(diff, True, gv, em_iter,
+                          conditional_covariance).transform_many(features)

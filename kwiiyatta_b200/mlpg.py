@@ -1,6 +1,7 @@
 """Posterior + MLPG on the B200 (nnmnkwii.baseline.gmm.MLPG as used at
-kwiiyatta/converter/gmm.py:28-34), optionally with global variance (``gv=``; kwiiyatta_b200.gv)
-or maximum-likelihood conversion over all mixture sequences (``em_iter=``)."""
+kwiiyatta/converter/gmm.py:28-34), optionally with global variance (``gv=``; kwiiyatta_b200.gv),
+maximum-likelihood conversion over all mixture sequences (``em_iter=``) or the full conditional
+covariance (``conditional_covariance='full'``)."""
 import numpy as np
 
 from . import _lib
@@ -17,13 +18,46 @@ class MLPG:
     here; the reference rebuilds it on every convert call (kwiiyatta/converter/gmm.py:32)."""
 
     def __init__(self, gmm, windows=None, swap=False, diff=False, precision='auto',
-                 device=None, gv=None, gv_iter=20, gv_weights=(1.0, 1.0), em_iter=0):
+                 device=None, gv=None, gv_iter=20, gv_weights=(1.0, 1.0), em_iter=0,
+                 conditional_covariance='diagonal'):
         torch = _lib.require_cuda()
         self._dev = torch.device('cuda' if device is None else device)
         with torch.cuda.device(self._dev):      # 'cuda' without an index: the current device
             self._setup(torch, gmm, windows, swap, diff, precision)
             self._setup_gv(torch, gv, gv_iter, gv_weights)
             self._setup_em(precision, em_iter)
+            self._setup_fullcov(torch, gmm, conditional_covariance)
+
+    def _setup_fullcov(self, torch, gmm, conditional_covariance):
+        """``conditional_covariance='full'``: the ML trajectory under the full conditional
+        covariance S_yy - A S_xy of each mixture (Toda, Black & Tokuda 2007), which couples the
+        static dimensions, instead of nnmnkwii's element-wise diagonal (``'diagonal'``)."""
+        if conditional_covariance not in ('diagonal', 'full'):
+            raise ValueError("conditional_covariance must be 'diagonal' or 'full', got "
+                             f'{conditional_covariance!r}')
+        self.conditional_covariance = conditional_covariance
+        self._fullcov = None
+        if conditional_covariance == 'diagonal':
+            return
+        if len(self.windows) == 1:
+            raise ValueError('the full conditional covariance is defined for MLPG trajectories '
+                             'only (not with a single static window)')
+        if self.gv is not None or self.em_iter:
+            raise NotImplementedError("conditional_covariance='full' together with GV or EM "
+                                      'conversion is not built')
+        lib = _lib.lib()
+        k, dh = self.num_mixtures, self.dim_half
+        c = torch.from_numpy(np.ascontiguousarray(gmm.covariances_, dtype=np.float64)).to(self._dev)
+        self._fullcov = torch.empty(lib.kw_convert_fullcov_prepared_len(k, dh),
+                                    dtype=torch.float64, device=self._dev)
+        info = torch.zeros(k, dtype=torch.int32, device=self._dev)
+        ws_bytes = lib.kw_convert_fullcov_prepare_workspace_bytes(k, dh)
+        _lib.call('kw_convert_fullcov_prepare', k, dh, int(self.diff), c, self._prepared,
+                  self._fullcov, info, _lib.workspace(ws_bytes, self._dev), ws_bytes,
+                  _lib.stream_ptr(torch))
+        if info.cpu().numpy().any():
+            raise np.linalg.LinAlgError('conditional covariance of some mixture is not positive '
+                                        'definite')
 
     def _setup_em(self, precision, em_iter):
         """``em_iter > 0``: every transform runs ``em_iter`` EM iterations of maximum-likelihood
@@ -108,11 +142,18 @@ class MLPG:
 
     def _launch(self, n_utts, off_dev, total, max_frames, src, out, mix, stream,
                 gv_f=None, gv_accepted=None, em_loglik=None):
-        """kw_convert_batch, kw_convert_gv_batch when GV statistics are set, or
-        kw_convert_em_batch when ``em_iter > 0``, on device tensors (``src`` (total, dim_half),
-        ``out`` (total, static_dim))."""
+        """kw_convert_batch, kw_convert_gv_batch when GV statistics are set,
+        kw_convert_em_batch when ``em_iter > 0``, or kw_convert_fullcov_batch with the full
+        conditional covariance, on device tensors (``src`` (total, dim_half), ``out`` (total,
+        static_dim))."""
         lib = _lib.lib()
         k, dh = self.num_mixtures, self.dim_half
+        if self._fullcov is not None:
+            ws_bytes = lib.kw_convert_fullcov_workspace_bytes(total, k, dh, self.precision)
+            _lib.call('kw_convert_fullcov_batch', n_utts, off_dev, total, int(max_frames), src, k,
+                      dh, self._prepared, self._fullcov, out, mix, self.precision,
+                      _lib.workspace(ws_bytes, src.device), ws_bytes, stream)
+            return
         if self.em_iter:
             ws_bytes = lib.kw_convert_em_workspace_bytes(total, k, dh, self._em_precision)
             _lib.call('kw_convert_em_batch', n_utts, off_dev, total, src, k, dh, self._prepared,
