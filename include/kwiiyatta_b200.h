@@ -295,6 +295,50 @@ int kw_convert_fullcov_batch(int n_utts, const int64_t* off_dev, int64_t total_f
                              double* out_dev, int32_t* mix_dev, int precision,
                              void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* Low-delay conversion (fixed-lag MLPG; Muramatsu et al., Interspeech 2008;
+ * oracle/mlpg_stream_ref.py) over n_slots concurrent streams, each one utterance arriving one
+ * static frame (static_dim = dim_half / 3 values, mel-cepstrum without c0) per call.  Static j of
+ * a stream completes its source vector x_{j-1} = [x~, delta, delta^2] (zero padded at the start
+ * and, when the stream ends, at the end), and with it the hard mixture, conditional mean and
+ * diagonal variance of frame j-1: n = j frames are known.  The frame emitted with static j is
+ * y^(n)[n-1-delay], where y^(n) is kw_convert_batch's MLPG solution of frames [0, n) alone; so
+ * frame s comes out delay + 1 frames after its static went in.  Ending a stream of T statics
+ * emits its last min(T, delay + 1) frames from y^(T), the offline solution; with delay >= T-1 the
+ * whole output equals kw_convert_batch's.  Per call and slot the cost is one E-step row, one
+ * conditional mean and O(delay) per static dimension.
+ *
+ * The state of n_slots streams (device, float64, length kw_convert_stream_state_len) holds per
+ * slot the frame count, the last two statics, the last two frames' precision terms and a ring of
+ * delay + 2 Cholesky factor rows per static dimension: 8 (14 + 4 (delay + 2)) static_dim + 8 bytes.
+ * kw_convert_stream_init empties every slot.  A state serves the n_slots, dim_half and delay it
+ * was made for, and one `prepared` block (diff mode comes from that block).
+ *
+ * kw_convert_stream_push delivers one static per slot for the m (0 <= m <= n_slots) distinct
+ * slots in the HOST array slots_host: static_dev (m, static_dim).  out_dev (m, static_dim)
+ * receives the emitted frames and frame_dev (m) int64 their indices in their streams, -1 (and a
+ * zero row) where a stream has not yet gone delay + 1 statics past its first.
+ * kw_convert_stream_end ends the streams of the m slots, which are empty afterwards: out_dev
+ * (m, delay + 1, static_dim) receives the last count_dev[i] (m, int64) frames of row i in order,
+ * zero rows after them (an empty slot emits 0 frames).
+ * Both check every argument before they queue any work, and a rejected call changes neither
+ * the workspace nor the state: slots in [0, n_slots) and distinct, delay in [0, 8192],
+ * dim_half a multiple of 3 and <= 80, precision 0 (FP64 E-step) or 1 (tensor cores, labels
+ * re-checked in FP64 near ties), and a workspace of kw_convert_stream_workspace_bytes for m rows
+ * (which does not depend on delay). */
+size_t kw_convert_stream_state_len(int n_slots, int dim_half, int delay);
+int kw_convert_stream_init(int n_slots, int dim_half, int delay, double* state_dev, void* stream);
+size_t kw_convert_stream_workspace_bytes(int m, int n_components, int dim_half, int delay,
+                                         int precision);
+int kw_convert_stream_push(int n_slots, int delay, int m, const int32_t* slots_host,
+                           const double* static_dev, int n_components, int dim_half,
+                           const double* prepared_dev, double* state_dev, double* out_dev,
+                           int64_t* frame_dev, int precision, void* workspace_dev,
+                           size_t workspace_bytes, void* stream);
+int kw_convert_stream_end(int n_slots, int delay, int m, const int32_t* slots_host,
+                          int n_components, int dim_half, const double* prepared_dev,
+                          double* state_dev, double* out_dev, int64_t* count_dev, int precision,
+                          void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* Soft-posterior mapping without MLPG (nnmnkwii MLPGBase.transform; the mlpg=False branch of
  * kwiiyatta/converter/gmm.py:30-31): out (total, dim_half) = sum_m p(m|x) (mu_y + S_yx S_xx^-1 (x - mu_x)).
  * `prepared_dev` comes from kw_convert_prepare with the same dim_half. */

@@ -64,6 +64,13 @@ SIGNATURES = {
     'kw_convert_fullcov_workspace_bytes': (_sz, [_i64, _i, _i, _i]),
     'kw_convert_fullcov_batch': (_i, [_i, _vp, _i64, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _i,
                                       _vp, _sz, _vp]),
+    'kw_convert_stream_state_len': (_sz, [_i, _i, _i]),
+    'kw_convert_stream_init': (_i, [_i, _i, _i, _vp, _vp]),
+    'kw_convert_stream_workspace_bytes': (_sz, [_i, _i, _i, _i, _i]),
+    'kw_convert_stream_push': (_i, [_i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp,
+                                    _sz, _vp]),
+    'kw_convert_stream_end': (_i, [_i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _sz,
+                                   _vp]),
 }
 
 

@@ -17,6 +17,7 @@
 // forward and the backward sweep: (3 sd^2 + sd) doubles per frame, 14 KB at sd = 24, where the
 // diagonal path's band takes 768 B.
 #include <algorithm>
+#include <vector>
 
 #include "common.cuh"
 
@@ -1083,15 +1084,222 @@ convert_fullcov_solve_kernel(const int64_t* __restrict__ off, int sd_arg,
 }
 
 // ------------------------------------------------------------------------------------------
+// Low-delay conversion (fixed-lag MLPG; Muramatsu et al., Interspeech 2008; restated in
+// oracle/mlpg_stream_ref.py) over many concurrent streams ("slots").  A stream delivers one static
+// frame per call.  Delivering static j completes the source vector x_{j-1} (its deltas need
+// static j), and with it the conditional mean and variance of frame j-1, so n = j frames are
+// known.  The emitted frame is y^(n)[n-1-L], y^(n) the MLPG solution of frames [0, n).
+// The system of [0, n) is the leading n x n block of the whole utterance's system except on row
+// n-1, which lacks frame n's terms on its diagonal and right-hand side.  So rows 0 .. n-2 of the
+// banded Cholesky factor are final and are carried forward one row per call with the recurrence
+// of convert_mlpg_kernel; row n-1 is formed provisionally (it is final when the stream ends), and
+// L + 1 steps of back substitution over a ring of the last factor rows give y^(n)[n-1-L].
+// Band entries and factor steps use the expressions of convert_band_kernel and
+// convert_mlpg_kernel, so with L >= T-1 a stream reproduces the offline conversion.
+
+// The state of n_slots streams (kw_convert_stream_state_len doubles).  Per (slot, static dim):
+// the last two statics, the precision terms p_w = 1 / D_w and b_w = p_w E_w of the last two
+// completed frames, and a ring of L + 2 factor rows (r = 1 / L_ii, e = L_{i,i-1}, z, c = R_{i,i+2});
+// frame / static / row i sits at i mod 2 (i mod (L + 2) in the ring).  Planes are (n_slots, sd).
+struct StreamState {
+    long long* count;  // (n_slots) statics delivered so far; 0 = empty slot
+    double* statics;   // (2, n_slots, sd)
+    double* terms;     // (2, 6, n_slots, sd): p_0, p_1, p_2, b_0, b_1, b_2
+    double* ring;      // (L + 2, 4, n_slots, sd): r, e, z, c
+    size_t len;        // in doubles
+};
+
+static StreamState view_stream_state(double* base, int n_slots, int sd, int delay) {
+    StreamState s;
+    const size_t plane = (size_t)n_slots * sd;
+    size_t o = 0;
+    s.count = reinterpret_cast<long long*>(base);  o += (size_t)n_slots;
+    s.statics = base + o;                          o += 2 * plane;
+    s.terms = base + o;                            o += 12 * plane;
+    s.ring = base + o;                             o += ((size_t)delay + 2) * 4 * plane;
+    s.len = o;
+    return s;
+}
+
+// Source vectors: one warp per slot row i, lane d < sd.  x_{j-1} = [x~, delta, delta^2] of the
+// statics j-2, j-1, j (zero outside [0, T); j = the static this call delivers, at the end the
+// missing one), in kw_delta_features' order of operations; rows of slots with no complete frame
+// get zeros.  Records j per row, stores static j and counts it (the end call empties the slot).
+__global__ void convert_stream_source_kernel(int m, int sd, int end, const int* __restrict__ slots,
+                                             const double* __restrict__ statics_in, StreamState s,
+                                             int n_slots, double* __restrict__ x,
+                                             long long* __restrict__ jrow) {
+    const int i = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5);
+    const int d = threadIdx.x & 31;
+    if (i >= m) return;
+    const int slot = slots[i];
+    const long long j = s.count[slot];
+    const size_t plane = (size_t)n_slots * sd;
+    if (d < sd) {
+        const size_t o = (size_t)slot * sd + d;
+        const double xm = j >= 2 ? s.statics[((j - 2) & 1) * plane + o] : 0.0;
+        const double xc = j >= 1 ? s.statics[((j - 1) & 1) * plane + o] : 0.0;
+        const double xp = end ? 0.0 : statics_in[(size_t)i * sd + d];
+        double* row = x + (size_t)i * 3 * sd;
+        row[d] = xc;
+        row[sd + d] = __dadd_rn(__dadd_rn(__dmul_rn(-0.5, xm), __dmul_rn(0.0, xc)), __dmul_rn(0.5, xp));
+        row[2 * sd + d] = __dadd_rn(__dadd_rn(xm, __dmul_rn(-2.0, xc)), xp);
+        if (!end) s.statics[(j & 1) * plane + o] = xp;   // replaces static j - 2, read above
+    }
+    __syncwarp();
+    if (d == 0) {
+        jrow[i] = j;
+        s.count[slot] = end ? 0 : j + 1;
+    }
+}
+
+// One row of the band from the precision terms of frames i-1 (m), i (c), i+1 (x): the expressions
+// of convert_band_kernel.
+__device__ __forceinline__ void stream_band_row(const double* pm, const double* bm, const double* pc,
+                                                const double* bc, const double* px, const double* bx,
+                                                const Windows& win, double& a, double& b, double& c,
+                                                double& rhs) {
+    a = 0.0; b = 0.0; c = 0.0; rhs = 0.0;
+#pragma unroll
+    for (int w = 0; w < 3; ++w) {
+        const double cm = win.c[w][0], c0 = win.c[w][1], cp = win.c[w][2];
+        a += cp * cp * pm[w] + c0 * c0 * pc[w] + cm * cm * px[w];
+        rhs += cp * bm[w] + c0 * bc[w] + cm * bx[w];
+        b += c0 * cp * pc[w] + cm * c0 * px[w];
+        c += cm * cp * px[w];
+    }
+}
+
+struct StreamStepArgs {
+    int m, n_slots, sd, Dh, delay;
+    const int* slots;
+    const long long* jrow;
+    const int32_t* mix;
+    const double* E;
+    const double* var;   // PreparedView::var
+    StreamState s;
+    Windows win;
+    double* out;         // push: (m, sd); end: (m, delay + 1, sd)
+    int64_t* index;      // push: emitted frame per row or -1; end: frames emitted per row
+};
+
+// One thread per (slot row, static dim).  Frame j-1 completes (n = j): row n-2 of the factor is
+// finalised into the ring, row n-1 is formed from frames n-2 and n-1 alone, and the back
+// substitution runs down to row max(0, n-1-L).  Push (END false): writes y^(n)[n-1-L] when that
+// frame exists.  End (END true): row n-1 is final, and y^(n) of the last min(n, L+1) frames is
+// written in order, zero rows after them.
+template <bool END>
+__global__ void __launch_bounds__(128) convert_stream_step_kernel(StreamStepArgs g) {
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= (long long)g.m * g.sd) return;
+    const int i = (int)(gid / g.sd), d = (int)(gid - (long long)i * g.sd);
+    const int sd = g.sd, L = g.delay, R = L + 2;
+    const long long j = g.jrow[i];
+    const size_t plane = (size_t)g.n_slots * sd;
+    const size_t o = (size_t)g.slots[i] * sd + d;
+    double* outp = END ? g.out + (size_t)i * (L + 1) * sd + d : g.out + (size_t)i * sd + d;
+    if (j == 0) {                     // nothing complete yet (push) / an empty slot (end)
+        if (END) {
+            for (int k = 0; k <= L; ++k) outp[(size_t)k * sd] = 0.0;
+        } else {
+            outp[0] = 0.0;
+        }
+        if (d == 0) g.index[i] = END ? 0 : -1;
+        return;
+    }
+    // precision terms of frames j-3 (m), j-2 (c) and the new frame j-1 (x)
+    double pm[3] = {0, 0, 0}, bm[3] = {0, 0, 0}, pc[3] = {0, 0, 0}, bc[3] = {0, 0, 0}, px[3], bx[3];
+    const int mx = g.mix[i];
+#pragma unroll
+    for (int w = 0; w < 3; ++w) {
+        const double prec = 1.0 / g.var[(size_t)mx * g.Dh + w * sd + d];
+        px[w] = prec;
+        bx[w] = prec * g.E[(size_t)i * g.Dh + w * sd + d];
+    }
+    double* t_c = g.s.terms + ((j - 2) & 1) * 6 * plane + o;
+    double* t_m = g.s.terms + ((j - 3) & 1) * 6 * plane + o;   // = frame j-1's place
+#pragma unroll
+    for (int w = 0; w < 3; ++w) {
+        if (j >= 2) { pc[w] = t_c[w * plane]; bc[w] = t_c[(3 + w) * plane]; }
+        if (j >= 3) { pm[w] = t_m[w * plane]; bm[w] = t_m[(3 + w) * plane]; }
+    }
+    if (!END) {
+#pragma unroll
+        for (int w = 0; w < 3; ++w) { t_m[w * plane] = px[w]; t_m[(3 + w) * plane] = bx[w]; }
+    }
+    double* ring = g.s.ring + o;
+    auto row_at = [&](long long r) -> double* { return ring + (size_t)(r % R) * 4 * plane; };
+    // the recurrence's carries: rows i-2 (_m2) and i-1 (_m1) of the row i it steps to, with the
+    // initial values of convert_mlpg_kernel before row 0
+    double c_m2 = 0, c_m1 = 0, b_m1 = 0, r_m1 = 1, r_m2 = 1, e_m1 = 0, z_m1 = 0, z_m2 = 0;
+    if (j >= 2) {                     // finalise row j-2: frames j-3, j-2, j-1 are all in
+        if (j >= 4) {
+            const double* p = row_at(j - 4);
+            r_m1 = p[0]; z_m1 = p[2 * plane]; c_m1 = p[3 * plane];
+        }
+        if (j >= 3) {
+            const double* p = row_at(j - 3);
+            c_m2 = c_m1; r_m2 = r_m1; z_m2 = z_m1;
+            r_m1 = p[0]; e_m1 = p[plane]; z_m1 = p[2 * plane]; c_m1 = p[3 * plane];
+            const double zero[3] = {0, 0, 0};
+            double a_, c_, rhs_;
+            stream_band_row(zero, zero, pm, bm, pc, bc, g.win, a_, b_m1, c_, rhs_);  // b_{j-3}
+        }
+        double a, b, c, rhs;
+        stream_band_row(pm, bm, pc, bc, px, bx, g.win, a, b, c, rhs);
+        const double f = c_m2 * r_m2;
+        const double e = (b_m1 - f * e_m1) * r_m1;
+        const double r = rsqrt(a - f * f - e * e);
+        const double z = (rhs - e * z_m1 - f * z_m2) * r;
+        double* p = row_at(j - 2);
+        p[0] = r; p[plane] = e; p[2 * plane] = z; p[3 * plane] = c;
+        c_m2 = c_m1; c_m1 = c; b_m1 = b;
+        r_m2 = r_m1; r_m1 = r; e_m1 = e;
+        z_m2 = z_m1; z_m1 = z;
+    }
+    // row j-1 from frames j-2 and j-1 (frame j is not in yet; at the end there is none)
+    const double zero[3] = {0, 0, 0};
+    double a, b_, c, rhs;
+    stream_band_row(pc, bc, px, bx, zero, zero, g.win, a, b_, c, rhs);
+    const double f = c_m2 * r_m2;
+    const double e = (b_m1 - f * e_m1) * r_m1;
+    const double r = rsqrt(a - f * f - e * e);
+    const double z = (rhs - e * z_m1 - f * z_m2) * r;
+    // back substitution L^T y = z from row j-1 down to row lo
+    const long long lo = j - 1 - L > 0 ? j - 1 - L : 0;
+    double y = z * r;
+    if (END) outp[(size_t)(j - 1 - lo) * sd] = y;
+    double y1 = y, y2 = 0.0, e_n1 = e;
+    for (long long k = j - 2; k >= lo; --k) {
+        const double* p = row_at(k);
+        const double rk = p[0], ek = p[plane], zk = p[2 * plane], ck = p[3 * plane];
+        y = (zk - e_n1 * y1 - (ck * rk) * y2) * rk;
+        if (END) outp[(size_t)(k - lo) * sd] = y;
+        y2 = y1; y1 = y;
+        e_n1 = ek;
+    }
+    if (END) {
+        const int count = (int)(j - lo);
+        for (int k = count; k <= L; ++k) outp[(size_t)k * sd] = 0.0;
+        if (d == 0) g.index[i] = count;
+    } else {
+        const bool emit = j - 1 - L >= 0;
+        outp[0] = emit ? y : 0.0;
+        if (d == 0) g.index[i] = emit ? j - 1 - L : -1;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // Host side of the hard-sequence conversions (kw_convert_batch, kw_convert_gv_batch,
 // kw_convert_em_batch, kw_convert_fullcov_batch): one workspace layout, one argument check and
 // the stages they share.
 
-enum ConvertKind { CONVERT_PLAIN, CONVERT_GV, CONVERT_EM, CONVERT_FULLCOV };
+enum ConvertKind { CONVERT_PLAIN, CONVERT_GV, CONVERT_EM, CONVERT_FULLCOV, CONVERT_STREAM };
 
 // The workspace of one conversion call, in this order: the hard-sequence buffers every kind uses
 // (the band set and the utterance flags except for the full-covariance kind, whose block solve
-// takes neither), then the GV step plane, the EM buffers or the block-solve chain, then the
+// takes neither, and the stream kind, which keeps its band in the stream state), then the GV
+// step plane, the EM buffers, the block-solve chain or the stream's source rows, then the
 // tensor-core region of the E-steps the call runs (precision 1 only: the hard-sequence E-step at
 // dim_half, and for EM also the E-step at 2 * dim_half).
 struct ConvertWorkspace {
@@ -1115,6 +1323,9 @@ struct ConvertWorkspace {
     double* pc;            // EM: (K, 2 Dh, 2 Dh)
     double* aux;           // EM: (K, 2 Dh + 2)
     double* chain;         // full covariance: (total, 3 sd^2 + sd) block-Cholesky factors and z
+    double* x;             // stream: (total, Dh) source vectors, one per slot row
+    int* slots;            // stream: (total) the slots of the rows
+    long long* jrow;       // stream: (total) the static each row delivers
     char* tc;              // tensor-core region of tc_bytes (0 at precision 0)
     size_t tc_bytes;
     size_t bytes;
@@ -1132,7 +1343,7 @@ static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, 
     w.cursor = c.take<int>((size_t)K);
     w.order = c.take<int>((size_t)total);
     w.E = c.take<double>((size_t)total * Dh);
-    if (kind != CONVERT_FULLCOV) {
+    if (kind != CONVERT_FULLCOV && kind != CONVERT_STREAM) {
         w.band = c.take<double>(4 * (size_t)total * sd);
         w.flags = c.take<unsigned char>((size_t)total);
     }
@@ -1150,6 +1361,11 @@ static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, 
         w.aux = c.take<double>((size_t)K * (D + 2));
     }
     if (kind == CONVERT_FULLCOV) w.chain = c.take<double>((size_t)total * (3 * (size_t)sd * sd + sd));
+    if (kind == CONVERT_STREAM) {
+        w.x = c.take<double>((size_t)total * Dh);
+        w.slots = c.take<int>((size_t)total);
+        w.jrow = c.take<long long>((size_t)total);
+    }
     if (precision == 1) {
         w.tc_bytes = tc_workspace_bytes(total, K, Dh);
         if (kind == CONVERT_EM)
@@ -1595,4 +1811,122 @@ extern "C" int kw_convert_fullcov_batch(int n_utts, const int64_t* off_dev, int6
         KW_CUDA_CHECK(cudaMemcpyAsync(mix_dev, w.mix, sizeof(int32_t) * total,
                                       cudaMemcpyDeviceToDevice, st));
     return KW_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Low-delay conversion over n_slots concurrent streams (kw_convert_stream_*).
+
+namespace kw {
+
+constexpr int STREAM_MAX_DELAY = 8192;  // 41 s of 5 ms frames; the push's work grows with it
+
+static int check_stream(const char* fn, int n_slots, int delay, int m, const int32_t* slots_host,
+                        int K, int Dh, int precision) {
+    KW_REQUIRE(n_slots > 0 && n_slots < (1 << 26), "%s: n_slots %d out of range", fn, n_slots);
+    KW_REQUIRE(delay >= 0 && delay <= STREAM_MAX_DELAY, "%s: delay %d is not in [0, %d]", fn,
+               delay, STREAM_MAX_DELAY);
+    KW_REQUIRE(m >= 0 && m <= n_slots, "%s: m %d is not in [0, n_slots = %d]", fn, m, n_slots);
+    KW_REQUIRE(m == 0 || slots_host != nullptr, "%s: slots missing", fn);
+    std::vector<char> seen(m > 0 ? (size_t)n_slots : 0, 0);
+    for (int i = 0; i < m; ++i) {
+        const int s = slots_host[i];
+        KW_REQUIRE(s >= 0 && s < n_slots, "%s: slot %d out of range [0, %d)", fn, s, n_slots);
+        KW_REQUIRE(!seen[s], "%s: slot %d given twice", fn, s);
+        seen[s] = 1;
+    }
+    return check_convert(fn, 1, 1, K, Dh, precision, Dh);
+}
+
+// Source rows, the hard sequence of the m frames, then the step (push) or end kernel.
+static int stream_run(const char* fn, bool end, int n_slots, int delay, int m,
+                      const int32_t* slots_host, const double* static_dev, int K, int Dh,
+                      const double* prepared_dev, double* state_dev, double* out_dev,
+                      int64_t* index_dev, int precision, void* workspace_dev,
+                      size_t workspace_bytes, cudaStream_t st) {
+    int rc = check_stream(fn, n_slots, delay, m, slots_host, K, Dh, precision);
+    if (rc != KW_OK) return rc;
+    KW_REQUIRE(state_dev != nullptr && out_dev != nullptr && index_dev != nullptr &&
+                   (end || static_dev != nullptr),
+               "%s: missing device buffer", fn);
+    const ConvertWorkspace w = carve_convert(CONVERT_STREAM, m, K, Dh, precision, workspace_dev);
+    if (w.bytes > workspace_bytes) return workspace_too_small(fn, w.bytes, workspace_bytes);
+    if (m == 0) return KW_OK;
+    const int sd = Dh / 3;
+    const StreamState s = view_stream_state(state_dev, n_slots, sd, delay);
+    const PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
+    // pageable or pinned: the call returns once slots_host has been read
+    KW_CUDA_CHECK(cudaMemcpyAsync(w.slots, slots_host, sizeof(int) * m, cudaMemcpyHostToDevice, st));
+    convert_stream_source_kernel<<<(unsigned)((32LL * m + 127) / 128), 128, 0, st>>>(
+        m, sd, end ? 1 : 0, w.slots, static_dev, s, n_slots, w.x, w.jrow);
+    KW_CUDA_CHECK(cudaGetLastError());
+    rc = hard_sequence(m, w.x, K, Dh, precision, v, w, st);
+    if (rc != KW_OK) return rc;
+    StreamStepArgs g;
+    g.m = m;
+    g.n_slots = n_slots;
+    g.sd = sd;
+    g.Dh = Dh;
+    g.delay = delay;
+    g.slots = w.slots;
+    g.jrow = w.jrow;
+    g.mix = w.mix;
+    g.E = w.E;
+    g.var = v.var;
+    g.s = s;
+    g.win = kDeltaWindows;
+    g.out = out_dev;
+    g.index = index_dev;
+    const unsigned blocks = (unsigned)(((long long)m * sd + 127) / 128);
+    if (end)
+        convert_stream_step_kernel<true><<<blocks, 128, 0, st>>>(g);
+    else
+        convert_stream_step_kernel<false><<<blocks, 128, 0, st>>>(g);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+}  // namespace kw
+
+extern "C" size_t kw_convert_stream_state_len(int n_slots, int Dh, int delay) {
+    return view_stream_state(nullptr, n_slots, Dh / 3, delay).len;
+}
+
+extern "C" int kw_convert_stream_init(int n_slots, int Dh, int delay, double* state_dev,
+                                      void* stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    KW_REQUIRE(n_slots > 0 && n_slots < (1 << 26),
+               "kw_convert_stream_init: n_slots %d out of range", n_slots);
+    KW_REQUIRE(Dh > 0 && Dh % 3 == 0,
+               "kw_convert_stream_init: dim_half %d is not static+delta+delta2 (multiple of 3)", Dh);
+    KW_REQUIRE(delay >= 0 && delay <= STREAM_MAX_DELAY,
+               "kw_convert_stream_init: delay %d is not in [0, %d]", delay, STREAM_MAX_DELAY);
+    KW_REQUIRE(state_dev != nullptr, "kw_convert_stream_init: missing state");
+    KW_CUDA_CHECK(cudaMemsetAsync(
+        state_dev, 0, sizeof(double) * kw_convert_stream_state_len(n_slots, Dh, delay), st));
+    return KW_OK;
+}
+
+extern "C" size_t kw_convert_stream_workspace_bytes(int m, int K, int Dh, int delay,
+                                                    int precision) {
+    (void)delay;
+    return carve_convert(CONVERT_STREAM, m, K, Dh, precision, nullptr).bytes;
+}
+
+extern "C" int kw_convert_stream_push(int n_slots, int delay, int m, const int32_t* slots_host,
+                                      const double* static_dev, int K, int Dh,
+                                      const double* prepared_dev, double* state_dev,
+                                      double* out_dev, int64_t* frame_dev, int precision,
+                                      void* workspace_dev, size_t workspace_bytes, void* stream) {
+    return stream_run("kw_convert_stream_push", false, n_slots, delay, m, slots_host, static_dev,
+                      K, Dh, prepared_dev, state_dev, out_dev, frame_dev, precision,
+                      workspace_dev, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int kw_convert_stream_end(int n_slots, int delay, int m, const int32_t* slots_host,
+                                     int K, int Dh, const double* prepared_dev, double* state_dev,
+                                     double* out_dev, int64_t* count_dev, int precision,
+                                     void* workspace_dev, size_t workspace_bytes, void* stream) {
+    return stream_run("kw_convert_stream_end", true, n_slots, delay, m, slots_host, nullptr, K,
+                      Dh, prepared_dev, state_dev, out_dev, count_dev, precision, workspace_dev,
+                      workspace_bytes, static_cast<cudaStream_t>(stream));
 }

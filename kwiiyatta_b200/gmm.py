@@ -607,6 +607,12 @@ class B200GMMFeatureConverter(FeatureConverter):
         conditional covariance (``MLPG(conditional_covariance=)``)."""
         return self._mlpg(diff, mlpg, gv, em_iter, conditional_covariance).transform(feature)
 
+    def stream(self, n_slots, delay, diff=False):
+        """Low-delay conversion of up to ``n_slots`` concurrent streams with a lag of ``delay``
+        frames (``MLPG.stream``).  The streams take (m, 24) frames, the mel-cepstrum without c0:
+        the caller re-attaches c0, as the mel-cepstrum layer does offline."""
+        return self._mlpg(diff).stream(n_slots, delay)
+
     def convert_many(self, features, diff=False, gv=False, em_iter=0,
                      conditional_covariance='diagonal'):
         """Batched ``convert`` over a list of (T_i, 72) arrays."""

@@ -1,7 +1,8 @@
 """Posterior + MLPG on the B200 (nnmnkwii.baseline.gmm.MLPG as used at
 kwiiyatta/converter/gmm.py:28-34), optionally with global variance (``gv=``; kwiiyatta_b200.gv),
 maximum-likelihood conversion over all mixture sequences (``em_iter=``) or the full conditional
-covariance (``conditional_covariance='full'``)."""
+covariance (``conditional_covariance='full'``), and low-delay conversion of many concurrent streams
+(``MLPG.stream``)."""
 import numpy as np
 
 from . import _lib
@@ -326,6 +327,20 @@ class MLPG:
                   _lib.stream_ptr(torch))
         return out.cpu().numpy()
 
+    def stream(self, n_slots, delay):
+        """Low-delay conversion of up to ``n_slots`` concurrent streams (``MLPGStream``): the frame
+        emitted for static frame ``j`` of a stream is frame ``j - 1 - delay`` of the MLPG solution
+        of the frames known so far (fixed-lag MLPG, Muramatsu et al., Interspeech 2008), so a
+        frame comes out ``delay + 1`` frames after its static went in.  With
+        ``delay >= T - 1`` a stream of ``T`` frames gets exactly ``transform``'s output."""
+        if self.gv is not None or self.em_iter or self._fullcov is not None:
+            raise ValueError('low-delay conversion is built for the hard-sequence MLPG with the '
+                             'diagonal conditional covariance only (no GV, EM or full covariance)')
+        if len(self.windows) == 1:
+            raise ValueError('low-delay conversion is defined for MLPG trajectories only (not '
+                             'with a single static window)')
+        return MLPGStream(self, n_slots, delay)
+
     def transform(self, src):
         src = np.asarray(src, dtype=np.float64)
         if src.ndim != 2:
@@ -334,3 +349,93 @@ class MLPG:
             # nnmnkwii: feature_dim == static_dim -> MLPGBase.transform (no trajectory smoothing)
             return self.transform_soft(src)
         return self.transform_many([src])[0]
+
+
+class MLPGStream:
+    """Low-delay conversion state of ``n_slots`` streams on an ``MLPG``'s device
+    (kw_convert_stream_*).  Each call delivers one static frame (``static_dim`` values: the
+    mel-cepstrum without c0) to each of a set of distinct slots; a slot holds one stream from its
+    first ``push`` to its ``end``."""
+
+    def __init__(self, mlpg, n_slots, delay):
+        torch = _lib.require_cuda()
+        self.mlpg, self.n_slots, self.delay = mlpg, int(n_slots), int(delay)
+        if self.n_slots < 1:
+            raise ValueError(f'n_slots must be >= 1, got {n_slots}')
+        if self.delay < 0:
+            raise ValueError(f'delay must be >= 0, got {delay}')
+        self._dev = mlpg._dev
+        with torch.cuda.device(self._dev):
+            n = _lib.lib().kw_convert_stream_state_len(self.n_slots, mlpg.dim_half, self.delay)
+            self._state = torch.empty(n, dtype=torch.float64, device=self._dev)
+            _lib.call('kw_convert_stream_init', self.n_slots, mlpg.dim_half, self.delay,
+                      self._state, _lib.stream_ptr(torch))
+
+    def _slots(self, slots):
+        s = np.asarray(slots)
+        if s.ndim != 1 or (s.size and s.dtype.kind not in 'iu'):
+            raise ValueError('slots must be a 1-D array of integers')
+        if s.size and (s.min() < 0 or s.max() >= self.n_slots):
+            raise ValueError(f'slots must be in [0, {self.n_slots})')
+        if len(np.unique(s)) != len(s):
+            raise ValueError('slots must be distinct')
+        return np.ascontiguousarray(s, dtype=np.int32)
+
+    def _workspace(self, m):
+        g = self.mlpg
+        ws_bytes = _lib.lib().kw_convert_stream_workspace_bytes(m, g.num_mixtures, g.dim_half,
+                                                               self.delay, g.precision)
+        return _lib.workspace(ws_bytes, self._dev), ws_bytes
+
+    @_on_own_device
+    def push_device(self, slots, frames):
+        """``frames`` (m, static_dim) float64 CUDA tensor, one static frame for each slot of the
+        host array ``slots``.  Returns CUDA tensors ``out`` (m, static_dim), the emitted frames,
+        and ``frame_index`` (m,) int64, their frame numbers in their streams (-1 and a zero row
+        where a stream has not yet emitted).  Queued on the current stream, no synchronisation."""
+        torch = _lib.require_cuda()
+        g = self.mlpg
+        s = self._slots(slots)
+        m = len(s)
+        if (tuple(frames.shape) != (m, g.static_dim) or frames.dtype != torch.float64
+                or not frames.is_cuda or frames.device.index != torch.cuda.current_device()):
+            raise ValueError(f'frames must be a float64 tensor of shape ({m}, {g.static_dim}) '
+                             f'on the MLPG\'s device {self._dev}')
+        frames = frames.contiguous()
+        out = torch.empty((m, g.static_dim), dtype=torch.float64, device=frames.device)
+        index = torch.empty(m, dtype=torch.int64, device=frames.device)
+        ws, ws_bytes = self._workspace(m)
+        _lib.call('kw_convert_stream_push', self.n_slots, self.delay, m, s, frames,
+                  g.num_mixtures, g.dim_half, g._prepared, self._state, out, index, g.precision,
+                  ws, ws_bytes, _lib.stream_ptr(torch))
+        return out, index
+
+    @_on_own_device
+    def push(self, slots, frames):
+        """``push_device`` from and to host arrays: ``frames`` (m, static_dim) -> (``out``
+        (m, static_dim), ``frame_index`` (m,)) as numpy arrays."""
+        torch = _lib.require_cuda()
+        f = np.ascontiguousarray(frames, dtype=np.float64)
+        if f.ndim != 2 or f.shape[1] != self.mlpg.static_dim:
+            raise ValueError(f'expected (m, {self.mlpg.static_dim}) static frames, got {f.shape}')
+        out, index = self.push_device(slots, torch.from_numpy(f).to(self._dev))
+        return out.cpu().numpy(), index.cpu().numpy()
+
+    @_on_own_device
+    def end(self, slots):
+        """End the streams of ``slots`` (which are then empty): a list with, per slot, the
+        (k, static_dim) array of its last k = min(T, delay + 1) frames (none for an empty
+        slot)."""
+        torch = _lib.require_cuda()
+        g = self.mlpg
+        s = self._slots(slots)
+        m = len(s)
+        out = torch.empty((m, self.delay + 1, g.static_dim), dtype=torch.float64,
+                          device=self._dev)
+        count = torch.empty(m, dtype=torch.int64, device=self._dev)
+        ws, ws_bytes = self._workspace(m)
+        _lib.call('kw_convert_stream_end', self.n_slots, self.delay, m, s, g.num_mixtures,
+                  g.dim_half, g._prepared, self._state, out, count, g.precision, ws, ws_bytes,
+                  _lib.stream_ptr(torch))
+        out, count = out.cpu().numpy(), count.cpu().numpy()
+        return [out[i, :int(count[i])].copy() for i in range(m)]
