@@ -142,7 +142,9 @@ int kw_gmm_normalize_resp(int64_t n_frames, int n_components, int dim, double* r
 
 /* Hard assignment argmax_k of the weighted log-probability (sklearn predict; with identity
  * precisions and equal weights this is the k-means assignment step).  labels_dev[n_frames] int32.
- * With precision 1 near-ties are re-evaluated in fp64, so the labels equal the fp64 argmax. */
+ * With precision 1 every frame whose tensor-core runner-up lies within 0.05 nat of its best is
+ * re-evaluated in fp64: the two of them, or all components when a third one is within 0.05 nat as
+ * well.  The labels therefore equal the fp64 argmax (the lowest index on equal fp64 values). */
 int kw_gmm_hard_labels(int64_t n_frames, const double* x_dev, int n_components, int dim,
                        const double* means_dev, const double* prec_chol_dev, const double* aux_dev,
                        int32_t* labels_dev, int precision,

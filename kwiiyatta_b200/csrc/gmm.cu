@@ -401,15 +401,19 @@ __global__ void gmm_reduce_partials_kernel(int K, int D, int chunks,
 // Cholesky factor sklearn keeps).  Both factorisations are blocked by FIN_NB columns so the
 // bulk of the flops are register-tiled panel products and the number of block-wide barriers
 // is ~2 per column instead of 3 plus a serial triangular sweep.
-// Dynamic smem: D * S doubles (S = D | 1), FIN_NB + 1 doubles per column of scratch, 3 D
-// doubles of diagonals / means.
+// Dynamic smem: D * S doubles (S = D | 1), FIN_NB + 1 doubles per column of scratch (for at
+// least two columns: the diagonal block also keeps its 1 / L[c][c] at scratch offset 2 FIN_NB,
+// past the end of a one-column scratch), 3 D doubles of diagonals / means.
 // ---------------------------------------------------------------------------------------
 constexpr int FIN_NB = 16;
 constexpr int FIN_THREADS = 512;
 
+__host__ __device__ inline size_t finalize_scratch(int D) {
+    return (size_t)(D > 2 ? D : 2) * (FIN_NB + 1);
+}
 static size_t finalize_smem_bytes(int D) {
     const size_t S = (size_t)D | 1;
-    return sizeof(double) * ((size_t)D * S + (size_t)D * (FIN_NB + 1) + 3 * (size_t)D);
+    return sizeof(double) * ((size_t)D * S + finalize_scratch(D) + 3 * (size_t)D);
 }
 
 __global__ void __launch_bounds__(FIN_THREADS)
@@ -421,7 +425,7 @@ gmm_finalize_kernel(int K, int D, double reg_covar, int weight_norm, int from_st
     extern __shared__ double A[];
     const int S = D | 1;
     double* T = A + (size_t)D * S;            // [column][FIN_NB + 1] scratch of the inverse
-    double* dg = T + (size_t)D * (FIN_NB + 1);   // L[j][j]
+    double* dg = T + finalize_scratch(D);     // L[j][j]
     double* zd = dg + D;                      // 1 / L[j][j]
     double* dm = zd + D;                      // first moments / n_k
     __shared__ int sh_fail;

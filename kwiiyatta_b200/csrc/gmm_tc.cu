@@ -535,16 +535,23 @@ __host__ __device__ inline EstepSmem estep_smem(int DP, int G) {
     return s;
 }
 
+// cand[n] of the mode-1 E-step: -1 = the label stands, k >= 0 = compare with component k in
+// fp64, REFINE_ALL = take the fp64 argmax over all components
+constexpr int32_t REFINE_ALL = -2;
+
 enum { BAR_A_FULL = 0, BAR_A_EMPTY, BAR_BLO_FULL0, BAR_BLO_FULL1, BAR_BLO_EMPTY0, BAR_BLO_EMPTY1,
        BAR_BHI_FULL0, BAR_BHI_FULL1,
        BAR_BHI_EMPTY0, BAR_BHI_EMPTY1, BAR_TM_FULL0, BAR_TM_FULL1, BAR_TM_EMPTY0, BAR_TM_EMPTY1 };
 
-template <int G>
+// MODE 0: weighted log-probabilities into wlpT; MODE 1: hard labels into mix and cand.  (The
+// mode is a template parameter so that each instantiation keeps only the registers of its own
+// epilogue.)
+template <int G, int MODE>
 __global__ void __launch_bounds__(576, 1)
 estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                 uint32_t tmem_cols, const __half* __restrict__ xt, const __half* __restrict__ bt,
                 const double* __restrict__ cst,
-                double* __restrict__ wlpT, int mode, int32_t* __restrict__ mix,
+                double* __restrict__ wlpT, int32_t* __restrict__ mix,
                 int32_t* __restrict__ cand, double near_tie, int late_release) {
     extern __shared__ __align__(128) unsigned char smem[];
     const EstepSmem L = estep_smem(DP, G);
@@ -704,6 +711,7 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
             const long long n = (long long)tile * TILE_M + row;
             double v1 = -CUDART_INF, v2 = -CUDART_INF;
+            float v3 = -CUDART_INF_F;     // third best: only compared with near_tie
             int k1 = 0, k2 = -1;
             // per-component constants [log|L|, log w, 4^t] (part 0 finishes the item's
             // components), prefetched one item ahead
@@ -800,20 +808,27 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                             const double q = c ? qb : qa;
                             const double wlp =
                                 (-0.5 * ((double)D * LOG2PI + q * cc[c][2]) + cc[c][0]) + cc[c][1];
-                            if (mode == 0) {
+                            if (MODE == 0) {
                                 if (n < N) wlpT[(size_t)k * Npad + n] = wlp;
                             } else if (wlp > v1) {
-                                v2 = v1; k2 = k1; v1 = wlp; k1 = k;
+                                v3 = (float)v2; v2 = v1; k2 = k1; v1 = wlp; k1 = k;
                             } else if (wlp > v2) {
-                                v2 = wlp; k2 = k;
+                                v3 = (float)v2; v2 = wlp; k2 = k;
+                            } else {
+                                v3 = fmaxf(v3, (float)wlp);
                             }
                         }
                     }
                 }
             }
-            if (part == 0 && mode == 1 && n < N) {
+            if (part == 0 && MODE == 1 && n < N) {
+                // to re-check in fp64: the runner-up when only it is within near_tie of the best,
+                // every component (REFINE_ALL) when a third one is as well -- with three near the
+                // top the tensor cores may have ranked the fp64 best third
                 mix[n] = k1;
-                cand[n] = (K > 1 && v1 - v2 < near_tie) ? k2 : -1;   // runner-up to re-check in fp64
+                cand[n] = (K > 2 && v1 - (double)v3 < near_tie) ? REFINE_ALL
+                          : (K > 1 && v1 - v2 < near_tie)         ? k2
+                                                                  : -1;
             }
         }
     }
@@ -877,47 +892,92 @@ lse_kernel(long long N, long long Npad, int K, double* __restrict__ respT,
     }
 }
 
-// Hard-assignment near-ties: frames whose two best components are closer than the tensor-core
-// error budget are re-evaluated for those two components in FP64 (one warp per frame), so the
-// mixture sequence equals the FP64 argmax.
-__global__ void refine_argmax_kernel(long long N, int D, const double* __restrict__ X,
+// FP64 weighted log-probability of component k (precision Cholesky Lk, aux ak) for the frame
+// whose features the warp holds as xr[t] = x[lane + 32 t] (D <= 160).  Lane l owns the columns
+// j = l + 32 t of y = x Lk, each summed over ascending d as in the FP64 E-step; the frame's
+// features reach the lanes by shuffle and the loads of Lk run ahead of the FMAs.  The sum of
+// squares only grows, column block by column block: as soon as the partial value is below
+// `floor`, the final one is too, and the function returns -inf.
+__device__ double warp_wlp_fp64(int D, const double (&xr)[5], const double* __restrict__ Lk,
+                                const double* __restrict__ ak, double floor) {
+    const int lane = threadIdx.x & 31;
+    const double LOG2PI = 1.8378770664093453;
+    double q = 0.0, w = -CUDART_INF;
+#pragma unroll
+    for (int t = 0; t < 5; ++t) {
+        if (32 * t >= D) break;
+        const int j = lane + 32 * t, jj = min(j, D - 1);
+        double y = 0.0;
+#pragma unroll
+        for (int tb = 0; tb <= t; ++tb) {
+            const double xv = xr[tb];
+            const int dn = min(32, D - 32 * tb);
+            for (int d0 = 0; d0 < dn; d0 += 16) {
+                double l[16];            // sixteen loads in flight before the first FMA
+#pragma unroll
+                for (int u = 0; u < 16; ++u)
+                    l[u] = Lk[(size_t)min(32 * tb + d0 + u, D - 1) * D + jj];
+#pragma unroll
+                for (int u = 0; u < 16; ++u) {
+                    const int d = 32 * tb + d0 + u;
+                    const double xd = __shfl_sync(0xffffffffu, xv, (d0 + u) & 31);
+                    // L is upper triangular; rows past D (last batch) contribute nothing
+                    y = fma(xd, (d <= j && d0 + u < dn) ? l[u] : 0.0, y);
+                }
+            }
+        }
+        if (j < D) {
+            y -= ak[j];
+            q = fma(y, y, q);
+        }
+        w = (-0.5 * ((double)D * LOG2PI + warp_sum(q)) + ak[D]) + ak[D + 1];
+        if (w < floor) return -CUDART_INF;
+    }
+    return w;
+}
+
+// Hard-assignment near-ties: frames whose best components are closer than the tensor-core error
+// budget are re-evaluated in FP64 (one warp per frame) -- the best and the runner-up, or all K
+// components when a third is close too -- so the mixture sequence equals the FP64 argmax (the
+// lowest index on equal FP64 values).  The label's own value comes first, so that the other
+// components stop as soon as they fall below it.
+__global__ void refine_argmax_kernel(long long N, int K, int D, const double* __restrict__ X,
                                      const double* __restrict__ prec_chol,
                                      const double* __restrict__ aux, int32_t* __restrict__ mix,
                                      const int32_t* __restrict__ cand) {
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
-    const double LOG2PI = 1.8378770664093453;
     // a warp looks at 32 frames at a time (one coalesced load of their candidates) and re-checks
     // the flagged ones in turn
     for (long long n0 = warp * 32; n0 < N; n0 += n_warps * 32) {
       const int mine = (n0 + lane < N) ? cand[n0 + lane] : -1;
-      unsigned todo = __ballot_sync(0xffffffffu, mine >= 0);
+      unsigned todo = __ballot_sync(0xffffffffu, mine != -1);
       while (todo) {
         const int src = __ffs(todo) - 1;
         todo &= todo - 1;
         const long long n = n0 + src;
         const int kb = __shfl_sync(0xffffffffu, mine, src);
         const int ka = mix[n];
-        double w[2];
-        for (int c = 0; c < 2; ++c) {
-            const int k = c == 0 ? ka : kb;
-            const double* Lk = prec_chol + (size_t)k * D * D;
-            const double* ak = aux + (size_t)k * (D + 2);
-            double q = 0.0;
-            for (int j = lane; j < D; j += 32) {
-                double y = 0.0;
-                for (int d = 0; d <= j; ++d) y = fma(X[n * D + d], Lk[(size_t)d * D + j], y);
-                y -= ak[j];
-                q = fma(y, y, q);
+        double xr[5];
+#pragma unroll
+        for (int t = 0; t < 5; ++t)
+            xr[t] = (lane + 32 * t < D) ? X[n * D + lane + 32 * t] : 0.0;
+        double wbest = warp_wlp_fp64(D, xr, prec_chol + (size_t)ka * D * D,
+                                     aux + (size_t)ka * (D + 2), -CUDART_INF);
+        int kbest = ka;
+        const bool all = kb == REFINE_ALL;
+        for (int c = 0; c < (all ? K : 1); ++c) {
+            const int k = all ? c : kb;
+            if (k == ka) continue;
+            const double w = warp_wlp_fp64(D, xr, prec_chol + (size_t)k * D * D,
+                                           aux + (size_t)k * (D + 2), wbest);
+            if (w > wbest || (w == wbest && k < kbest)) {
+                wbest = w;
+                kbest = k;
             }
-            q = warp_sum(q);
-            w[c] = (-0.5 * ((double)D * LOG2PI + q) + ak[D]) + ak[D + 1];
         }
-        if (lane == 0) {
-            const bool take_b = (w[1] > w[0]) || (w[1] == w[0] && kb < ka);
-            if (take_b) mix[n] = kb;
-        }
+        if (lane == 0) mix[n] = kbest;
       }
     }
 }
@@ -1986,14 +2046,17 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
         KW_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)L.total));
         kern<<<grid, 576, L.total, st>>>(N, Npad, (int)n_tiles, K, D, DP, cols, w.xt, w.bt, w.cst,
-                                         resp, mode, mix, w.cand, 0.05, late_release);
+                                         resp, mix, w.cand, 0.05, late_release);
         return KW_OK;
     };
-    rc = (G == 2) ? launch(tc::estep_tc_kernel<2>) : launch(tc::estep_tc_kernel<1>);
+    if (mode == 1)
+        rc = (G == 2) ? launch(tc::estep_tc_kernel<2, 1>) : launch(tc::estep_tc_kernel<1, 1>);
+    else
+        rc = (G == 2) ? launch(tc::estep_tc_kernel<2, 0>) : launch(tc::estep_tc_kernel<1, 0>);
     if (rc != KW_OK) return rc;
     KW_CUDA_CHECK(cudaGetLastError());
     if (mode == 1) {
-        tc::refine_argmax_kernel<<<sms * 4, 256, 0, st>>>(N, D, X, pc, aux, mix, w.cand);
+        tc::refine_argmax_kernel<<<sms * 4, 256, 0, st>>>(N, K, D, X, pc, aux, mix, w.cand);
         KW_CUDA_CHECK(cudaGetLastError());
         return KW_OK;
     }
@@ -2008,7 +2071,10 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
         const int n_mt_pad = (w.n_mtiles + 3) / 4 * 4;
         // one 64-frame tile per block: 512 K bytes of shared memory, several blocks per SM
         const int sm = K * 64 * (int)sizeof(double);
-        lgrid = (unsigned)((N + 63) / 64);
+        // every M-step tile up to n_mt_pad: the M-step reads the flags of all 2 n_tiles tiles (the
+        // last one of a final E-tile with at most 64 frames included) and sums the tile weights of
+        // all n_mt_pad; a block past N writes "no weight"
+        lgrid = (unsigned)n_mt_pad;
         KW_CUDA_CHECK(cudaFuncSetAttribute(tc::lse_prep_kernel<64>,
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
         tc::lse_prep_kernel<64><<<lgrid, 128, sm, st>>>(

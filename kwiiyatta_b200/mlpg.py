@@ -123,7 +123,7 @@ class MLPG:
         self.dim_half = d // 2
         self.static_dim = d // 2 // len(windows)
         # 'auto' = the tcgen05 posterior whenever the kernels hold the frame width: its hard
-        # labels are re-checked in FP64 where the two best mixtures are close, so the mixture
+        # labels are re-checked in FP64 where the best mixtures are close, so the mixture
         # sequence and the (FP64) MLPG output are those of the FP64 path
         self.precision = {'fp64': 0, 'tc': 1, 0: 0, 1: 1,
                           'auto': 1 if self.dim_half <= 144 else 0}[precision]
