@@ -16,7 +16,6 @@
 // restated in oracle/mlpg_full_ref.py).  Its workspace keeps the block factors between the
 // forward and the backward sweep: (3 sd^2 + sd) doubles per frame, 14 KB at sd = 24, where the
 // diagonal path's band takes 768 B.
-#include <algorithm>
 #include <vector>
 
 #include "common.cuh"
@@ -1299,9 +1298,9 @@ enum ConvertKind { CONVERT_PLAIN, CONVERT_GV, CONVERT_EM, CONVERT_FULLCOV, CONVE
 // The workspace of one conversion call, in this order: the hard-sequence buffers every kind uses
 // (the band set and the utterance flags except for the full-covariance kind, whose block solve
 // takes neither, and the stream kind, which keeps its band in the stream state), then the GV
-// step plane, the EM buffers, the block-solve chain or the stream's source rows, then the
-// tensor-core region of the E-steps the call runs (precision 1 only: the hard-sequence E-step at
-// dim_half, and for EM also the E-step at 2 * dim_half).
+// step plane, the EM buffers, the block-solve chain or the stream's source rows, then the GMM
+// layer's region of the E-steps the call runs: the hard-sequence labels at dim_half, and for EM
+// also the posteriors at 2 * dim_half.
 struct ConvertWorkspace {
     int32_t* mix;          // (total) hard mixture sequence
     int* counts;           // K      (counting sort of the frames by mixture)
@@ -1316,7 +1315,6 @@ struct ConvertWorkspace {
     double* z;             // EM: (total, 2 Dh) joint frames [x | W y]
     double* resp;          // EM: (K, resp_pad(total))
     double* lse;           // EM: (total) per-frame log-normaliser
-    double* lsep;          // EM: E-step partial sums (at most one per frame) + the two-value total
     double* q;             // EM: (total, Dh)
     double* prec;          // EM: (total, Dh)
     double* means;         // EM: (K, 2 Dh)
@@ -1326,8 +1324,7 @@ struct ConvertWorkspace {
     double* x;             // stream: (total, Dh) source vectors, one per slot row
     int* slots;            // stream: (total) the slots of the rows
     long long* jrow;       // stream: (total) the static each row delivers
-    char* tc;              // tensor-core region of tc_bytes (0 at precision 0)
-    size_t tc_bytes;
+    GmmWorkspace gmm;      // the E-steps
     size_t bytes;
 };
 
@@ -1353,7 +1350,6 @@ static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, 
         w.z = c.take<double>((size_t)total * D);
         w.resp = c.take<double>((size_t)K * (size_t)resp_pad(total));
         w.lse = c.take<double>((size_t)total);
-        w.lsep = c.take<double>((size_t)total + 2);
         w.q = c.take<double>((size_t)total * Dh);
         w.prec = c.take<double>((size_t)total * Dh);
         w.means = c.take<double>((size_t)K * D);
@@ -1366,12 +1362,8 @@ static ConvertWorkspace carve_convert(ConvertKind kind, long long total, int K, 
         w.slots = c.take<int>((size_t)total);
         w.jrow = c.take<long long>((size_t)total);
     }
-    if (precision == 1) {
-        w.tc_bytes = tc_workspace_bytes(total, K, Dh);
-        if (kind == CONVERT_EM)
-            w.tc_bytes = std::max(w.tc_bytes, tc_workspace_bytes(total, K, 2 * Dh));
-    }
-    w.tc = c.take<char>(w.tc_bytes);
+    w.gmm = kind == CONVERT_EM ? carve_gmm(c, total, K, 2 * Dh, precision, GmmUse::Posterior)
+                               : carve_gmm(c, total, K, Dh, precision, GmmUse::Labels);
     w.bytes = align_up(c.used, 256);
     return w;
 }
@@ -1383,9 +1375,9 @@ static int check_convert(const char* fn, int n_utts, long long total, int K, int
     KW_REQUIRE(n_utts > 0 && total > 0 && K > 0, "%s: bad sizes", fn);
     KW_REQUIRE(Dh % 3 == 0, "%s: dim_half %d is not static+delta+delta2 (multiple of 3)", fn, Dh);
     KW_REQUIRE(precision == 0 || precision == 1, "%s: precision must be 0 or 1", fn);
-    if (estep_dim > 144) {
-        set_error("%s: dim_half %d: the E-step at dimension %d > 144 is not supported", fn, Dh,
-                  estep_dim);
+    if (estep_dim > GMM_MAX_DIM) {
+        set_error("%s: dim_half %d: the E-step at dimension %d > %d is not supported", fn, Dh,
+                  estep_dim, GMM_MAX_DIM);
         return KW_ERR_UNSUPPORTED;
     }
     KW_REQUIRE(Dh <= 80, "%s: dim_half %d > 80 unsupported", fn, Dh);
@@ -1405,16 +1397,10 @@ static const Windows kDeltaWindows = {{{0.0, 1.0, 0.0}, {-0.5, 0.0, 0.5}, {1.0, 
 // scatter) and one pass per mixture.
 static int hard_sequence(long long total, const double* src, int K, int Dh, int precision,
                          const PreparedView& v, const ConvertWorkspace& w, cudaStream_t st) {
-    int rc;
-    if (precision == 1) {
-        rc = pack_frames_tc(total, src, K, Dh, w.tc, w.tc_bytes, st, /*mstep_parts=*/false);
-        if (rc != KW_OK) return rc;
-        rc = estep_tc(total, src, K, Dh, v.src_means, v.px_prec_chol, v.px_aux, nullptr, nullptr,
-                      1, w.mix, w.tc, w.tc_bytes, st);
-    } else {
-        rc = estep_fp64(total, src, K, Dh, v.px_prec_chol, v.px_aux, nullptr, nullptr, 1, w.mix,
-                        st);
-    }
+    int rc = pack_frames(total, src, Dh, precision, w.gmm, st, /*mstep_parts=*/false);
+    if (rc == KW_OK)
+        rc = estep_labels(total, src, K, Dh, v.src_means, v.px_prec_chol, v.px_aux, precision,
+                          w.gmm, w.mix, st);
     if (rc != KW_OK) return rc;
     KW_CUDA_CHECK(cudaMemsetAsync(w.counts, 0, sizeof(int) * K, st));
     convert_hist_kernel<<<296, 256, sizeof(int) * K, st>>>(total, K, w.mix, w.counts);
@@ -1513,7 +1499,7 @@ extern "C" int kw_convert_prepare(int K, int Dh, int diff, const double* weights
 extern "C" size_t kw_convert_soft_workspace_bytes(int64_t total_frames, int K, int Dh) {
     Carver c(nullptr);
     c.take<double>((size_t)K * (size_t)resp_pad(total_frames));
-    c.take<double>((size_t)((total_frames + 63) / 64) + 1);
+    carve_gmm(c, total_frames, K, Dh, 0, GmmUse::Posterior);
     return align_up(c.used, 256);
 }
 
@@ -1529,14 +1515,16 @@ extern "C" int kw_convert_soft_batch(int64_t total, const double* src_dev, int K
         return KW_ERR_WORKSPACE;
     }
     Carver c(workspace_dev);
-    double* resp = c.take<double>((size_t)K * (size_t)resp_pad(total));
-    double* lse = c.take<double>((size_t)((total + 63) / 64) + 1);
+    Posterior post;
+    post.resp = c.take<double>((size_t)K * (size_t)resp_pad(total));
+    const GmmWorkspace gmm = carve_gmm(c, total, K, Dh, 0, GmmUse::Posterior);
     PreparedView v = view_prepared(const_cast<double*>(prepared_dev), K, Dh);
-    int rc = estep_fp64(total, src_dev, K, Dh, v.px_prec_chol, v.px_aux, resp, lse, 0, nullptr, st);
+    int rc = estep_posterior(total, src_dev, K, Dh, nullptr, v.px_prec_chol, v.px_aux, 0, gmm,
+                             post, st);
     if (rc != KW_OK) return rc;
     const size_t smem = sizeof(double) * ((size_t)SOFT_FT * Dh + SOFT_FT);
     convert_soft_kernel<false><<<(unsigned)((total + SOFT_FT - 1) / SOFT_FT), 96, smem, st>>>(
-        total, resp_pad(total), K, Dh, src_dev, resp, v, out_dev, nullptr);
+        total, resp_pad(total), K, Dh, src_dev, post.resp, v, out_dev, nullptr);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }
@@ -1709,15 +1697,12 @@ extern "C" int kw_convert_em_batch(int n_utts, const int64_t* off_dev, int64_t t
         convert_em_frames_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(
             total, sd, out_dev, w.flags, kDeltaWindows, D, Dh, w.z);
         KW_CUDA_CHECK(cudaGetLastError());
-        int r;
-        if (precision == 1) {
-            r = pack_frames_tc(total, w.z, K, D, w.tc, w.tc_bytes, st, /*mstep_parts=*/false);
-            if (r != KW_OK) return r;
-            r = estep_tc(total, w.z, K, D, w.means, w.pc, w.aux, w.resp, w.lsep, 0, nullptr, w.tc,
-                         w.tc_bytes, st, 0, w.lse);
-        } else {
-            r = estep_fp64(total, w.z, K, D, w.pc, w.aux, w.resp, w.lsep, 0, nullptr, st, w.lse);
-        }
+        Posterior post;
+        post.resp = w.resp;
+        post.lse_frame = w.lse;
+        int r = pack_frames(total, w.z, D, precision, w.gmm, st, /*mstep_parts=*/false);
+        if (r == KW_OK)
+            r = estep_posterior(total, w.z, K, D, w.means, w.pc, w.aux, precision, w.gmm, post, st);
         if (r != KW_OK) return r;
         if (loglik_dev != nullptr) {
             convert_em_loglik_kernel<<<(unsigned)((32LL * n_utts + 255) / 256), 256, 0, st>>>(

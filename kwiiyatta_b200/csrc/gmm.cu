@@ -191,11 +191,6 @@ __global__ void reduce_fixed_kernel(const double* __restrict__ in, long long n, 
     }
 }
 
-void launch_reduce_fixed(const double* in, long long n, double extra, double* out,
-                         cudaStream_t st) {
-    reduce_fixed_kernel<<<1, 256, 0, st>>>(in, n, extra, out);
-}
-
 // ---------------------------------------------------------------------------------------
 // M-step sufficient statistics: grid (K, n_chunks, n_tile_pairs).  CTA = one W x W output tile
 // (W = 16*TM) of S_k over one chunk of frames; 256 threads, TM x TM accumulators each.
@@ -745,80 +740,81 @@ static int m_chunks(int K) {
 
 long long resp_pad(long long n) { return (n + 127) / 128 * 128; }
 
-struct GmmWorkspace {
-    double* lse_partial;
-    double* partial;
-    size_t bytes;
-};
-
-static GmmWorkspace carve_gmm(long long N, int K, int D, void* base) {
-    Carver c(base);
-    GmmWorkspace w;
-    w.lse_partial = c.take<double>((size_t)((N + E_FT - 1) / E_FT) + 1);
-    w.partial = c.take<double>((size_t)m_chunks(K) * K * stats_block(D));
-    w.bytes = align_up(c.used, 256);
+GmmWorkspace carve_gmm(Carver& c, long long N, int K, int D, int precision, GmmUse use) {
+    GmmWorkspace w = {};
+    if (use == GmmUse::Fit || (use == GmmUse::Posterior && precision == 0))
+        w.lse_partial = c.take<double>((size_t)((N + E_FT - 1) / E_FT) + 1);
+    if (use == GmmUse::Fit) w.partial = c.take<double>((size_t)m_chunks(K) * K * stats_block(D));
+    if (precision == 1) {
+        w.tc = carve_tc(c, N, K, D);
+        w.lse_partial = w.tc.lse_partial;
+    }
     return w;
 }
 
-template <int TN>
-static int launch_estep(long long N, const double* X, int K, int D, const double* pc,
-                        const double* aux, double* resp, double* lse_partial, int mode,
-                        int32_t* mix, cudaStream_t st, double* lse_frame) {
+// Columns per thread of the FP64 E-step (TN) and M-step (TM) kernels at dimension D.
+static int fp64_class(int D) { return D <= 16 ? 1 : D <= 32 ? 2 : D <= 48 ? 3 : D <= 80 ? 5 : 9; }
+
+// gmm_estep_kernel: mode 0 writes resp, lse_partial and lse_frame; mode 1 the labels.
+static int estep_fp64(long long N, const double* X, int K, int D, const double* pc,
+                      const double* aux, double* resp, double* lse_partial, int mode,
+                      int32_t* labels, cudaStream_t st, double* lse_frame) {
+    static_assert(GMM_MAX_DIM <= 16 * 9, "TN = 9 covers GMM_MAX_DIM columns");
+    const int TN = fp64_class(D);
+    auto kern = TN == 9   ? gmm_estep_kernel<9>
+                : TN == 5 ? gmm_estep_kernel<5>
+                : TN == 3 ? gmm_estep_kernel<3>
+                : TN == 1 ? gmm_estep_kernel<1>
+                          : gmm_estep_kernel<2>;
     const int Dp = (D + E_KC - 1) / E_KC * E_KC;
     const size_t smem = sizeof(double) * ((size_t)E_FT * (Dp + 1) + 2 * E_KC * 16 * TN);
-    auto kern = gmm_estep_kernel<TN>;
     KW_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)smem));
     const long long grid = (N + E_FT - 1) / E_FT;
     kern<<<(unsigned)grid, 256, smem, st>>>(N, resp_pad(N), X, K, D, pc, aux, resp, lse_partial,
-                                            mode, mix, lse_frame);
+                                            mode, labels, lse_frame);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }
 
-int estep_fp64(long long N, const double* X, int K, int D, const double* pc, const double* aux,
-               double* resp, double* lse_partial, int mode, int32_t* mix, cudaStream_t st,
-               double* lse_frame) {
-    if (D <= 16) return launch_estep<1>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
-                                        lse_frame);
-    if (D <= 32) return launch_estep<2>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
-                                        lse_frame);
-    if (D <= 48) return launch_estep<3>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
-                                        lse_frame);
-    if (D <= 80) return launch_estep<5>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
-                                        lse_frame);
-    if (D <= 144) return launch_estep<9>(N, X, K, D, pc, aux, resp, lse_partial, mode, mix, st,
-                                        lse_frame);
-    set_error("dim %d > 144 is not supported by the E-step kernels", D);
-    return KW_ERR_UNSUPPORTED;
+int estep_posterior(long long N, const double* X, int K, int D, const double* means,
+                    const double* pc, const double* aux, int precision, const GmmWorkspace& w,
+                    const Posterior& out, cudaStream_t st) {
+    long long n_partials = (N + E_FT - 1) / E_FT;
+    const int rc =
+        precision == 1
+            ? estep_tc_posterior(N, K, D, means, pc, aux, w.tc, out, n_partials, st)
+            : estep_fp64(N, X, K, D, pc, aux, out.resp, w.lse_partial, 0, nullptr, st,
+                         out.lse_frame);
+    if (rc != KW_OK || out.total == nullptr) return rc;
+    reduce_fixed_kernel<<<1, 256, 0, st>>>(w.lse_partial, n_partials, (double)N, out.total);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
 }
 
-template <int TM>
-static int launch_mstats(long long N, const double* X, int K, int D, const double* resp,
-                         const double* centres, double* partial, int chunks, double resp_floor,
-                         cudaStream_t st) {
-    const int W = 16 * TM;
-    const int n_tiles = (D + W - 1) / W;
-    const int n_pairs = n_tiles * (n_tiles + 1) / 2;
+int estep_labels(long long N, const double* X, int K, int D, const double* means,
+                 const double* pc, const double* aux, int precision, const GmmWorkspace& w,
+                 int32_t* labels, cudaStream_t st) {
+    if (precision == 1) return estep_tc_labels(N, X, K, D, means, pc, aux, w.tc, labels, st);
+    return estep_fp64(N, X, K, D, pc, aux, nullptr, nullptr, 1, labels, st, nullptr);
+}
+
+static int mstats_fp64(long long N, const double* X, int K, int D, const double* resp,
+                       const double* centres, double* partial, double* stats, double resp_floor,
+                       cudaStream_t st) {
+    const int TM = fp64_class(D);
+    auto kern = TM == 9   ? gmm_mstats_kernel<9>
+                : TM == 5 ? gmm_mstats_kernel<5>
+                : TM == 3 ? gmm_mstats_kernel<3>
+                : TM == 1 ? gmm_mstats_kernel<1>
+                          : gmm_mstats_kernel<2>;
+    const int chunks = m_chunks(K);
+    const int n_tiles = (D + 16 * TM - 1) / (16 * TM);
     long long fpc = (N + chunks - 1) / chunks;
     fpc = (fpc + M_SEG - 1) / M_SEG * M_SEG;
-    gmm_mstats_kernel<TM><<<dim3(K, chunks, n_pairs), 256, 0, st>>>(
+    kern<<<dim3(K, chunks, n_tiles * (n_tiles + 1) / 2), 256, 0, st>>>(
         N, resp_pad(N), X, K, D, resp, centres, partial, fpc, n_tiles, resp_floor);
     KW_CUDA_CHECK(cudaGetLastError());
-    return KW_OK;
-}
-
-int mstats_fp64(long long N, const double* X, int K, int D, const double* resp,
-                const double* centres, double* partial, double* stats, double resp_floor,
-                cudaStream_t st) {
-    const int chunks = m_chunks(K);
-    int rc;
-    if (D <= 16) rc = launch_mstats<1>(N, X, K, D, resp, centres, partial, chunks, resp_floor, st);
-    else if (D <= 32) rc = launch_mstats<2>(N, X, K, D, resp, centres, partial, chunks, resp_floor, st);
-    else if (D <= 48) rc = launch_mstats<3>(N, X, K, D, resp, centres, partial, chunks, resp_floor, st);
-    else if (D <= 80) rc = launch_mstats<5>(N, X, K, D, resp, centres, partial, chunks, resp_floor, st);
-    else rc = launch_mstats<9>(N, X, K, D, resp, centres, partial, chunks, resp_floor, st);
-    if (rc != KW_OK) return rc;
     gmm_reduce_partials_kernel<<<296, 256, 0, st>>>(K, D, chunks, partial, stats);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
@@ -849,9 +845,28 @@ extern "C" size_t kw_gmm_stats_len(int K, int D) { return (size_t)K * stats_bloc
 extern "C" size_t kw_gmm_resp_len(int64_t n_frames, int K) { return (size_t)K * (size_t)resp_pad(n_frames); }
 
 extern "C" size_t kw_gmm_workspace_bytes(int64_t n_frames, int K, int D, int precision) {
-    size_t b = carve_gmm(n_frames, K, D, nullptr).bytes;
-    if (precision == 1) b += tc_workspace_bytes(n_frames, K, D);
-    return b;
+    Carver c(nullptr);
+    carve_gmm(c, n_frames, K, D, precision, GmmUse::Fit);
+    return align_up(c.used, 256);
+}
+
+static int dim_unsupported(const char* fn, int D) {
+    set_error("%s: dim %d > %d is not supported by the E-step and tensor-core kernels", fn, D,
+              GMM_MAX_DIM);
+    return KW_ERR_UNSUPPORTED;
+}
+
+// The layout of kw_gmm_workspace_bytes over the caller's workspace.
+static int carve_fit(long long N, int K, int D, int precision, void* base, size_t bytes,
+                     GmmWorkspace& w) {
+    Carver c(base);
+    w = carve_gmm(c, N, K, D, precision, GmmUse::Fit);
+    const size_t need = align_up(c.used, 256);
+    if (need > bytes) {
+        set_error("GMM workspace too small: need %zu bytes, got %zu", need, bytes);
+        return KW_ERR_WORKSPACE;
+    }
+    return KW_OK;
 }
 
 extern "C" int kw_gmm_estep(int64_t N, const double* x_dev, int K, int D, const double* means_dev,
@@ -862,37 +877,31 @@ extern "C" int kw_gmm_estep(int64_t N, const double* x_dev, int K, int D, const 
     KW_REQUIRE(N > 0 && K > 0 && D > 0, "kw_gmm_estep: N, K, D must be positive");
     KW_REQUIRE(precision == 0 || precision == 1, "GMM precision must be 0 (fp64) or 1 (tensor)");
     KW_REQUIRE(resp_form == 0 || resp_form == 1, "resp_form must be 0 or 1");
-    GmmWorkspace w = carve_gmm(N, K, D, workspace_dev);
-    if (w.bytes > workspace_bytes) {
-        set_error("GMM workspace too small: need %zu bytes, got %zu", w.bytes, workspace_bytes);
-        return KW_ERR_WORKSPACE;
+    if (D > GMM_MAX_DIM) return dim_unsupported("kw_gmm_estep", D);
+    if (precision == 1 && resp_form == 1 && K > TC_RESP_FORM1_MAX_K) {
+        set_error("resp_form 1 supports at most %d components, got %d", TC_RESP_FORM1_MAX_K, K);
+        return KW_ERR_UNSUPPORTED;
     }
-    double* tail = stats_dev + (size_t)K * stats_block(D);
-    if (precision == 1) {
-        return estep_tc(N, x_dev, K, D, means_dev, prec_chol_dev, aux_dev, resp_dev, tail, 0,
-                        nullptr, static_cast<char*>(workspace_dev) + w.bytes,
-                        workspace_bytes - w.bytes, st, resp_form);
-    }
-    int rc = estep_fp64(N, x_dev, K, D, prec_chol_dev, aux_dev, resp_dev, w.lse_partial, 0,
-                        nullptr, st);
+    GmmWorkspace w;
+    int rc = carve_fit(N, K, D, precision, workspace_dev, workspace_bytes, w);
     if (rc != KW_OK) return rc;
-    const long long nblk = (N + E_FT - 1) / E_FT;
-    launch_reduce_fixed(w.lse_partial, nblk, (double)N, tail, st);
-    KW_CUDA_CHECK(cudaGetLastError());
-    return KW_OK;
+    Posterior out;
+    out.resp = resp_dev;
+    out.total = stats_dev + (size_t)K * stats_block(D);
+    out.resp_form = resp_form;
+    return estep_posterior(N, x_dev, K, D, means_dev, prec_chol_dev, aux_dev, precision, w, out,
+                           st);
 }
 
 extern "C" int kw_gmm_normalize_resp(int64_t N, int K, int D, double* resp_dev,
                                      void* workspace_dev, size_t workspace_bytes, void* stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     KW_REQUIRE(N > 0 && K > 0 && D > 0, "kw_gmm_normalize_resp: N, K, D must be positive");
-    GmmWorkspace w = carve_gmm(N, K, D, workspace_dev);
-    if (w.bytes > workspace_bytes) {
-        set_error("GMM workspace too small: need %zu bytes, got %zu", w.bytes, workspace_bytes);
-        return KW_ERR_WORKSPACE;
-    }
-    return normalize_resp_tc(N, K, D, resp_dev, static_cast<char*>(workspace_dev) + w.bytes,
-                             workspace_bytes - w.bytes, st);
+    if (D > GMM_MAX_DIM) return dim_unsupported("kw_gmm_normalize_resp", D);
+    GmmWorkspace w;
+    int rc = carve_fit(N, K, D, 1, workspace_dev, workspace_bytes, w);
+    if (rc != KW_OK) return rc;
+    return normalize_resp_tc(N, K, resp_dev, w.tc, st);
 }
 
 extern "C" int kw_gmm_hard_labels(int64_t N, const double* x_dev, int K, int D,
@@ -902,16 +911,12 @@ extern "C" int kw_gmm_hard_labels(int64_t N, const double* x_dev, int K, int D,
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     KW_REQUIRE(N > 0 && K > 0 && D > 0, "kw_gmm_hard_labels: N, K, D must be positive");
     KW_REQUIRE(precision == 0 || precision == 1, "GMM precision must be 0 (fp64) or 1 (tensor)");
-    GmmWorkspace w = carve_gmm(N, K, D, workspace_dev);
-    if (w.bytes > workspace_bytes) {
-        set_error("GMM workspace too small: need %zu bytes, got %zu", w.bytes, workspace_bytes);
-        return KW_ERR_WORKSPACE;
-    }
-    if (precision == 1)
-        return estep_tc(N, x_dev, K, D, means_dev, prec_chol_dev, aux_dev, nullptr, nullptr, 1,
-                        labels_dev, static_cast<char*>(workspace_dev) + w.bytes,
-                        workspace_bytes - w.bytes, st);
-    return estep_fp64(N, x_dev, K, D, prec_chol_dev, aux_dev, nullptr, nullptr, 1, labels_dev, st);
+    if (D > GMM_MAX_DIM) return dim_unsupported("kw_gmm_hard_labels", D);
+    GmmWorkspace w;
+    int rc = carve_fit(N, K, D, precision, workspace_dev, workspace_bytes, w);
+    if (rc != KW_OK) return rc;
+    return estep_labels(N, x_dev, K, D, means_dev, prec_chol_dev, aux_dev, precision, w,
+                        labels_dev, st);
 }
 
 extern "C" int kw_gmm_mstep_accumulate(int64_t N, const double* x_dev, int K, int D,
@@ -931,15 +936,12 @@ extern "C" int kw_gmm_mstep_accumulate(int64_t N, const double* x_dev, int K, in
         set_error("dim %d too large", D);
         return KW_ERR_UNSUPPORTED;
     }
-    GmmWorkspace w = carve_gmm(N, K, D, workspace_dev);
-    if (w.bytes > workspace_bytes) {
-        set_error("GMM workspace too small: need %zu bytes, got %zu", w.bytes, workspace_bytes);
-        return KW_ERR_WORKSPACE;
-    }
+    if (precision == 1 && D > GMM_MAX_DIM) return dim_unsupported("kw_gmm_mstep_accumulate", D);
+    GmmWorkspace w;
+    int rc = carve_fit(N, K, D, precision, workspace_dev, workspace_bytes, w);
+    if (rc != KW_OK) return rc;
     if (precision == 1)
-        return mstats_tc(N, x_dev, K, D, resp_dev, centres_dev, stats_dev,
-                         static_cast<char*>(workspace_dev) + w.bytes, workspace_bytes - w.bytes,
-                         st, resp_form);
+        return mstats_tc(N, K, D, resp_dev, centres_dev, stats_dev, w.tc, st, resp_form);
     return mstats_fp64(N, x_dev, K, D, resp_dev, centres_dev, w.partial, stats_dev, RESP_FLOOR, st);
 }
 
@@ -948,13 +950,11 @@ extern "C" int kw_gmm_pack_frames(int64_t N, const double* x_dev, int K, int D, 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     KW_REQUIRE(N > 0 && K > 0 && D > 0, "kw_gmm_pack_frames: N, K, D must be positive");
     if (precision != 1) return KW_OK;
-    GmmWorkspace w = carve_gmm(N, K, D, workspace_dev);
-    if (w.bytes > workspace_bytes) {
-        set_error("GMM workspace too small: need %zu bytes, got %zu", w.bytes, workspace_bytes);
-        return KW_ERR_WORKSPACE;
-    }
-    return pack_frames_tc(N, x_dev, K, D, static_cast<char*>(workspace_dev) + w.bytes,
-                          workspace_bytes - w.bytes, st);
+    if (D > GMM_MAX_DIM) return dim_unsupported("kw_gmm_pack_frames", D);
+    GmmWorkspace w;
+    int rc = carve_fit(N, K, D, precision, workspace_dev, workspace_bytes, w);
+    if (rc != KW_OK) return rc;
+    return pack_frames(N, x_dev, D, precision, w, st);
 }
 
 extern "C" int kw_gmm_mstep_finalize(int K, int D, double reg_covar, int weight_norm,

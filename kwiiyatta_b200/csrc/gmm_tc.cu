@@ -772,7 +772,7 @@ estep_tc_kernel(long long N, long long Npad, int n_tiles, int K, int D, int DP,
                 // Every warp frees the accumulator stage as soon as its own columns are in
                 // registers, so the MMAs of item g + 2 do not wait for the rest of this item's
                 // epilogue (they did: 14 % of the MMA warp's time in EM).  With `late_release`
-                // part 0 frees it only after the partial sums (see estep_tc for when).
+                // part 0 frees it only after the partial sums (see launch_estep_tc for when).
                 if (lane == 0 && (part > 0 || !late_release)) mbar_arrive(bars + BAR_TM_EMPTY0 + s);
                 // The partial sums and their named barrier therefore live in a ring of their own,
                 // four slots deep: parts 1..3 can only write slot g % 4 after the MMAs of item g,
@@ -1891,30 +1891,6 @@ constexpr int TC_STAT_CHUNKS = 1184;
 // statistics move by 1.6e-13 of their largest entry, six orders below the rounding of the
 // split-fp16 contraction itself (tools/time_mstep_real.py).  The FP64 path keeps 1e-16 per frame.
 constexpr float TC_TILE_FLOOR = 1e-8f;
-constexpr int TC_RESP_FORM1_MAX_K = 384;     // K x 64 frames of doubles in shared memory
-
-struct TcWorkspace {
-    double* colpartial;
-    double* xinfo;
-    __half* xt;
-    __half* bt;
-    float* sc;
-    double* cst;
-    double* lse_partial;
-    int32_t* cand;
-    float* mu32;
-    float* mpartial;
-    int* item_count;       // tiles with weight per M-step work item
-    int* item_order;       // work items, most tiles first
-    float* wts;            // per (component, tile): scaled weights + inverse scale (M-step)
-    double* tsum;          // per (component, tile): weight of the tile
-    int* item_counter;
-    unsigned char* tflags;
-    double* mraw;
-    int m_chunks, tiles_per_chunk, n_mtiles;
-    size_t bytes;
-};
-
 static inline int tc_dp(int D) { return (D + 15) / 16 * 16; }
 
 static int device_sms() {
@@ -1942,11 +1918,10 @@ static int tc_m_chunks(int K, long long n_mtiles) {
     return best;
 }
 
-static TcWorkspace carve_tc(long long N, int K, int D, void* base) {
+TcWorkspace carve_tc(Carver& c, long long N, int K, int D) {
     const int DP = tc_dp(D);
     const long long n_tiles = (N + tc::TILE_M - 1) / tc::TILE_M;
     const tc::MstepGeom G = tc::mstep_geom(DP);
-    Carver c(base);
     TcWorkspace w;
     w.n_mtiles = (int)(2 * n_tiles);
     w.m_chunks = tc_m_chunks(K, w.n_mtiles);
@@ -1968,33 +1943,14 @@ static TcWorkspace carve_tc(long long N, int K, int D, void* base) {
     w.item_order = c.take<int>((size_t)K * w.m_chunks);
     w.tflags = c.take<unsigned char>((size_t)K * (size_t)((w.n_mtiles + 3) / 4 * 4));
     w.mraw = c.take<double>((size_t)K * (G.partial_len + 1));
-    w.bytes = align_up(c.used, 256);
     return w;
 }
 
-size_t tc_workspace_bytes(long long N, int K, int D) { return carve_tc(N, K, D, nullptr).bytes; }
-
-static int tc_check(long long N, int K, int D, void* workspace, size_t workspace_bytes,
-                    TcWorkspace& w) {
-    if (tc_dp(D) > 144) {
-        set_error("dim %d > 144 is not supported by the tensor-core kernels", D);
-        return KW_ERR_UNSUPPORTED;
-    }
-    w = carve_tc(N, K, D, workspace);
-    if (w.bytes > workspace_bytes) {
-        set_error("tensor-core workspace too small: need %zu bytes, got %zu", w.bytes,
-                  workspace_bytes);
-        return KW_ERR_WORKSPACE;
-    }
-    return KW_OK;
-}
-
 // Centre, scale, split and tile the frames once per (X, workspace).
-int pack_frames_tc(long long N, const double* X, int K, int D, void* workspace,
-                   size_t workspace_bytes, cudaStream_t st, bool mstep_parts) {
-    TcWorkspace w;
-    int rc = tc_check(N, K, D, workspace, workspace_bytes, w);
-    if (rc != KW_OK) return rc;
+int pack_frames(long long N, const double* X, int D, int precision, const GmmWorkspace& gw,
+                cudaStream_t st, bool mstep_parts) {
+    if (precision != 1) return KW_OK;
+    const TcWorkspace& w = gw.tc;
     const int DP = tc_dp(D);
     const long long n_tiles = (N + tc::TILE_M - 1) / tc::TILE_M;
     const long long fpc = (N + TC_STAT_CHUNKS - 1) / TC_STAT_CHUNKS;
@@ -2009,17 +1965,12 @@ int pack_frames_tc(long long N, const double* X, int K, int D, void* workspace,
     return KW_OK;
 }
 
-// wlp (or resp, or argmax) through the tensor-core path; the frames must have been packed into
-// this workspace by pack_frames_tc.  mode 0: resp + sum of logsumexp into lse_out[0] and N into
-// lse_out[1] (with resp_form 0, each frame's logsumexp into lse_frame unless it is NULL);
-// mode 1: hard labels into mix (FP64 re-check of near ties).
-int estep_tc(long long N, const double* X, int K, int D, const double* means, const double* pc,
-             const double* aux, double* resp, double* lse_out, int mode, int32_t* mix,
-             void* workspace, size_t workspace_bytes, cudaStream_t st, int resp_form,
-             double* lse_frame) {
-    TcWorkspace w;
-    int rc = tc_check(N, K, D, workspace, workspace_bytes, w);
-    if (rc != KW_OK) return rc;
+// pack_l_kernel, then estep_tc_kernel<G, mode> over the frames pack_frames left in w: mode 0 writes
+// the weighted log-probabilities into resp, mode 1 the labels into mix and the near ties into
+// w.cand.
+static int launch_estep_tc(long long N, int K, int D, const double* means, const double* pc,
+                           const double* aux, const TcWorkspace& w, int mode, double* resp,
+                           int32_t* mix, cudaStream_t st) {
     const int DP = tc_dp(D);
     const long long n_tiles = (N + tc::TILE_M - 1) / tc::TILE_M;
     const long long Npad = resp_pad(N);
@@ -2029,11 +1980,10 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
     tc::pack_l_kernel<<<dim3(KI * G, tc::PACK_L_SLICES), 256, 3 * sizeof(double) * DP, st>>>(K, D, DP, G, means, pc, aux,
                                                                 w.xinfo, w.bt, w.cst);
     KW_CUDA_CHECK(cudaGetLastError());
-    const int sms = device_sms();
     const tc::EstepSmem L = tc::estep_smem(DP, G);
     uint32_t cols = 32;
     while (cols < 2u * G * DP + DP + 16) cols <<= 1;  // two accumulator stages + the frame tile (hi+ones, lo)
-    const int grid = (int)std::min<long long>(n_tiles, sms);
+    const int grid = (int)std::min<long long>(n_tiles, device_sms());
     // When the epilogue frees an accumulator stage, measured on one B200 (commit 5844b33): early
     // release takes 4 % off the EM E-step (one component per item, 27 MMAs: the MMA warp was
     // waiting for the stage) and adds 10 % to the conversion posterior (two components per item,
@@ -2049,23 +1999,37 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
                                          resp, mix, w.cand, 0.05, late_release);
         return KW_OK;
     };
+    int rc;
     if (mode == 1)
         rc = (G == 2) ? launch(tc::estep_tc_kernel<2, 1>) : launch(tc::estep_tc_kernel<1, 1>);
     else
         rc = (G == 2) ? launch(tc::estep_tc_kernel<2, 0>) : launch(tc::estep_tc_kernel<1, 0>);
     if (rc != KW_OK) return rc;
     KW_CUDA_CHECK(cudaGetLastError());
-    if (mode == 1) {
-        tc::refine_argmax_kernel<<<sms * 4, 256, 0, st>>>(N, K, D, X, pc, aux, mix, w.cand);
-        KW_CUDA_CHECK(cudaGetLastError());
-        return KW_OK;
-    }
+    return KW_OK;
+}
+
+// Hard labels, with the FP64 re-check of near ties.
+int estep_tc_labels(long long N, const double* X, int K, int D, const double* means,
+                    const double* pc, const double* aux, const TcWorkspace& w, int32_t* labels,
+                    cudaStream_t st) {
+    const int rc = launch_estep_tc(N, K, D, means, pc, aux, w, 1, nullptr, labels, st);
+    if (rc != KW_OK) return rc;
+    tc::refine_argmax_kernel<<<device_sms() * 4, 256, 0, st>>>(N, K, D, X, pc, aux, labels,
+                                                               w.cand);
+    KW_CUDA_CHECK(cudaGetLastError());
+    return KW_OK;
+}
+
+// The posterior; n_partials: how many log-likelihood partials it leaves in w.lse_partial.
+int estep_tc_posterior(long long N, int K, int D, const double* means, const double* pc,
+                       const double* aux, const TcWorkspace& w, const Posterior& out,
+                       long long& n_partials, cudaStream_t st) {
+    const int rc = launch_estep_tc(N, K, D, means, pc, aux, w, 0, out.resp, nullptr, st);
+    if (rc != KW_OK) return rc;
+    const long long Npad = resp_pad(N);
     unsigned lgrid = (unsigned)((N + 127) / 128);
-    if (resp_form == 1) {
-        if (K > TC_RESP_FORM1_MAX_K) {
-            set_error("resp_form 1 supports at most %d components, got %d", TC_RESP_FORM1_MAX_K, K);
-            return KW_ERR_UNSUPPORTED;
-        }
+    if (out.resp_form == 1) {
         // EM iteration: the M-step's inputs straight from the log-probabilities
         KW_CUDA_CHECK(cudaMemsetAsync(w.item_count, 0, sizeof(int) * (size_t)K * w.m_chunks, st));
         const int n_mt_pad = (w.n_mtiles + 3) / 4 * 4;
@@ -2078,36 +2042,27 @@ int estep_tc(long long N, const double* X, int K, int D, const double* means, co
         KW_CUDA_CHECK(cudaFuncSetAttribute(tc::lse_prep_kernel<64>,
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
         tc::lse_prep_kernel<64><<<lgrid, 128, sm, st>>>(
-            N, Npad, K, resp, w.lse_partial, n_mt_pad, w.tflags, w.wts, w.tsum,
+            N, Npad, K, out.resp, w.lse_partial, n_mt_pad, w.tflags, w.wts, w.tsum,
             TC_TILE_FLOOR, w.tiles_per_chunk, w.item_count);
     } else {
-        tc::lse_kernel<<<lgrid, 128, 0, st>>>(N, Npad, K, resp, w.lse_partial, lse_frame);
+        tc::lse_kernel<<<lgrid, 128, 0, st>>>(N, Npad, K, out.resp, w.lse_partial, out.lse_frame);
     }
     KW_CUDA_CHECK(cudaGetLastError());
-    launch_reduce_fixed(w.lse_partial, (long long)lgrid, (double)N, lse_out, st);
-    KW_CUDA_CHECK(cudaGetLastError());
+    n_partials = lgrid;
     return KW_OK;
 }
 
-// Weighted log-probabilities left by estep_tc(resp_form 1) -> responsibilities, in place.
-int normalize_resp_tc(long long N, int K, int D, double* resp, void* workspace,
-                      size_t workspace_bytes, cudaStream_t st) {
-    TcWorkspace w;
-    int rc = tc_check(N, K, D, workspace, workspace_bytes, w);
-    if (rc != KW_OK) return rc;
+// Weighted log-probabilities left by the posterior with resp_form 1 -> responsibilities, in place.
+int normalize_resp_tc(long long N, int K, double* resp, const TcWorkspace& w, cudaStream_t st) {
     tc::lse_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(N, resp_pad(N), K, resp,
                                                               w.lse_partial, nullptr);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }
 
-// M-step statistics on the tensor cores (frames packed by pack_frames_tc).
-int mstats_tc(long long N, const double* X, int K, int D, const double* resp, const double* centres,
-              double* stats, void* workspace, size_t workspace_bytes, cudaStream_t st,
-              int resp_form) {
-    TcWorkspace w;
-    int rc = tc_check(N, K, D, workspace, workspace_bytes, w);
-    if (rc != KW_OK) return rc;
+// M-step statistics on the tensor cores (frames packed by pack_frames).
+int mstats_tc(long long N, int K, int D, const double* resp, const double* centres, double* stats,
+              const TcWorkspace& w, cudaStream_t st, int resp_form) {
     const int DP = tc_dp(D);
     const tc::MstepGeom G = tc::mstep_geom(DP);
     tc::pack_centres_kernel<<<K, 160, 0, st>>>(K, D, G.DA, centres, w.xinfo, DP, w.mu32);
@@ -2117,7 +2072,7 @@ int mstats_tc(long long N, const double* X, int K, int D, const double* resp, co
     KW_CUDA_CHECK(cudaMemsetAsync(w.item_counter, 0, sizeof(int), st));
     const int n_mt_pad = (w.n_mtiles + 3) / 4 * 4;
     if (resp_form == 0) {
-        // (resp_form 1: estep_tc left flags, weights, tile sums and item counts in the workspace)
+        // (resp_form 1: the posterior left flags, weights, tile sums and item counts in the workspace)
         KW_CUDA_CHECK(cudaMemsetAsync(w.item_count, 0, sizeof(int) * (size_t)items, st));
         const long long warps = (long long)K * (n_mt_pad / 4);
         tc::mstats_tc_prep_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(

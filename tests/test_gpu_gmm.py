@@ -228,3 +228,39 @@ def test_estep_for_mstep_form(cuda, n, d, k):
     assert abs(float(lse.sum()) - float(tail_plain[0])) <= 1e-9 * abs(float(tail_plain[0]))
     scale = stats_plain.abs().max().item()
     assert (stats_log - stats_plain).abs().max().item() <= 1e-12 * scale
+
+
+@pytest.mark.parametrize('entry,precision,resp_form,d,k,why', [
+    ('kw_gmm_estep', 1, 1, 8, 385, 'at most 384 components'),
+    ('kw_gmm_estep', 1, 0, 145, 3, 'dim 145 > 144'),
+    ('kw_gmm_hard_labels', 1, 0, 145, 3, 'dim 145 > 144'),
+    ('kw_gmm_mstep_accumulate', 0, 1, 8, 3, 'takes responsibilities'),
+])
+def test_rejected_call_enqueues_nothing(cuda, entry, precision, resp_form, d, k, why):
+    """A call the GMM layer rejects raises before it queues any work: the caller's output
+    buffers and the workspace keep their bytes."""
+    from kwiiyatta_b200 import _lib
+    torch = cuda
+    n = 1000
+    lib = _lib.lib()
+    x = torch.from_numpy(np.random.default_rng(3).standard_normal((n, d))).cuda()
+    means = torch.zeros((k, d), dtype=torch.float64, device='cuda')
+    pc = torch.eye(d, dtype=torch.float64, device='cuda').repeat(k, 1, 1).contiguous()
+    aux = torch.zeros((k, d + 2), dtype=torch.float64, device='cuda')
+
+    def pattern(nbytes):
+        return torch.full((nbytes,), 0xA5, dtype=torch.uint8, device='cuda')
+    out = pattern(8 * lib.kw_gmm_resp_len(n, k))        # responsibilities or labels
+    stats = pattern(8 * lib.kw_gmm_stats_len(k, d))
+    nbytes = lib.kw_gmm_workspace_bytes(n, k, d, precision)
+    ws = pattern(nbytes)
+    tail = (ws, nbytes, _lib.stream_ptr(torch))
+    args = {'kw_gmm_estep': (n, x, k, d, means, pc, aux, out, stats, precision, resp_form) + tail,
+            'kw_gmm_hard_labels': (n, x, k, d, means, pc, aux, out, precision) + tail,
+            'kw_gmm_mstep_accumulate': (n, x, k, d, out, means, stats, precision,
+                                        resp_form) + tail}[entry]
+    with pytest.raises(NotImplementedError, match=why):
+        _lib.call(entry, *args)
+    torch.cuda.synchronize()
+    for buf in (out, stats, ws):
+        assert bool((buf == 0xA5).all())
