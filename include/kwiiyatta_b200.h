@@ -179,6 +179,59 @@ int kw_gmm_precision_cholesky(int n_components, int dim, const double* weights_d
                               void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Joint GMM with diagonal covariance blocks  (GaussianMixture(covariance_type='diagonal_blocks')).
+ * D = 2 Dh is even, 2 <= D <= 144.  Each Dh x Dh block Sxx, Sxy, Syx, Syy of a covariance is
+ * diagonal, so the model is one 2 x 2 Gaussian per component and feature pair (x_d, y_d) with
+ * y_d = z[Dh + d].  FP64 on the CUDA cores; the summation order is fixed (bitwise reproducible).
+ * One EM iteration = kw_gmm_db_estep + kw_gmm_db_mstep_accumulate (+ the caller's all-reduce of
+ * `stats`) + kw_gmm_db_mstep_finalize, as for the full model.
+ *
+ * Compact model buffers (device, float64):
+ *   weights (K), means (K, D) as for the full model;
+ *   covariances (K, Dh, 3): per pair [ S_xx[d][d], S_xy[d][d], S_yy[d][d] ] (reg_covar included);
+ *   factors (K, Dh, 3): per pair [ a, b, c ] of the upper factor U = [[a, b], [0, c]] with
+ *     Sigma_d^-1 = U U^T.  In sklearn's (K, D, D) precisions_cholesky_ these are the entries
+ *     (d, d), (d, Dh + d) and (Dh + d, Dh + d); every other entry is zero;
+ *   aux (K, 2): [ log|U_k| (sum of log a + log c over the pairs), log w_k ].
+ * stats layout: K blocks of (1 + D + 3 Dh): [ n_k, sum r (z - c_k), per pair sum r u^2,
+ *   sum r u v, sum r v^2 ] with u = x_d - c_k[d], v = y_d - c_k[Dh + d], followed by the same
+ *   2 scalars as the full model [ sum_n log p(x_n), n_frames ].  Length kw_gmm_db_stats_len.
+ * Responsibilities: the full model's layout (kw_gmm_resp_len).
+ * Every entry point checks all its arguments before it queues any work: n_frames >= 0,
+ * n_components >= 1, the dimension, reg_covar >= 0, weight_norm, NULL buffers and the workspace
+ * size (KW_ERR_INVALID / KW_ERR_WORKSPACE).
+ * ------------------------------------------------------------------------------------------ */
+size_t kw_gmm_db_stats_len(int n_components, int dim);
+size_t kw_gmm_db_workspace_bytes(int64_t n_frames, int n_components, int dim);
+
+/* E-step: responsibilities into resp_dev, {sum_n log p(x_n), n_frames} into the stats tail, and
+ * (when lse_frame_dev is not NULL) each frame's log-normaliser logsumexp_k log(w_k N(x_n | k)). */
+int kw_gmm_db_estep(int64_t n_frames, const double* x_dev, int n_components, int dim,
+                    const double* means_dev, const double* factors_dev, const double* aux_dev,
+                    double* resp_dev, double* stats_dev, double* lse_frame_dev,
+                    void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* M-step statistics around centres_dev (K, D) from responsibilities; frames with r_nk <= 1e-16
+ * are skipped, as in the full model's FP64 M-step. */
+int kw_gmm_db_mstep_accumulate(int64_t n_frames, const double* x_dev, int n_components, int dim,
+                               const double* resp_dev, const double* centres_dev,
+                               double* stats_dev, void* workspace_dev, size_t workspace_bytes,
+                               void* stream);
+
+/* Parameters from (all-reduced) statistics; weight_norm and info_dev as kw_gmm_mstep_finalize
+ * (the pivot index counts in the expanded D x D matrix). */
+int kw_gmm_db_mstep_finalize(int n_components, int dim, double reg_covar, int weight_norm,
+                             const double* stats_dev, const double* centres_dev,
+                             double* weights_dev, double* means_dev, double* covariances_dev,
+                             double* factors_dev, double* aux_dev, int32_t* info_dev,
+                             void* stream);
+
+/* factors / aux from given compact covariances and weights. */
+int kw_gmm_db_precision_cholesky(int n_components, int dim, const double* weights_dev,
+                                 const double* covariances_dev, double* factors_dev,
+                                 double* aux_dev, int32_t* info_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Conversion: posterior + conditional Gaussian + MLPG  (nnmnkwii MLPG.transform,
  * kwiiyatta/converter/gmm.py:28-34).  dim_half = D/2 (72), static_dim = dim_half/3 (24).
  *

@@ -38,6 +38,13 @@ SIGNATURES = {
     'kw_gmm_mstep_finalize': (_i, [_i, _i, _dbl, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                    _vp]),
     'kw_gmm_precision_cholesky': (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'kw_gmm_db_stats_len': (_sz, [_i, _i]),
+    'kw_gmm_db_workspace_bytes': (_sz, [_i64, _i, _i]),
+    'kw_gmm_db_estep': (_i, [_i64, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kw_gmm_db_mstep_accumulate': (_i, [_i64, _vp, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kw_gmm_db_mstep_finalize': (_i, [_i, _i, _dbl, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                      _vp, _vp]),
+    'kw_gmm_db_precision_cholesky': (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     'kw_convert_prepared_len': (_sz, [_i, _i]),
     'kw_convert_prepare': (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     'kw_convert_soft_workspace_bytes': (_sz, [_i64, _i, _i]),

@@ -6,7 +6,8 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_PATH = os.path.join(HERE, 'libkwiiyatta_b200.so')
-SOURCES = ['dtw.cu', 'gmm.cu', 'gmm_tc.cu', 'convert.cu', 'assemble.cu', 'capi.cu']
+SOURCES = ['dtw.cu', 'gmm.cu', 'gmm_tc.cu', 'gmm_diagblocks.cu', 'convert.cu', 'assemble.cu',
+           'capi.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '--threads', '0',
               '-shared', '-Xcompiler', '-fPIC']
 

@@ -112,6 +112,9 @@ def load_converter(path, Converter=B200GMMFeatureConverter, **kwargs):
     with np.load(path) as data:
         state = {k: data[k] for k in data.files}
     layers = {k[6:]: state.pop(k) for k in list(state) if k.startswith('layer_')}
+    kind = str(state.get('covariance_type', 'full'))
+    if kind != 'full':
+        kwargs.setdefault('covariance_type', kind)
     backend = Converter(components=int(state['n_components']), verbose=0, **kwargs)
     backend.load_state_dict(state)
     node = backend

@@ -58,6 +58,10 @@ long long resp_pad(long long n);
 
 constexpr int GMM_MAX_DIM = 144;            // the E-step at both precisions, every tensor-core kernel
 constexpr int TC_RESP_FORM1_MAX_K = 384;    // resp_form 1: K x 64 frames of doubles in shared memory
+constexpr double RESP_FLOOR = 1e-16;        // the FP64 M-steps skip responsibilities at or below this
+
+// reduce_fixed_kernel: out = { sum of in[0, n) in a fixed order, extra }.
+int reduce_fixed(const double* in, long long n, double extra, double* out, cudaStream_t st);
 
 // The tensor-core region of a GMM workspace (precision 1).
 struct TcWorkspace {

@@ -19,7 +19,6 @@ namespace kw {
 
 constexpr int E_FT = 64;   // frames per CTA tile in the E-step
 constexpr int E_KC = 16;   // contraction chunk
-constexpr double RESP_FLOOR = 1e-16;  // responsibilities at or below this are skipped in the M-step
 constexpr int M_FB = 8;    // frames per smem stage in the M-step (static smem < 48 KB)
 
 __host__ __device__ static inline size_t stats_block(int D) { return 1 + (size_t)D + (size_t)D * D; }
@@ -787,7 +786,11 @@ int estep_posterior(long long N, const double* X, int K, int D, const double* me
             : estep_fp64(N, X, K, D, pc, aux, out.resp, w.lse_partial, 0, nullptr, st,
                          out.lse_frame);
     if (rc != KW_OK || out.total == nullptr) return rc;
-    reduce_fixed_kernel<<<1, 256, 0, st>>>(w.lse_partial, n_partials, (double)N, out.total);
+    return reduce_fixed(w.lse_partial, n_partials, (double)N, out.total, st);
+}
+
+int reduce_fixed(const double* in, long long n, double extra, double* out, cudaStream_t st) {
+    reduce_fixed_kernel<<<1, 256, 0, st>>>(in, n, extra, out);
     KW_CUDA_CHECK(cudaGetLastError());
     return KW_OK;
 }

@@ -1,4 +1,4 @@
-"""Joint full-covariance GMM on the B200: the back-end behind kwiiyatta's converter seam.
+"""Joint GMM on the B200: the back-end behind kwiiyatta's converter seam.
 
 * ``GaussianMixture`` keeps the slice of ``sklearn.mixture.GaussianMixture`` the reference
   uses (kwiiyatta/converter/gmm.py:13-26; nnmnkwii's MLPG reads ``weights_``, ``means_``,
@@ -8,8 +8,11 @@
   and is what ``MelCepstrumConverter(Converter=...)`` / ``Config.create_converter(Converter=...)``
   (kwiiyatta/converter/__init__.py:9-14, kwiiyatta/config.py:59-69) receive.
 
-Every E-step / M-step / finalisation runs in csrc/gmm.cu through the C ABI; the only
-host-side arithmetic is the scalar convergence test.  With ``torch.distributed`` initialised
+Two model types: ``covariance_type='full'`` (sklearn's, the default) and
+``'diagonal_blocks'``, a joint model whose four D/2 x D/2 covariance blocks are diagonal (each
+x_d is coupled to y_d only).  Every E-step / M-step / finalisation runs in csrc/gmm.cu,
+csrc/gmm_tc.cu or csrc/gmm_diagblocks.cu through the C ABI; the only host-side arithmetic is the
+scalar convergence test.  With ``torch.distributed`` initialised
 the per-iteration sufficient statistics are summed over ranks (one all-reduce per iteration);
 every rank then finalises identical parameters.
 """
@@ -62,6 +65,26 @@ def _as_device(x, torch, device):
 _on_own_device = _lib.device_guard(lambda self, *a: self.device)
 
 
+def _pair_index(d, device, torch):
+    """Rows and columns of the (D, D) entries a diagonal-blocks model keeps: per pair d the
+    upper-pattern entries (d, d), (d, Dh + d), (Dh + d, Dh + d)."""
+    i = torch.arange(d // 2, device=device)
+    return i, i + d // 2
+
+
+def _expand_pairs(torch, compact, symmetric):
+    """(K, Dh, 3) compact covariances (``symmetric``) or precision factors -> (K, D, D)."""
+    k, dh, _ = compact.shape
+    i, j = _pair_index(2 * dh, compact.device, torch)
+    out = torch.zeros((k, 2 * dh, 2 * dh), dtype=compact.dtype, device=compact.device)
+    out[:, i, i] = compact[:, :, 0]
+    out[:, i, j] = compact[:, :, 1]
+    out[:, j, j] = compact[:, :, 2]
+    if symmetric:
+        out[:, j, i] = compact[:, :, 1]
+    return out
+
+
 class GaussianMixture:
     covariance_type = 'full'
 
@@ -70,15 +93,20 @@ class GaussianMixture:
                  means_init=None, precisions_init=None, random_state=None, warm_start=False,
                  verbose=0, verbose_interval=10, precision='auto', resp_init=None,
                  process_group=None, device=None, reorder_every=10):
-        if covariance_type != 'full':
-            raise NotImplementedError("only covariance_type='full' is built "
-                                      '(kwiiyatta/converter/gmm.py:17-18)')
+        if covariance_type not in ('full', 'diagonal_blocks'):
+            raise NotImplementedError("only covariance_type='full' (kwiiyatta/converter/gmm.py:"
+                                      "17-18) and 'diagonal_blocks' are built")
+        if covariance_type == 'diagonal_blocks' and PRECISIONS[precision] == 1:
+            raise ValueError("covariance_type='diagonal_blocks' runs in FP64 only: use "
+                             "precision='fp64' or 'auto'")
         if n_init != 1 or warm_start:
             raise NotImplementedError('n_init > 1 / warm_start are not built')
         if precisions_init is not None:
             raise NotImplementedError('precisions_init is not built; pass resp_init or '
                                       'means_init + weights_init')
         self.n_components = n_components
+        self.covariance_type = covariance_type
+        self._db = covariance_type == 'diagonal_blocks'
         self.tol = tol
         self.reg_covar = reg_covar
         self.max_iter = max_iter
@@ -90,7 +118,8 @@ class GaussianMixture:
         self.verbose = verbose
         self.verbose_interval = verbose_interval
         self.precision_request = precision
-        self.precision = PRECISIONS[precision]      # -1 ('auto') until the frames are seen
+        # -1 ('auto') until the frames are seen; the diagonal-blocks model has the FP64 path only
+        self.precision = 0 if self._db else PRECISIONS[precision]
         self.resp_init = resp_init
         self.process_group = process_group
         self.device = device
@@ -113,14 +142,12 @@ class GaussianMixture:
         self._weights = torch.empty(k, **f64)
         self._means = [torch.empty((k, d), **f64), torch.empty((k, d), **f64)]
         self._cur = 0
-        self._cov = torch.empty((k, d, d), **f64)
-        self._pc = torch.empty((k, d, d), **f64)
-        self._aux = torch.empty((k, d + 2), **f64)
+        self._alloc_model(torch, k, d, dev)
         self._info = torch.zeros(k, dtype=torch.int32, device=dev)
-        self._stats = torch.zeros(lib.kw_gmm_stats_len(k, d), **f64)
+        self._stats = torch.zeros(self._stats_len(k, d), **f64)
         self._npad = lib.kw_gmm_resp_len(n, k) // k
         self._resp = torch.zeros((k, self._npad), **f64)   # component-major
-        self._ws_bytes = lib.kw_gmm_workspace_bytes(n, k, d, self.precision)
+        self._ws_bytes = self._workspace_bytes(n, k, d)
         self._ws = _lib.workspace(self._ws_bytes, dev)
         # two slots of pinned host memory for the per-iteration scalars (sum log p, n) and the
         # finalisation flags: copied asynchronously, read half an iteration later
@@ -128,7 +155,35 @@ class GaussianMixture:
         self._host_info = torch.empty((2, k), dtype=torch.int32).pin_memory()
         self._tickets = 0
 
+    def _alloc_model(self, torch, k, d, dev):
+        """Covariances, precision factors and aux: (K, D, D), (K, D, D), (K, D + 2) for the full
+        model; the compact (K, D/2, 3), (K, D/2, 3), (K, 2) of include/kwiiyatta_b200.h for
+        diagonal blocks."""
+        f64 = dict(dtype=torch.float64, device=dev)
+        if self._db:
+            if d % 2:
+                raise ValueError(f"covariance_type='diagonal_blocks' needs an even dimension, "
+                                 f'got {d}')
+            self._pc = torch.empty((k, d // 2, 3), **f64)
+            self._aux = torch.empty((k, 2), **f64)
+        else:
+            self._pc = torch.empty((k, d, d), **f64)
+            self._aux = torch.empty((k, d + 2), **f64)
+        self._cov = torch.empty(self._pc.shape, **f64)
+
+    def _stats_len(self, k, d):
+        lib = _lib.lib()
+        return lib.kw_gmm_db_stats_len(k, d) if self._db else lib.kw_gmm_stats_len(k, d)
+
+    def _workspace_bytes(self, n, k, d):
+        lib = _lib.lib()
+        if self._db:
+            return lib.kw_gmm_db_workspace_bytes(n, k, d)
+        return lib.kw_gmm_workspace_bytes(n, k, d, self.precision)
+
     def _pack(self, torch, x):
+        if self._db:
+            return
         n, d = x.shape
         _lib.call('kw_gmm_pack_frames', n, x, self.n_components, d, self.precision, self._ws,
                   self._ws_bytes, _lib.stream_ptr(torch))
@@ -163,6 +218,11 @@ class GaussianMixture:
         responsibilities themselves are never written (kw_gmm_estep resp_form 1)."""
         x = self._frames(x)
         n, d = x.shape
+        if self._db:
+            _lib.call('kw_gmm_db_estep', n, x, self.n_components, d, self._means[self._cur],
+                      self._pc, self._aux, self._resp, self._stats, None, self._ws,
+                      self._ws_bytes, _lib.stream_ptr(torch))
+            return
         self._resp_log = (bool(for_mstep) and self.precision == 1
                           and self.n_components <= RESP_FORM1_MAX_COMPONENTS)
         _lib.call('kw_gmm_estep', n, x, self.n_components, d, self._means[self._cur], self._pc,
@@ -181,6 +241,10 @@ class GaussianMixture:
     def _accumulate(self, torch, x, centres):
         x = self._frames(x)
         n, d = x.shape
+        if self._db:
+            _lib.call('kw_gmm_db_mstep_accumulate', n, x, self.n_components, d, self._resp,
+                      centres, self._stats, self._ws, self._ws_bytes, _lib.stream_ptr(torch))
+            return
         _lib.call('kw_gmm_mstep_accumulate', n, x, self.n_components, d, self._resp, centres,
                   self._stats, self.precision, int(self._resp_log), self._ws, self._ws_bytes,
                   _lib.stream_ptr(torch))
@@ -193,8 +257,8 @@ class GaussianMixture:
     def _finalize(self, torch, centres, weight_norm):
         k, d = centres.shape
         new = self._means[self._cur ^ 1]
-        _lib.call('kw_gmm_mstep_finalize', k, d, float(self.reg_covar), weight_norm, self._stats,
-                  centres, self._weights, new, self._cov, self._pc, self._aux, self._info,
+        entry = 'kw_gmm_db_mstep_finalize' if self._db else 'kw_gmm_mstep_finalize'
+        _lib.call(entry, k, d, float(self.reg_covar), weight_norm, self._stats, centres, self._weights, new, self._cov, self._pc, self._aux, self._info,
                   _lib.stream_ptr(torch))
         self._cur ^= 1
 
@@ -253,7 +317,7 @@ class GaussianMixture:
         count = torch.tensor([float(n)], dtype=torch.float64, device=dev)
         if multi:
             dist.all_reduce(count, group=self.process_group)
-        if self.precision_request == 'auto':
+        if self.precision_request == 'auto' and not self._db:
             self.precision = resolve_precision('auto', int(count.item()), k, d)
         self._alloc(torch, n, d, dev)
         self._x_src, self._x_used, self._iters_done = x, None, 0
@@ -390,13 +454,30 @@ class GaussianMixture:
             self._weights.copy_(_as_device(self.weights_init, torch, dev))
         if self.means_init is not None:
             self._means[self._cur].copy_(_as_device(self.means_init, torch, dev))
+        self._precision_cholesky(torch)
+
+    def _precision_cholesky(self, torch):
+        """Precision factors and aux of ``_cov`` and ``_weights`` (and, for the full model, of the
+        current means)."""
         k, d = self._means[self._cur].shape
+        if self._db:
+            _lib.call('kw_gmm_db_precision_cholesky', k, d, self._weights, self._cov, self._pc,
+                      self._aux, self._info, _lib.stream_ptr(torch))
+            return
         _lib.call('kw_gmm_precision_cholesky', k, d, self._weights, self._means[self._cur],
                   self._cov, self._pc, self._aux, self._info, _lib.stream_ptr(torch))
 
     def _publish(self):
+        """The fitted attributes.  A diagonal-blocks model publishes full (K, D, D) covariances
+        and precision Cholesky factors, zero outside its pattern, so that every consumer of a
+        full model (MLPG conversion, sklearn-style code) takes it as it is."""
         self.weights_ = self._weights.cpu().numpy()
         self.means_ = self._means[self._cur].cpu().numpy()
+        if self._db:
+            import torch
+            self.covariances_ = _expand_pairs(torch, self._cov, True).cpu().numpy()
+            self.precisions_cholesky_ = _expand_pairs(torch, self._pc, False).cpu().numpy()
+            return
         self.covariances_ = self._cov.cpu().numpy()
         self.precisions_cholesky_ = self._pc.cpu().numpy()
 
@@ -407,7 +488,9 @@ class GaussianMixture:
 
     @_on_own_device
     def set_parameters(self, weights, means, covariances):
-        """Load an existing model (e.g. a fitted sklearn GaussianMixture's attributes)."""
+        """Load an existing model (e.g. a fitted sklearn GaussianMixture's attributes).  With
+        ``covariance_type='diagonal_blocks'`` the (K, D, D) covariances must be zero outside the
+        pattern of diagonal blocks (ValueError otherwise)."""
         torch = _lib.require_cuda()
         dev = torch.device('cuda' if self.device is None else self.device)
         means = np.asarray(means, dtype=np.float64)
@@ -417,12 +500,23 @@ class GaussianMixture:
         self._weights = _as_device(weights, torch, dev)
         self._means = [_as_device(means, torch, dev), torch.empty((k, d), **f64)]
         self._cur = 0
-        self._cov = _as_device(covariances, torch, dev)
-        self._pc = torch.empty((k, d, d), **f64)
-        self._aux = torch.empty((k, d + 2), **f64)
+        self._alloc_model(torch, k, d, dev)
+        cov = _as_device(covariances, torch, dev)
+        if self._db:
+            if tuple(cov.shape) != (k, d, d):
+                raise ValueError(f'covariances must have shape {(k, d, d)}, got '
+                                 f'{tuple(cov.shape)}')
+            keep = _expand_pairs(torch, torch.ones((1, d // 2, 3), **f64), True)[0] != 0
+            if bool((cov[:, ~keep] != 0).any()):
+                raise ValueError("covariance_type='diagonal_blocks': a covariance has a non-zero "
+                                 'entry outside the diagonal blocks')
+            i, j = _pair_index(d, dev, torch)
+            # the lower triangle, as sklearn's Cholesky reads it
+            self._cov = torch.stack([cov[:, i, i], cov[:, j, i], cov[:, j, j]], dim=-1)
+        else:
+            self._cov = cov
         self._info = torch.zeros(k, dtype=torch.int32, device=dev)
-        _lib.call('kw_gmm_precision_cholesky', k, d, self._weights, self._means[0], self._cov,
-                  self._pc, self._aux, self._info, _lib.stream_ptr(torch))
+        self._precision_cholesky(torch)
         self._check_info()
         self._publish()
         return self
@@ -436,11 +530,10 @@ class GaussianMixture:
         lib = _lib.lib()
         self._npad = lib.kw_gmm_resp_len(n, k) // k
         self._resp = torch.empty((k, self._npad), dtype=torch.float64, device=x.device)
-        self._stats = torch.zeros(lib.kw_gmm_stats_len(k, d), dtype=torch.float64,
-                                  device=x.device)
+        self._stats = torch.zeros(self._stats_len(k, d), dtype=torch.float64, device=x.device)
         if self.precision < 0:      # 'auto' on a model that was loaded, not fitted: FP64 posteriors
             self.precision = 0
-        self._ws_bytes = lib.kw_gmm_workspace_bytes(n, k, d, self.precision)
+        self._ws_bytes = self._workspace_bytes(n, k, d)
         self._ws = _lib.workspace(self._ws_bytes, x.device)
         self._pack(torch, x)
         self._estep(torch, x)
@@ -545,7 +638,7 @@ class B200GMMFeatureConverter(FeatureConverter):
         """The fitted model and its hyper-parameters as plain numpy arrays / scalars."""
         g = self.gmm
         return {'weights': g.weights_, 'means': g.means_, 'covariances': g.covariances_,
-                'n_components': g.n_components, 'max_iter': g.max_iter, 'tol': g.tol,
+                'covariance_type': g.covariance_type, 'n_components': g.n_components, 'max_iter': g.max_iter, 'tol': g.tol,
                 'reg_covar': g.reg_covar,
                 'random_state': -1 if g.random_state is None else g.random_state,
                 'n_iter': getattr(g, 'n_iter_', 0), 'converged': getattr(g, 'converged_', False),
@@ -553,7 +646,12 @@ class B200GMMFeatureConverter(FeatureConverter):
                 **({} if self._gv is None else {'gv_mean': self._gv.mean, 'gv_var': self._gv.var})}
 
     def load_state_dict(self, state):
+        """``state`` as ``state_dict`` gives it; one without 'covariance_type' is a full model."""
         g = self.gmm
+        kind = str(state.get('covariance_type', 'full'))
+        if kind != g.covariance_type:
+            raise ValueError(f'the state holds a covariance_type={kind!r} model, this converter '
+                             f'was built for {g.covariance_type!r}')
         g.set_parameters(np.asarray(state['weights']), np.asarray(state['means']),
                          np.asarray(state['covariances']))
         g.max_iter, g.tol, g.reg_covar = int(state['max_iter']), float(state['tol']), \
@@ -573,6 +671,9 @@ class B200GMMFeatureConverter(FeatureConverter):
     def load(cls, path, **kwargs):
         with np.load(path) as state:
             state = {k: state[k] for k in state.files}
+        kind = str(state.get('covariance_type', 'full'))
+        if kind != 'full':
+            kwargs.setdefault('covariance_type', kind)
         conv = cls(components=int(state['n_components']), verbose=0, **kwargs)
         return conv.load_state_dict(state)
 

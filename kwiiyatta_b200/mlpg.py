@@ -113,8 +113,10 @@ class MLPG:
             raise NotImplementedError('a single window must be the static window (0, 0, [1.0])')
         if swap:
             raise NotImplementedError('swap=True is not built')
-        if getattr(gmm, 'covariance_type', 'full') != 'full':
-            raise AssertionError("covariance_type must be 'full'")
+        # a diagonal-blocks model publishes its expanded (K, D, D) covariances: the kernels of the
+        # full model convert it unchanged
+        if getattr(gmm, 'covariance_type', 'full') not in ('full', 'diagonal_blocks'):
+            raise AssertionError("covariance_type must be 'full' or 'diagonal_blocks'")
         self.windows = windows
         self.diff = bool(diff)
         dev = self._dev
